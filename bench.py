@@ -16,6 +16,10 @@ run also reports the skipping variant as `skip_variant`.
 `e2e` is the same metric through the host-buffer C-ABI call lsb_sort_host (pinned host memory
 in, pinned host memory out, copies inside the timed region, wall clock); `e2e.overlapped` (N = 1)
 is two sorters fed from two threads, so one batch's copy in shares the link with another's copy out.
+`--dump-outputs DIR` writes a fixed sample of the last timed step's sorted output as .npy files (see dump_outputs),
+so that two builds run with the same arguments can be compared output for output.
+`cpu_baseline` and --impl reference need oracle/_ref, which oracle/build_ref.sh builds only where the reference's
+source is present; without it `cpu_baseline.value` is null.
 """
 import argparse
 import json
@@ -82,10 +86,15 @@ class ClockSampler:
 # --------------------------------------------------------------------------------------
 # reference arm / cpu_baseline: the UNMODIFIED mpi_lsbsort.cpp (oracle/_ref, ranks = threads)
 # --------------------------------------------------------------------------------------
-def run_reference_once(n, ranks):
+def reference_binary():
+    """path of the reference program oracle/build_ref.sh builds, or None: it needs the reference's source,
+    which the repository does not contain, and bench.py never compiles into the tree itself"""
     from oracle import oracle as O  # the one place bench.py may execute oracle/: the CPU baseline
-    if not os.path.exists(O.REF_BIN):
-        O.build()
+    return O.REF_BIN if os.path.exists(O.REF_BIN) else None
+
+
+def run_reference_once(n, ranks):
+    from oracle import oracle as O
     env = dict(os.environ, SHIM_RANKS=str(ranks))
     out = subprocess.run([O.REF_BIN, "--n", str(n), "--no-verify"], env=env, check=True, capture_output=True,
                          text=True).stdout
@@ -105,6 +114,10 @@ def cpu_baseline(sample_log2=None):
     """bounded sample of the same workload on the host cores; ~10-30 s of CPU work"""
     cores = host_threads()
     ranks = max(1, min(cores, 64))
+    if reference_binary() is None:
+        return {"value": None, "unit": UNIT, "kind": "reference",
+                "note": "not measured: the reference program oracle/_ref/mpi_lsbsort_shim is not built "
+                        "(oracle/build_ref.sh needs the reference's source)"}
     n = 1 << (sample_log2 or 24)
     rate, secs = run_reference_once(n, ranks)
     if sample_log2 is None and secs < 1.5:  # fast host: take a bigger, steadier sample (~10-20 s of CPU work)
@@ -125,6 +138,37 @@ def bench_shape(args, world):
     return per, world << per, "weak"
 
 
+DUMP_ELEMENTS = 1 << 20  # in all ranks together: 4 float64 arrays of this length are 32 MiB
+DUMP_BLOCKS = 1024
+DUMP_SEED = 20261020
+
+
+def dump_outputs(sorter, out_dir, rank, world):
+    """--dump-outputs: the sorted shard the last timed step left on this GPU, as a fixed sample.
+
+    A shard with more than DUMP_ELEMENTS / world elements is sampled as DUMP_BLOCKS contiguous blocks, one at a
+    seeded offset inside each of DUMP_BLOCKS equal strata; the offsets depend on the shard size only, so two builds
+    run with the same arguments dump the same positions.  Written as float64, which holds every value exactly:
+    index.npy (global position), key_hi.npy / key_lo.npy (upper and lower 32 bits of the key), val.npy.
+    With several GPUs each rank writes rank<r>_<name>.npy for its shard."""
+    import numpy as np
+    here, want = sorter.here, DUMP_ELEMENTS // world
+    if here <= want:
+        starts, blen = np.array([0], dtype=np.int64), here
+    else:
+        blen = want // DUMP_BLOCKS
+        stratum = here // DUMP_BLOCKS
+        rng = np.random.default_rng([DUMP_SEED, here])
+        starts = np.arange(DUMP_BLOCKS, dtype=np.int64) * stratum + rng.integers(0, stratum - blen + 1, DUMP_BLOCKS)
+    elts = np.concatenate([sorter.download(local_off=int(s), count=blen) for s in starts])
+    index = (sorter.first_global + starts[:, None] + np.arange(blen, dtype=np.int64)[None, :]).reshape(-1)
+    os.makedirs(out_dir, exist_ok=True)
+    prefix = f"rank{rank}_" if world > 1 else ""
+    for name, a in (("index", index), ("key_hi", elts["key"] >> np.uint64(32)),
+                    ("key_lo", elts["key"] & np.uint64(0xFFFFFFFF)), ("val", elts["val"])):
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a.astype(np.float64))
+
+
 def config_dict(args, world, n, here, npass):
     return {"workload": workload_name(world, args), "n_total": n, "n_per_gpu": here, "radix_bits": args.radix,
             "passes": npass, "pcg_streams": world, "key_mask": hex(args.key_mask), "and_draws": args.and_draws,
@@ -135,6 +179,9 @@ def config_dict(args, world, n, here, npass):
 def main_reference(args, rank):
     if rank != 0:
         return 0
+    if reference_binary() is None:
+        raise SystemExit("bench.py --impl reference: oracle/_ref/mpi_lsbsort_shim is not built "
+                         "(oracle/build_ref.sh needs the reference's source)")
     world = args.gpus
     cores = host_threads()
     ranks = max(1, min(cores, 64))
@@ -245,16 +292,20 @@ def main_cuda(args, rank, world, local_rank, own_process_group=True, tag=None):
     step_ms, launches, part_ms, part_launches = [], 0, 0.0, 0
     if rank == 0:
         sampler.start()
-    for _ in range(args.steps):
-        sorter.generate()          # fresh input, resident in HBM before the timed region
-        barrier()
-        st = sorter.my_sort()      # CUDA events bracket the kernels on the sort stream
-        barrier()
-        step_ms.append(max_over_ranks(st.device_ms))
-        launches += st.kernel_launches
-        part_ms += st.partition_ms
-        part_launches += st.partition_launches
-    clocks = sampler.stop() if rank == 0 else None
+    try:  # the nvidia-smi sampler must not outlive a failed step
+        for _ in range(args.steps):
+            sorter.generate()          # fresh input, resident in HBM before the timed region
+            barrier()
+            st = sorter.my_sort()      # CUDA events bracket the kernels on the sort stream
+            barrier()
+            step_ms.append(max_over_ranks(st.device_ms))
+            launches += st.kernel_launches
+            part_ms += st.partition_ms
+            part_launches += st.partition_launches
+    finally:
+        clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(sorter, args.dump_outputs, rank, world)
     total_s = sum(step_ms) / 1e3
     value = n * args.steps / total_s / 1e6
 
@@ -512,7 +563,13 @@ def main():
     ap.add_argument("--no-alt", action="store_true", help="skip the short run of the other pass shape (N = 1)")
     ap.add_argument("--clock-period-ms", type=int, default=100, help="nvidia-smi sampling period during the timed region")
     ap.add_argument("--suite", default="", help="'name:flags;name:flags;...': several configurations in one launch, one JSON line each")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write a fixed sample of the last step's sorted output to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.suite:
+        ap.error("--dump-outputs writes one configuration's outputs; it does not combine with --suite")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -4,6 +4,7 @@ run without a GPU instead of falling back."""
 import ctypes
 import os
 import subprocess
+import sys
 
 import pytest
 
@@ -38,14 +39,15 @@ def test_struct_layouts_match_header(tmp_path):
 
 
 def test_no_cpu_fallback():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+    """with no CUDA device visible the library raises instead of sorting on the host; the check runs in a child
+    process with CUDA_VISIBLE_DEVICES empty, so it holds on a machine with a GPU as well"""
     if not os.path.exists(lsb.library_path()):
         pytest.skip("liblsbsort.so not built")
-    with pytest.raises(lsb.LsbError) as e:
-        lsb.DistributedSorter(100)
-    assert "no CPU fallback" in str(e.value)
+    code = ("import sys; sys.path.insert(0, sys.argv[1]); import distributed_lsb_b200 as lsb\n"
+            "try:\n    lsb.DistributedSorter(100)\nexcept lsb.LsbError as e:\n    print(e)\n")
+    out = subprocess.run([sys.executable, "-c", code, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, check=True).stdout
+    assert "no CPU fallback" in out
 
 
 def test_product_never_imports_oracle():
