@@ -695,10 +695,11 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
   const bool two_step = p.lo_bits && !(c->cfg.flags & LSB_FLAG_ONE_PASS);
   const bool timed = (c->cfg.flags & LSB_FLAG_PHASE_EVENTS) != 0;
   const int xbuf = c->cur ^ 1;
-  int last_x = -1, prev_x = -1;
+  int last_x = -1, prev_x = -1, sorted_parts = 0;
   for (int q = 0; q < V; q++) {
     const int64_t m = part_len(c, q);
     if (m <= 0) continue;
+    const int slot = sorted_parts++ & 1;  // empty parts take no scratch: alternate over the parts that are sorted
     Elt* part = c->buf[c->cur] + c->pstart[q];
     const int64_t* segs = c->seg_start + 2 * (1 + q);
     const uint32_t* tiles = c->seg_tiles + 2 * (1 + q);
@@ -712,8 +713,8 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
       sorted = part;
       (*subpasses) += 2;
     } else {  // one launch; its output lives in an alternating scratch until it has been exchanged
-      Elt* out = c->scratch[q & 1];
-      if (prev_x >= 0) CU(c, cudaStreamWaitEvent(c->stream, c->ev_x[prev_x], 0));  // scratch[q & 1] was read by that exchange
+      Elt* out = c->scratch[slot];
+      if (prev_x >= 0) CU(c, cudaStreamWaitEvent(c->stream, c->ev_x[prev_x], 0));  // scratch[slot] was read by that exchange
       if (p.lo_bits) rc = launch_onepass(c, part, out, m, p.shift, p.bits, c->localbase_v + (size_t)q * nb, 0, c->tune.op_ctas_mgpu);
       else rc = launch_partition(c, part, m, p.shift, p.hi_bits, segs, tiles, c->bases_v + ((size_t)q * 2 + 1) * 257, out);
       if (rc) return rc;

@@ -66,12 +66,12 @@ def test_tune_keys_match_the_header_and_conftest():
     if not os.path.exists(lsb.library_path()):
         pytest.skip("liblsbsort.so not built")
     from conftest import LIB_DEFAULT_TUNE, apply_session_tune
+    from patterns import TUNE_DEFAULTS
     header = open(os.path.join(ROOT, "include", "lsbsort.h")).read()
     doc = header[header.index("process-wide tunable"):header.index("int lsb_tune(")]
     keys = set(re.findall(r'"([a-z0-9_]+)"', doc))
     assert {"op_t1", "vparts", "ex_u", "pt_direct", "pt_chunks", "pt_variant", "pt_pf_tiles"} <= keys
-    sane = {"op_cfg": 1, "op_t1": 232, "op_nx": 6, "op_lead": 3, "op_hints": 15, "op_persist": 0, "op_ctas_mgpu": 3,
-            "timeout_ms": 4000, "vparts": 16, "vramp": 130, "ex_ctas": 1, "ex_threads": 0, "ex_u": 4}
+    sane = dict(TUNE_DEFAULTS)
     sane.update(LIB_DEFAULT_TUNE)
     assert keys == set(sane), keys ^ set(sane)
     try:
