@@ -19,5 +19,6 @@ from .lsbsort import (  # noqa: F401
     header_symbols,
     library_path,
     load_library,
+    sort_pairs,
     tune,
 )

@@ -13,9 +13,18 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include "lsb_keyorder.cuh"
+
 namespace lsb {
 
 typedef unsigned __int128 u128;
+
+// What a digit is read from: the key itself (uint64 ascending, ORD = false: the kernels compile exactly as without key
+// orders) or order_key(key, korder) (ORD = true: one instantiation serves every order, korder holds its flags).
+template <bool ORD>
+__device__ __forceinline__ uint64_t digit_key(uint64_t k, uint32_t korder) {
+  return ORD ? order_key(k, korder) : k;
+}
 
 struct __align__(16) Elt {
   uint64_t key;
@@ -163,6 +172,7 @@ struct HistArgs {
   int32_t shift[HIST_MAX_SUB];
   uint32_t mask[HIST_MAX_SUB];
   unsigned long long* out;  // [nsub][256], accumulated with atomics (caller zeroes)
+  uint32_t korder;          // key-order flags (ORD instantiations)
 };
 
 template <int NSUB, bool BYTES>
@@ -185,7 +195,7 @@ __device__ __forceinline__ void hist_key(unsigned* sh, uint64_t k, const int* sh
   }
 }
 
-template <int NSUB, bool BYTES>
+template <int NSUB, bool BYTES, bool ORD>
 __global__ void __launch_bounds__(HIST_THREADS) subdigit_hist_kernel(const HistArgs a) {
   __shared__ unsigned sh[NSUB * 256];
   for (int i = threadIdx.x; i < NSUB * 256; i += HIST_THREADS) sh[i] = 0;
@@ -202,13 +212,13 @@ __global__ void __launch_bounds__(HIST_THREADS) subdigit_hist_kernel(const HistA
   for (; (i - lane) + 31 + (U - 1) * stride < a.m; i += U * stride) {
     uint64_t k[U];
 #pragma unroll
-    for (int u = 0; u < U; u++) k[u] = ld_stream_key(a.src + i + u * stride);
+    for (int u = 0; u < U; u++) k[u] = digit_key<ORD>(ld_stream_key(a.src + i + u * stride), a.korder);
 #pragma unroll
     for (int u = 0; u < U; u++) hist_key<NSUB, BYTES>(sh, k[u], shift, mask, 0xffffffffu);
   }
   for (; i < a.m; i += stride) {
     const unsigned active = __activemask();
-    hist_key<NSUB, BYTES>(sh, ld_stream_key(a.src + i), shift, mask, active);
+    hist_key<NSUB, BYTES>(sh, digit_key<ORD>(ld_stream_key(a.src + i), a.korder), shift, mask, active);
   }
   __syncthreads();
   for (int j = threadIdx.x; j < NSUB * 256; j += HIST_THREADS)
@@ -434,28 +444,32 @@ __device__ __forceinline__ RowPlan row_plan(int count) {
   return r;
 }
 
-// 8-bit digit of an element in shared memory; BYTE: the digit is exactly byte `shift / 8` of the key
-template <bool BYTE>
-__device__ __forceinline__ unsigned tile_bin(const Elt* e, int shift, unsigned mask) {
+// 8-bit digit of an element in shared memory; BYTE: the digit is exactly byte `shift / 8` of the key (raw key bits,
+// so never under a key order)
+template <bool BYTE, bool ORD>
+__device__ __forceinline__ unsigned tile_bin(const Elt* e, int shift, unsigned mask, uint32_t korder) {
+  static_assert(!(BYTE && ORD), "the byte path reads the raw key");
   if (BYTE) return reinterpret_cast<const unsigned char*>(e)[shift >> 3];
-  return (unsigned)(e->key >> shift) & mask;
+  return (unsigned)(digit_key<ORD>(e->key, korder) >> shift) & mask;
 }
 
 // Stable ranks, step 1: every element's rank among the elements of its bin that precede it IN ITS
 // WARP's rows (8 ballots per row find the peers; a per-warp counter per bin runs over the rows).
 // On return info[j] = bin | rank << 8 for row j, and the warp's counters hold its counts per bin --
 // no separate counting pass over the tile.  s_whist must be zero on entry.
-template <class C, bool FULL, bool BYTE>
+template <class C, bool FULL, bool BYTE, bool ORD>
 __device__ __forceinline__ void op_rank(const Elt* __restrict__ s_raw, const RowPlan& rp, int shift, unsigned mask,
-                                        unsigned short* __restrict__ s_whist, unsigned (&info)[C::IPT], unsigned& info_p) {
+                                        uint32_t korder, unsigned short* __restrict__ s_whist, unsigned (&info)[C::IPT],
+                                        unsigned& info_p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   unsigned short* wh = s_whist + warp * 256;
   const unsigned lt = lanemask_lt();
   const Elt* row = s_raw + (FULL ? warp * (32 * C::IPT) : rp.row0 * 32) + lane;
   // all digits first: the loads must not sit inside the serial chain of counter updates below
 #pragma unroll
-  for (int j = 0; j < C::IPT; j++) info[j] = (FULL || j < rp.nfull) ? tile_bin<BYTE>(row + j * 32, shift, mask) : 0;
-  info_p = (!FULL && lane < rp.ptail) ? tile_bin<BYTE>(row + rp.nfull * 32, shift, mask) : 0;
+  for (int j = 0; j < C::IPT; j++)
+    info[j] = (FULL || j < rp.nfull) ? tile_bin<BYTE, ORD>(row + j * 32, shift, mask, korder) : 0;
+  info_p = (!FULL && lane < rp.ptail) ? tile_bin<BYTE, ORD>(row + rp.nfull * 32, shift, mask, korder) : 0;
 #pragma unroll
   for (int j = 0; j < C::IPT; j++) {
     if (FULL || j < rp.nfull) {
@@ -564,6 +578,7 @@ struct PartArgs {
   int32_t log_chunks;              // log2 of the number of bulk copies a tile arrives in (pieces of whole warps' rows)
   int64_t d_begin, d_end;
   int32_t pf_tiles;                // L2PF: tile blockIdx.x + pf_tiles is pulled into L2 when this tile starts
+  uint32_t korder;                 // key-order flags (ORD instantiations)
 };
 
 // L2PF (compile-time; lsb_tune "pt_variant" 1 = default, 0 = off): in direct mode the CTA of tile t also starts a bulk
@@ -596,7 +611,7 @@ constexpr int PT_PROF0 = 24, PT_PROF_TILES = 39;
 #endif
 
 // (round 1's kernel, kept as measured: a leaner restatement on the helpers above ran 7 % slower)
-template <class C, bool FULL>
+template <class C, bool FULL, bool ORD>
 __device__ __forceinline__ void partition_tile(const PartArgs& a, unsigned char* smem, uint64_t* s_bar,
                                                unsigned* s_wtot, int tile, int seg, int count, bool first,
                                                int first_tile PT_T_ARG) {
@@ -622,7 +637,7 @@ __device__ __forceinline__ void partition_tile(const PartArgs& a, unsigned char*
     const int idx = idx0 + j * 32;
     bins[j] = 0;
     if (FULL || idx < count) {
-      const unsigned bin = (unsigned)(s_raw[idx].key >> a.shift) & a.mask;
+      const unsigned bin = (unsigned)(digit_key<ORD>(s_raw[idx].key, a.korder) >> a.shift) & a.mask;
       bins[j] = bin;
       atomicAdd(wh32 + (bin >> 1), 1u << ((bin & 1u) * 16));
     }
@@ -734,7 +749,7 @@ __device__ __forceinline__ void partition_tile(const PartArgs& a, unsigned char*
     el.val = 0;
     if (valid) {
       el = s_raw[s_perm[p]];
-      const unsigned bin = (unsigned)(el.key >> a.shift) & a.mask;
+      const unsigned bin = (unsigned)(digit_key<ORD>(el.key, a.korder) >> a.shift) & a.mask;
       const long long g = s_bindst[bin] + p;
       Elt* out;
       if (a.world == 1) {
@@ -770,7 +785,7 @@ __device__ __forceinline__ void partition_issue_load(const PartArgs& a, unsigned
   }
 }
 
-template <class C, bool L2PF>
+template <class C, bool L2PF, bool ORD>
 __global__ void __launch_bounds__(C::THREADS, C::MINB) partition_kernel(const PartArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   __shared__ __align__(8) uint64_t s_bar[PT_MAX_CHUNKS];
@@ -803,9 +818,9 @@ __global__ void __launch_bounds__(C::THREADS, C::MINB) partition_kernel(const Pa
     PT_T(0);
     PT_T(1);
     if (cnt == C::TILE)
-      partition_tile<C, true>(a, smem, s_bar, s_wtot, (int)blockIdx.x, 0, cnt, blockIdx.x == 0, 0 PT_T_PASS);
+      partition_tile<C, true, ORD>(a, smem, s_bar, s_wtot, (int)blockIdx.x, 0, cnt, blockIdx.x == 0, 0 PT_T_PASS);
     else
-      partition_tile<C, false>(a, smem, s_bar, s_wtot, (int)blockIdx.x, 0, cnt, blockIdx.x == 0, 0 PT_T_PASS);
+      partition_tile<C, false, ORD>(a, smem, s_bar, s_wtot, (int)blockIdx.x, 0, cnt, blockIdx.x == 0, 0 PT_T_PASS);
     return;
   }
   if (tid == 0) {
@@ -843,9 +858,9 @@ __global__ void __launch_bounds__(C::THREADS, C::MINB) partition_kernel(const Pa
   PT_T(1);
   const int count = s_count;
   if (count == C::TILE)
-    partition_tile<C, true>(a, smem, s_bar, s_wtot, tile, s_seg, count, s_first, s_first_tile PT_T_PASS);
+    partition_tile<C, true, ORD>(a, smem, s_bar, s_wtot, tile, s_seg, count, s_first, s_first_tile PT_T_PASS);
   else
-    partition_tile<C, false>(a, smem, s_bar, s_wtot, tile, s_seg, count, s_first, s_first_tile PT_T_PASS);
+    partition_tile<C, false, ORD>(a, smem, s_bar, s_wtot, tile, s_seg, count, s_first, s_first_tile PT_T_PASS);
 }
 
 // ------------------------------------------------------------------------------------
@@ -993,12 +1008,13 @@ struct ExchVrArgs {
   int32_t V, next_nb;
   int64_t pstart[17];      // first local index of every destination part (the same cut on every GPU); [V] = per
   unsigned* next_dense;    // [G][V][next_nb]
+  uint32_t korder;         // key-order flags (ORD instantiations)
 };
 
 // EX_THREADS = 512 when the exchange has the SMs to itself or shares them with partition_kernel CTAs that
 // come and go; 256 (12.8 K registers) fits beside three resident CTAs of the persistent one-pass kernel.
 // EX_U = 16-byte elements in flight per thread.
-template <int EX_THREADS, int EX_U>
+template <int EX_THREADS, int EX_U, bool ORD>
 __global__ void __launch_bounds__(EX_THREADS) exchange_vr_kernel(const ExchVrArgs a) {
   __shared__ Elt* s_dst[8];
   __shared__ long long s_lim[8];
@@ -1030,7 +1046,8 @@ __global__ void __launch_bounds__(EX_THREADS) exchange_vr_kernel(const ExchVrArg
     for (int u = 0; u < EX_U; u++) {
       const int64_t i = c0 + u * EX_THREADS + threadIdx.x;
       if (i < a.m) {
-        const unsigned d = (unsigned)(e[u].key >> a.shift) & a.mask;
+        const uint64_t dk = digit_key<ORD>(e[u].key, a.korder);
+        const unsigned d = (unsigned)(dk >> a.shift) & a.mask;
         const long long g = __ldg(a.mybase + d) + (i - __ldg(a.localbase + d));
         int r = 0;
         for (int q = 1; q < a.world; q++) r += (g >= s_lim[q]);
@@ -1039,7 +1056,7 @@ __global__ void __launch_bounds__(EX_THREADS) exchange_vr_kernel(const ExchVrArg
         if (a.has_next) {
           int v = 0;
           for (int q = 1; q < a.V; q++) v += (j >= s_pstart[q]);
-          const unsigned dn = (unsigned)(e[u].key >> a.next_shift) & a.next_mask;
+          const unsigned dn = (unsigned)(dk >> a.next_shift) & a.next_mask;
           const unsigned slot = (unsigned)(r * a.V + v) * (unsigned)a.next_nb + dn;
           // skew: when the whole warp counts into one slot, one lane adds the population count; a thread also
           // holds back a run of equal slots and adds it once (constant digits: one atomic per thread per launch)
@@ -1065,14 +1082,16 @@ __global__ void __launch_bounds__(EX_THREADS) exchange_vr_kernel(const ExchVrArg
 // How many distinct values does digit (shift, mask) take over the first `m` (<= 65 536) elements?  The exchange
 // kernel's fused next-digit count uses one L2 atomic per element, which is only cheap when the digit has thousands
 // of live bins; the host reads this estimate (minimum over the GPUs) to decide per pass.
-__global__ void __launch_bounds__(1024) live_bins_kernel(const Elt* src, int m, int shift, uint32_t mask, unsigned* out) {
+template <bool ORD>
+__global__ void __launch_bounds__(1024) live_bins_kernel(const Elt* src, int m, int shift, uint32_t mask, unsigned* out,
+                                                         uint32_t korder) {
   __shared__ unsigned bits[2048];  // 65 536-bit bitmap
   __shared__ unsigned total;
   for (int i = threadIdx.x; i < 2048; i += 1024) bits[i] = 0;
   if (threadIdx.x == 0) total = 0;
   __syncthreads();
   for (int i = threadIdx.x; i < m; i += 1024) {
-    const unsigned d = (unsigned)(ld_stream_key(src + i) >> shift) & mask;
+    const unsigned d = (unsigned)(digit_key<ORD>(ld_stream_key(src + i), korder) >> shift) & mask;
     atomicOr(&bits[d >> 5], 1u << (d & 31));
   }
   __syncthreads();
@@ -1094,8 +1113,10 @@ __host__ __device__ __forceinline__ uint64_t mix64(uint64_t k, uint64_t v) {
   return x;
 }
 
-// out[0..3] = checksum (sum mix, xor mix, xor key, sum val); out[4] = order violations
-__global__ void __launch_bounds__(256) verify_kernel(const Elt* src, int64_t m, unsigned long long* out) {
+// out[0..3] = checksum of the raw records (sum mix, xor mix, xor key, sum val); out[4] = order violations of
+// (digit_key(key), val)
+template <bool ORD>
+__global__ void __launch_bounds__(256) verify_kernel(const Elt* src, int64_t m, unsigned long long* out, uint32_t korder) {
   uint64_t s = 0, x = 0, xk = 0, sv = 0, bad = 0;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += stride) {
@@ -1104,7 +1125,8 @@ __global__ void __launch_bounds__(256) verify_kernel(const Elt* src, int64_t m, 
     s += h; x ^= h; xk ^= e.key; sv += e.val;
     if (i > 0) {
       const Elt p = ld_stream(src + i - 1);
-      if (p.key > e.key || (p.key == e.key && p.val >= e.val)) bad++;
+      const uint64_t pk = digit_key<ORD>(p.key, korder), ek = digit_key<ORD>(e.key, korder);
+      if (pk > ek || (pk == ek && p.val >= e.val)) bad++;
     }
   }
 #pragma unroll

@@ -104,6 +104,7 @@ struct OnePassArgs {
   unsigned* biglist;    // [nsuper][256]: the segments with more than one sub-tile
   unsigned long long timeout_ns;
   unsigned long long* prof;  // [OP_NPROF] stage clocks (LSB_OP_PROF builds only)
+  uint32_t korder;      // key-order flags (ORD instantiations)
 };
 
 // wait until *p >= want; false on time-out or when another CTA already gave up
@@ -143,14 +144,14 @@ constexpr int OP_NPROF = 40;   // the whole table: 0..23 one-pass kernel, 24..39
 
 // K1 tile body after the tile has landed in shared memory: rank by the low byte, publish the
 // pieces, write the tile sorted by low byte into its place in the supertile scratch.
-template <class C, bool FULL, bool BYTE>
+template <class C, bool FULL, bool BYTE, bool ORD>
 __device__ __forceinline__ void k1_tile(const OnePassArgs& a, const Elt* s_raw, unsigned short* s_perm,
                                         unsigned short* s_whist, unsigned* s_wtot, int count, int s, int slot, int idx,
                                         Elt* xo, uint64_t pol_x) {
   const int tid = threadIdx.x;
   unsigned info[C::IPT], info_p;
   const RowPlan rp = FULL ? RowPlan{0, 0, 0} : row_plan<C>(count);
-  op_rank<C, FULL, BYTE>(s_raw, rp, a.shift, 255u, s_whist, info, info_p);
+  op_rank<C, FULL, BYTE, ORD>(s_raw, rp, a.shift, 255u, a.korder, s_whist, info, info_p);
   __syncthreads();
   if (tid < 256) {
     unsigned tile_count, binstart;
@@ -172,7 +173,7 @@ __device__ __forceinline__ void k1_tile(const OnePassArgs& a, const Elt* s_raw, 
 // of a step are the K1 tiles of supertile `step`, the other 256 are the segments of supertile
 // `step - lead`.  Every dependency of an item points to a smaller ticket, every claimed ticket is
 // held by a running CTA, so the spin-waits below cannot deadlock.
-template <class C, bool BYTE>
+template <class C, bool BYTE, bool ORD>
 __global__ void __launch_bounds__(C::THREADS, C::MINB) onepass_kernel(const OnePassArgs a) {
   extern __shared__ __align__(128) unsigned char smem[];
   Elt* s_raw = reinterpret_cast<Elt*>(smem + C::SMEM_RAW);
@@ -272,8 +273,8 @@ __global__ void __launch_bounds__(C::THREADS, C::MINB) onepass_kernel(const OneP
       parity ^= 1u;
       OP_T(3);  // K1: tile load
       Elt* xo = a.X + (size_t)slot * S + (size_t)idx * C::TILE;
-      if (count == C::TILE) k1_tile<C, true, BYTE>(a, s_raw, s_perm, s_whist, s_wtot, count, s, slot, idx, xo, pol_x);
-      else k1_tile<C, false, BYTE>(a, s_raw, s_perm, s_whist, s_wtot, count, s, slot, idx, xo, pol_x);
+      if (count == C::TILE) k1_tile<C, true, BYTE, ORD>(a, s_raw, s_perm, s_whist, s_wtot, count, s, slot, idx, xo, pol_x);
+      else k1_tile<C, false, BYTE, ORD>(a, s_raw, s_perm, s_whist, s_wtot, count, s, slot, idx, xo, pol_x);
       __syncthreads();
       OP_T(7);  // K1: rank, scan, write
       // completion by warp 0 while the dispatcher already prepares the next item: the tile's X
@@ -389,7 +390,7 @@ __global__ void __launch_bounds__(C::THREADS, C::MINB) onepass_kernel(const OneP
 
           unsigned info[C::IPT], info_p;
           const RowPlan rp = row_plan<C>(count);
-          op_rank<C, false, BYTE>(s_raw, rp, shift_hi, mask_hi, s_whist, info, info_p);
+          op_rank<C, false, BYTE, ORD>(s_raw, rp, shift_hi, mask_hi, a.korder, s_whist, info, info_p);
           __syncthreads();
           OP_T(13);  // K2: rank
           if (s_lastg && tid == 0) st_release_u32(a.free2 + s, 1u);
@@ -446,7 +447,7 @@ __global__ void __launch_bounds__(C::THREADS, C::MINB) onepass_kernel(const OneP
             const int p = k * C::THREADS + tid;
             if (p < count) {
               const Elt el = s_raw[s_perm[p]];
-              st_elt_hint(s_binptr[(unsigned)(el.key >> shift_hi) & mask_hi] + p, el, pol_dst);
+              st_elt_hint(s_binptr[(unsigned)(digit_key<ORD>(el.key, a.korder) >> shift_hi) & mask_hi] + p, el, pol_dst);
             }
           }
           OP_T(20);  // K2: scatter
@@ -498,6 +499,7 @@ struct DigitHistArgs {
   int32_t out_off[DH_MAX_DIGITS];     // first bin of the digit in `out`
   void* out;                          // u64 or u32 bins, caller zeroes
   int32_t out_u32;
+  uint32_t korder;                    // key-order flags (ORD instantiations)
 };
 
 __device__ __forceinline__ void dh_global_add(const DigitHistArgs& a, int bin, unsigned v) {
@@ -516,7 +518,7 @@ __device__ __forceinline__ void dh_add(unsigned* sh, int idx, unsigned c, const 
   }
 }
 
-template <int NDIG>  // digits per role (0 = run-time count)
+template <int NDIG, bool ORD>  // digits per role (0 = run-time count)
 __global__ void __launch_bounds__(DH_THREADS, 1) digit_hist_kernel(const DigitHistArgs a) {
   extern __shared__ __align__(16) unsigned dh_sh[];
   const int role = blockIdx.x % a.nroles;
@@ -538,6 +540,9 @@ __global__ void __launch_bounds__(DH_THREADS, 1) digit_hist_kernel(const DigitHi
       ok[u] = i < a.m;
       k[u] = ok[u] ? ld_stream_key(a.src + i) : 0;
     }
+    // after all U loads: an encode inside the conditional load above makes each load wait for the previous one
+#pragma unroll
+    for (int u = 0; u < U; u++) k[u] = digit_key<ORD>(k[u], a.korder);
     const bool whole = base - threadIdx.x + chunk <= a.m;  // CTA-uniform: no lane is out of range
 #pragma unroll
     for (int u = 0; u < U; u++) {

@@ -225,6 +225,10 @@ int fail(lsb_ctx* c, int code, const std::string& msg) {
 
 inline int64_t div_ceil(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
+constexpr uint32_t KEY_ORDER_FLAGS = LSB_FLAG_KEY_I64 | LSB_FLAG_KEY_F64 | LSB_FLAG_DESCENDING;
+// digits come from order_key(key) (the ORD = true instantiation of every digit-reading kernel), not from the raw key
+inline bool ordered(const lsb_ctx* c) { return (c->cfg.flags & KEY_ORDER_FLAGS) != 0; }
+
 PassPlan plan_pass(const lsb_ctx* c, int digit) {
   PassPlan p;
   p.shift = c->cfg.radix_bits * digit;
@@ -324,6 +328,7 @@ int launch_digit_hist(lsb_ctx* c, const Elt* src, int64_t m, const int* shift, c
     a.m = m;
     a.out = out;
     a.out_u32 = out_u32 ? 1 : 0;
+    a.korder = c->cfg.flags;
     int nd = 0, role = 0, role_bins = 0;
     a.role_first[0] = 0;
     while (first + nd < ndig && nd < DH_MAX_DIGITS) {
@@ -347,14 +352,45 @@ int launch_digit_hist(lsb_ctx* c, const Elt* src, int64_t m, const int* shift, c
       const int groups = (int)std::max<int64_t>(1, std::min<int64_t>(c->num_sms / a.nroles, chunks));
       bool one_each = true;
       for (int r = 0; r < a.nroles; r++) one_each = one_each && (a.role_first[r + 1] - a.role_first[r] == 1);
-      if (one_each) digit_hist_kernel<1><<<groups * a.nroles, DH_THREADS, DH_SMEM, c->stream>>>(a);
-      else digit_hist_kernel<0><<<groups * a.nroles, DH_THREADS, DH_SMEM, c->stream>>>(a);
+      const int grid = groups * a.nroles;
+      if (ordered(c)) {
+        if (one_each) digit_hist_kernel<1, true><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
+        else digit_hist_kernel<0, true><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
+      } else {
+        if (one_each) digit_hist_kernel<1, false><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
+        else digit_hist_kernel<0, false><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
+      }
       c->launches++;
       CU(c, cudaGetLastError());
     }
     first += nd;
   }
   return LSB_OK;
+}
+
+template <bool ORD>
+void launch_subdigit_hist_kernel(const HistArgs& a, int grid, bool bytes, cudaStream_t stream) {
+#define LSB_HIST(N, B) subdigit_hist_kernel<N, B, ORD><<<grid, HIST_THREADS, 0, stream>>>(a)
+  if (bytes && a.nsub == 8) LSB_HIST(8, true);
+  else switch (a.nsub) {
+    case 1: LSB_HIST(1, false); break;
+    case 2: LSB_HIST(2, false); break;
+    case 3: LSB_HIST(3, false); break;
+    case 4: LSB_HIST(4, false); break;
+    case 5: LSB_HIST(5, false); break;
+    case 6: LSB_HIST(6, false); break;
+    case 7: LSB_HIST(7, false); break;
+    case 8: LSB_HIST(8, false); break;
+    case 9: LSB_HIST(9, false); break;
+    case 10: LSB_HIST(10, false); break;
+    case 11: LSB_HIST(11, false); break;
+    case 12: LSB_HIST(12, false); break;
+    case 13: LSB_HIST(13, false); break;
+    case 14: LSB_HIST(14, false); break;
+    case 15: LSB_HIST(15, false); break;
+    default: LSB_HIST(16, false); break;
+  }
+#undef LSB_HIST
 }
 
 // 256-bin histograms of up to HIST_MAX_SUB sub-digits in one read + their exclusive scans (two-step shape)
@@ -371,30 +407,12 @@ int launch_subdigit_hist(lsb_ctx* c, const Elt* src, const SubPass* subs, int ns
       a.mask[s] = (1u << subs[s].bits) - 1;
     }
     a.out = c->hist;
+    a.korder = c->cfg.flags;
     const int grid = (int)std::min<int64_t>((int64_t)c->num_sms * 4, div_ceil(c->here, HIST_THREADS));
     bool bytes = true;  // sub-digits are exactly bytes 0..nsub-1 of the key (radix 8 and 16)
     for (int s = 0; s < nsub; s++) bytes = bytes && subs[s].shift == 8 * s && subs[s].bits == 8;
-#define LSB_HIST(N, B) subdigit_hist_kernel<N, B><<<grid, HIST_THREADS, 0, c->stream>>>(a)
-    if (bytes && nsub == 8) LSB_HIST(8, true);
-    else switch (nsub) {
-      case 1: LSB_HIST(1, false); break;
-      case 2: LSB_HIST(2, false); break;
-      case 3: LSB_HIST(3, false); break;
-      case 4: LSB_HIST(4, false); break;
-      case 5: LSB_HIST(5, false); break;
-      case 6: LSB_HIST(6, false); break;
-      case 7: LSB_HIST(7, false); break;
-      case 8: LSB_HIST(8, false); break;
-      case 9: LSB_HIST(9, false); break;
-      case 10: LSB_HIST(10, false); break;
-      case 11: LSB_HIST(11, false); break;
-      case 12: LSB_HIST(12, false); break;
-      case 13: LSB_HIST(13, false); break;
-      case 14: LSB_HIST(14, false); break;
-      case 15: LSB_HIST(15, false); break;
-      default: LSB_HIST(16, false); break;
-    }
-#undef LSB_HIST
+    if (ordered(c)) launch_subdigit_hist_kernel<true>(a, grid, bytes, c->stream);
+    else launch_subdigit_hist_kernel<false>(a, grid, bytes, c->stream);
     c->launches++;
   }
   CU(c, cudaGetLastError());
@@ -457,13 +475,18 @@ int launch_partition(lsb_ctx* c, const Elt* src, int64_t m, int shift, int bits,
   a.d_begin = 0;
   a.d_end = m;
   a.pf_tiles = g_tune.pt_pf_tiles > 0 ? g_tune.pt_pf_tiles : std::max(1, c->num_sms / 2);
+  a.korder = c->cfg.flags;
   c->part_elems += m;
   if (m > 0) {
     const unsigned grid = (unsigned)div_ceil(m, c->tile);
-    if (a.direct && g_tune.pt_variant)  // the prefetch needs blockIdx-ordered tiles
-      partition_kernel<TileCfg, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
-    else
-      partition_kernel<TileCfg, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+    const bool l2pf = a.direct && g_tune.pt_variant;  // the prefetch needs blockIdx-ordered tiles
+    if (ordered(c)) {
+      if (l2pf) partition_kernel<TileCfg, true, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      else partition_kernel<TileCfg, false, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+    } else {
+      if (l2pf) partition_kernel<TileCfg, true, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      else partition_kernel<TileCfg, false, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+    }
     c->launches++;
   }
   CU(c, cudaGetLastError());
@@ -520,17 +543,20 @@ int launch_onepass(lsb_ctx* c, const Elt* src, Elt* dst, int64_t m, int shift, i
     a.biglist = ctl + o_biglist;
     a.timeout_ns = (unsigned long long)c->tune.timeout_ms * 1000000ULL;
     a.prof = c->op_prof;
+    a.korder = c->cfg.flags;
     const int per_sm = ctas_per_sm > 0 ? std::min(ctas_per_sm, c->op_resident) : c->op_resident;
     // every claimed item must belong to a resident CTA: never launch more CTAs than fit
     const int64_t useful = div_ceil(m, c->op_tile) + 256;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)c->num_sms * per_sm, useful));
     const bool byte = (shift % 8) == 0 && bits == 16;  // both digit halves are whole bytes of the key
     if (c->tune.op_cfg == 1) {
-      if (byte) onepass_kernel<TileCfgS, true><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
-      else onepass_kernel<TileCfgS, false><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
+      if (ordered(c)) onepass_kernel<TileCfgS, false, true><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
+      else if (byte) onepass_kernel<TileCfgS, true, false><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
+      else onepass_kernel<TileCfgS, false, false><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
     } else {
-      if (byte) onepass_kernel<TileCfg, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
-      else onepass_kernel<TileCfg, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      if (ordered(c)) onepass_kernel<TileCfg, false, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      else if (byte) onepass_kernel<TileCfg, true, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      else onepass_kernel<TileCfg, false, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
     }
     c->launches += 2;
     CU(c, cudaGetLastError());
@@ -637,7 +663,9 @@ int plan_fusion(lsb_ctx* c) {
   const int m = (int)std::min<int64_t>(c->here, 65536);
   for (int p = 0; p < c->npasses; p++) {
     const PassPlan q = plan_pass(c, p);
-    live_bins_kernel<<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, (uint32_t)((1u << q.bits) - 1), d + p);
+    const uint32_t mask = (uint32_t)((1u << q.bits) - 1);
+    if (ordered(c)) live_bins_kernel<true><<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, mask, d + p, c->cfg.flags);
+    else live_bins_kernel<false><<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, mask, d + p, 0);
     c->launches++;
   }
   CU(c, cudaGetLastError());
@@ -747,13 +775,20 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
     x.next_nb = next_nb;
     for (int i = 0; i <= LSB_MAX_PARTS; i++) x.pstart[i] = c->pstart[std::min(i, V)];
     x.next_dense = c->next_dense;
+    x.korder = c->cfg.flags;
     // 512 threads next to partition_kernel CTAs that come and go; 256 fit beside three resident one-pass CTAs
     const int ex_threads = c->tune.ex_threads ? c->tune.ex_threads : ((c->cfg.flags & LSB_FLAG_ONE_PASS) ? 256 : 512);
     const int ex_u = c->tune.ex_u == 8 ? 8 : 4;
     const int grid = (int)std::min<int64_t>((int64_t)c->num_sms * c->tune.ex_ctas, div_ceil(m, (int64_t)ex_threads * ex_u));
-    if (ex_threads == 256) exchange_vr_kernel<256, 4><<<grid, 256, 0, c->xstream>>>(x);
-    else if (ex_u == 8) exchange_vr_kernel<512, 8><<<grid, 512, 0, c->xstream>>>(x);
-    else exchange_vr_kernel<512, 4><<<grid, 512, 0, c->xstream>>>(x);
+    if (ordered(c)) {
+      if (ex_threads == 256) exchange_vr_kernel<256, 4, true><<<grid, 256, 0, c->xstream>>>(x);
+      else if (ex_u == 8) exchange_vr_kernel<512, 8, true><<<grid, 512, 0, c->xstream>>>(x);
+      else exchange_vr_kernel<512, 4, true><<<grid, 512, 0, c->xstream>>>(x);
+    } else {
+      if (ex_threads == 256) exchange_vr_kernel<256, 4, false><<<grid, 256, 0, c->xstream>>>(x);
+      else if (ex_u == 8) exchange_vr_kernel<512, 8, false><<<grid, 512, 0, c->xstream>>>(x);
+      else exchange_vr_kernel<512, 4, false><<<grid, 512, 0, c->xstream>>>(x);
+    }
     c->launches++;
     CU(c, cudaGetLastError());
     if (timed) {
@@ -935,6 +970,8 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   if (cfg->n < 0 || cfg->world_size < 1 || cfg->world_size > LSB_MAX_GPUS || cfg->world_rank < 0 ||
       cfg->world_rank >= cfg->world_size || cfg->radix_bits < 1 || cfg->radix_bits > 16 || cfg->ranks < 0)
     return fail(nullptr, LSB_ERR_ARG, "bad lsb_config (n >= 0, 1 <= world_size <= 8, 1 <= radix_bits <= 16)");
+  if ((cfg->flags & LSB_FLAG_KEY_I64) && (cfg->flags & LSB_FLAG_KEY_F64))
+    return fail(nullptr, LSB_ERR_ARG, "bad lsb_config: LSB_FLAG_KEY_I64 and LSB_FLAG_KEY_F64 exclude each other");
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -995,27 +1032,34 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   CUC(cudaMalloc(&c->counts_all, sizeof(unsigned long long) * 65536 * c->G));
   CUC(cudaMalloc(&c->mybase, sizeof(int64_t) * 65536));
   // one-pass kernel: supertile scratch, piece table, control block, frontier table
-#define LSB_PT_ATTR(V)                                                                                                     \
-  CUC(cudaFuncSetAttribute(partition_kernel<TileCfg, V>, cudaFuncAttributeMaxDynamicSharedMemorySize, TileCfg::SMEM));     \
-  CUC(cudaFuncSetAttribute(partition_kernel<TileCfg, V>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-  LSB_PT_ATTR(false)
-  LSB_PT_ATTR(true)
+#define LSB_PT_ATTR(V, O)                                                                                                     \
+  CUC(cudaFuncSetAttribute(partition_kernel<TileCfg, V, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, TileCfg::SMEM));     \
+  CUC(cudaFuncSetAttribute(partition_kernel<TileCfg, V, O>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+  LSB_PT_ATTR(false, false)
+  LSB_PT_ATTR(true, false)
+  LSB_PT_ATTR(false, true)
+  LSB_PT_ATTR(true, true)
 #undef LSB_PT_ATTR
-#define LSB_OP_ATTR(CFG, B)                                                                                       \
-  CUC(cudaFuncSetAttribute(onepass_kernel<CFG, B>, cudaFuncAttributeMaxDynamicSharedMemorySize, CFG::SMEM));     \
-  CUC(cudaFuncSetAttribute(onepass_kernel<CFG, B>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-  LSB_OP_ATTR(TileCfg, true)
-  LSB_OP_ATTR(TileCfg, false)
-  LSB_OP_ATTR(TileCfgS, true)
-  LSB_OP_ATTR(TileCfgS, false)
+#define LSB_OP_ATTR(CFG, B, O)                                                                                       \
+  CUC(cudaFuncSetAttribute(onepass_kernel<CFG, B, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, CFG::SMEM));     \
+  CUC(cudaFuncSetAttribute(onepass_kernel<CFG, B, O>, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+  LSB_OP_ATTR(TileCfg, true, false)
+  LSB_OP_ATTR(TileCfg, false, false)
+  LSB_OP_ATTR(TileCfgS, true, false)
+  LSB_OP_ATTR(TileCfgS, false, false)
+  LSB_OP_ATTR(TileCfg, false, true)
+  LSB_OP_ATTR(TileCfgS, false, true)
 #undef LSB_OP_ATTR
-  CUC(cudaFuncSetAttribute(digit_hist_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
-  CUC(cudaFuncSetAttribute(digit_hist_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
+  CUC(cudaFuncSetAttribute(digit_hist_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
+  CUC(cudaFuncSetAttribute(digit_hist_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
+  CUC(cudaFuncSetAttribute(digit_hist_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
+  CUC(cudaFuncSetAttribute(digit_hist_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
+  // every claimed one-pass item must belong to a resident CTA: residency of the instantiation this context launches
   if (c->tune.op_cfg == 1) {
     c->op_tile = TileCfgS::TILE;
-    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, onepass_kernel<TileCfgS, true>, TileCfgS::THREADS, TileCfgS::SMEM));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, ordered(c) ? onepass_kernel<TileCfgS, false, true> : onepass_kernel<TileCfgS, true, false>, TileCfgS::THREADS, TileCfgS::SMEM));
   } else {
-    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, onepass_kernel<TileCfg, true>, TileCfg::THREADS, TileCfg::SMEM));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, ordered(c) ? onepass_kernel<TileCfg, false, true> : onepass_kernel<TileCfg, true, false>, TileCfg::THREADS, TileCfg::SMEM));
   }
   if (c->tune.op_persist > 0) {
     int max_persist = 0;
@@ -1388,7 +1432,8 @@ static int local_verify(lsb_ctx* c) {
   CU(c, cudaMemsetAsync(c->small + 40, 0, 8 * sizeof(unsigned long long), c->stream));
   if (c->here > 0) {
     int grid = (int)std::min<int64_t>((int64_t)c->num_sms * 8, div_ceil(c->here, 256));
-    verify_kernel<<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40);
+    if (ordered(c)) verify_kernel<true><<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40, c->cfg.flags);
+    else verify_kernel<false><<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40, 0);
     CU(c, cudaGetLastError());
   }
   return LSB_OK;
@@ -1439,8 +1484,9 @@ int lsb_verify_device(lsb_ctx* c, lsb_verify* out) {
     out->order_violations += (int64_t)r[4];
     out->elements += (int64_t)r[5];
     if (r[5] == 0) continue;
-    if (have_prev && (pk > r[6] || (pk == r[6] && pv >= r[7]))) out->order_violations++;
-    pk = r[8];
+    const uint64_t fk = order_key(r[6], c->cfg.flags);
+    if (have_prev && (pk > fk || (pk == fk && pv >= r[7]))) out->order_violations++;
+    pk = order_key(r[8], c->cfg.flags);
     pv = r[9];
     have_prev = true;
   }

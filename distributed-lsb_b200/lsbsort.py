@@ -28,6 +28,11 @@ FLAG_PHASE_EVENTS = 1
 FLAG_TWO_LEVEL = 2
 FLAG_ONE_PASS = 4
 FLAG_NO_SKIP = 8
+# key orders (include/lsbsort.h): the sort is stable and ascending by order_key(key); key bits are never rewritten
+FLAG_KEY_I64 = 16
+FLAG_KEY_F64 = 32
+FLAG_DESCENDING = 64
+KEY_DTYPE_FLAGS = {np.dtype(np.uint64): 0, np.dtype(np.int64): FLAG_KEY_I64, np.dtype(np.float64): FLAG_KEY_F64}
 
 
 class LsbError(RuntimeError):
@@ -273,3 +278,27 @@ class DistributedSorter:
         if rc and (raise_on_failure or rc != -6):
             self._check(rc, "lsb_verify_device")
         return v
+
+
+def sort_pairs(keys, vals=None, descending=False, device=0):
+    """Stable sort of a 1-D numpy array of uint64, int64 or float64 keys, with 8-byte `vals` (default arange(n) as int64,
+    so the returned vals are the stable argsort), on one GPU through sort_host.  The order is numpy's and torch's: NaNs
+    last (first when descending), -0.0 == +0.0, equal keys in input order.  Returns (keys, vals) in the input dtypes;
+    the records are permuted, never rewritten (-0.0 and NaN payloads come back as they went in)."""
+    keys = np.ascontiguousarray(keys)
+    if keys.dtype not in KEY_DTYPE_FLAGS:
+        raise TypeError(f"sort_pairs: keys must be uint64, int64 or float64, not {keys.dtype}")
+    vals = np.arange(len(keys), dtype=np.int64) if vals is None else np.ascontiguousarray(vals)
+    if keys.ndim != 1 or vals.shape != keys.shape:
+        raise ValueError(f"sort_pairs: keys and vals must be 1-D of one length, not {keys.shape} and {vals.shape}")
+    if vals.dtype.itemsize != 8:
+        raise TypeError(f"sort_pairs: vals must have an 8-byte dtype, not {vals.dtype}")
+    n = len(keys)
+    recs = np.empty(n, dtype=ELT)
+    recs["key"] = keys.view(np.uint64)
+    recs["val"] = vals.view(np.uint64)
+    out = np.empty(n, dtype=ELT)
+    flags = KEY_DTYPE_FLAGS[keys.dtype] | (FLAG_DESCENDING if descending else 0)
+    with DistributedSorter(n, ranks=1, device=device, flags=flags) as s:
+        s.sort_host(recs, out)
+    return out["key"].view(keys.dtype).copy(), out["val"].view(vals.dtype).copy()

@@ -93,6 +93,26 @@ typedef struct lsb_config {
                                     (a stable pass on a constant digit is the identity; the
                                     reference always runs it; chpl passes nBits for the same
                                     purpose, chpl/arkouda-radix-sort.chpl:70,78)              */
+/*
+ * Key orders.  Without a type flag the key is a uint64, sorted ascending.  The result of every
+ * sort is "stable, ascending by order_key(key)", where
+ *   uint64:            order_key(k) = k
+ *   LSB_FLAG_KEY_I64:  order_key(k) = k ^ 2^63                 (two's-complement int64)
+ *   LSB_FLAG_KEY_F64:  -0.0 is first read as +0.0; any NaN (exponent all ones, mantissa != 0,
+ *                      either sign) maps to ~0; every other value k to k ^ (sign ? ~0 : 2^63)
+ *   LSB_FLAG_DESCENDING (with either type flag or neither): ~order_key_ascending(k)
+ * That is the order of np.argsort(x, kind="stable") and torch.sort(x, stable=True[, descending=True]):
+ * NaNs last ascending and first descending, -0.0 == +0.0, equal keys in input order (for G > 1:
+ * global index order, also descending).  The sort never rewrites key bits: the output holds the
+ * input's records permuted (-0.0 stays -0.0, NaN payloads survive), so lsb_checksum is unchanged.
+ * lsb_histogram, lsb_starts and lsb_pass count and move by the digits of order_key(key), a pass
+ * whose digit of order_key is constant is skipped, and lsb_verify_device checks that
+ * (order_key(key), val) strictly increases.  KEY_I64 | KEY_F64 together: LSB_ERR_ARG from lsb_create.
+ * Definition: distributed-lsb_b200/csrc/lsb_keyorder.cuh.
+ */
+#define LSB_FLAG_KEY_I64 16u     /* key is a two's-complement int64                             */
+#define LSB_FLAG_KEY_F64 32u     /* key is an IEEE-754 binary64                                 */
+#define LSB_FLAG_DESCENDING 64u  /* largest first                                               */
 
 /* what lsb_sort / lsb_pass measured, device time from CUDA events on the sort stream */
 typedef struct lsb_stats {
@@ -114,7 +134,7 @@ typedef struct lsb_stats {
 } lsb_stats;
 
 typedef struct lsb_verify {
-  int64_t order_violations;  /* i with (key,val)[i-1] >= (key,val)[i], within and across shards */
+  int64_t order_violations;  /* i with (order_key(key),val)[i-1] >= (...)[i], within and across shards */
   int64_t elements;          /* global element count seen                                   */
   uint64_t checksum[4];      /* global multiset hash, see lsb_checksum                      */
 } lsb_verify;
@@ -185,12 +205,14 @@ int lsb_host_free(void* ptr);
 
 /* ---- the hot path ---------------------------------------------------------------- */
 
-/* mySort (:580-585): all ceil(64/radix_bits) passes, least significant digit first;
- * on return the shard holds its slice of the globally, stably sorted array.
+/* mySort (:580-585): all ceil(64/radix_bits) passes, least significant digit first, on the digits
+ * of order_key(key) (see the key orders above); on return the shard holds its slice of the
+ * globally, stably sorted array.
  * Collective: every process must call it.  stats may be NULL. */
 int lsb_sort(lsb_ctx* ctx, lsb_stats* stats);
 
-/* globalShuffle(A, B, digit) (:481-577): one stable pass on digit `digit`. Collective. */
+/* globalShuffle(A, B, digit) (:481-577): one stable pass on digit `digit` of order_key(key).
+ * Collective. */
 int lsb_pass(lsb_ctx* ctx, int digit, lsb_stats* stats);
 
 /* host-buffer form of mySort for one process: upload `count` elements (must equal
@@ -201,9 +223,10 @@ int lsb_sort_host(lsb_ctx* ctx, const lsb_elt* host_in, lsb_elt* host_out, int64
 
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
-/* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard */
+/* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard; d is the
+ * digit of order_key(key) */
 int lsb_histogram(lsb_ctx* ctx, int digit, int64_t* host_counts);
-/* starts[d]: global output index of the first of MY elements whose digit is d, i.e.
+/* starts[d]: global output index of the first of MY elements whose digit (of order_key(key)) is d, i.e.
  * GlobalStarts[d*R + myRank] after copyCountsToGlobalCounts + exclusiveScan +
  * copyStartsFromGlobalStarts (:519-525; order defined at :350). Collective. */
 int lsb_starts(lsb_ctx* ctx, int digit, int64_t* host_starts);
@@ -219,8 +242,8 @@ int lsb_digit_bits(const lsb_ctx* ctx, int digit);
  * out[0] = sum mix(key,val), out[1] = xor mix(key,val), out[2] = xor key, out[3] = sum val */
 int lsb_checksum(lsb_ctx* ctx, uint64_t out[4]);
 
-/* Collective.  Checks that (key,val) is strictly increasing inside every shard and
- * across shard boundaries, and returns the global multiset hash.  Because val is the
+/* Collective.  Checks that (order_key(key),val) is strictly increasing inside every shard and
+ * across shard boundaries, and returns the global multiset hash (of the raw key bits).  Because val is the
  * unique original index (:654), "strictly increasing in (key,val) and same multiset as
  * the input" is equivalent to "equals std::stable_sort by key of the input" (:722-726).
  * Returns LSB_ERR_VERIFY if order_violations != 0. */
