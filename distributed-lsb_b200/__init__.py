@@ -20,5 +20,6 @@ from .lsbsort import (  # noqa: F401
     library_path,
     load_library,
     sort_pairs,
+    sort_tensor,
     tune,
 )

@@ -25,6 +25,7 @@
 #include "../../include/lsbsort.h"
 #include "lsb_kernels.cuh"
 #include "lsb_onepass.cuh"
+#include "lsb_io.cuh"
 
 #include <nccl.h>  // types only: the library itself is bound at run time, see NcclApi
 #include <dlfcn.h>
@@ -156,6 +157,7 @@ struct lsb_ctx {
   ncclComm_t comm = nullptr;
   bool comm_ready = false;
   cudaEvent_t ev_start = nullptr, ev_stop = nullptr;
+  cudaEvent_t ev_caller = nullptr;  // lsb_sort_device: the caller's stream up to the call
   std::vector<cudaEvent_t> phase_ev;
   std::vector<int> phase_kind;  // 0 count, 1 scan/collective, 2 scatter (one-pass / partition), 3 exchange
   int64_t launches = 0;
@@ -906,6 +908,54 @@ int check_ready(lsb_ctx* c) {
   return LSB_OK;
 }
 
+// ---- lsb_sort_device: the caller's arrays <-> the shard's records --------------------------------------------------------
+
+inline bool ranges_overlap(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
+  const uintptr_t x = (uintptr_t)a, y = (uintptr_t)b;
+  return x < y + b_bytes && y < x + a_bytes;
+}
+
+// NULL or 8-byte-aligned device memory of this context's device that is not one of its own shards
+int check_device_array(lsb_ctx* c, const void* p, const char* name, int64_t count) {
+  if (!p) return LSB_OK;
+  if ((uintptr_t)p & 7) return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not 8-byte aligned");
+  cudaPointerAttributes at;
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
+    cudaGetLastError();  // not sticky: clear it so that the next launch check does not report it
+    return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not CUDA memory");
+  }
+  if (at.type != cudaMemoryTypeDevice || at.device != c->cfg.device)
+    return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not device memory of device " +
+                                    std::to_string(c->cfg.device));
+  const size_t shard_bytes = (size_t)std::max<int64_t>(c->per, 1) * sizeof(Elt);
+  for (int b = 0; b < 2; b++)
+    if (ranges_overlap(p, (size_t)count * sizeof(uint64_t), c->buf[b], shard_bytes))
+      return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " overlaps the context's own shards");
+  return LSB_OK;
+}
+
+int io_grid(const lsb_ctx* c, int64_t count) {
+  return (int)std::min<int64_t>((int64_t)c->num_sms * IO_CTAS_PER_SM, div_ceil(count, IO_THREADS));
+}
+
+int launch_pack(lsb_ctx* c, const uint64_t* keys, const uint64_t* vals) {
+  const PackArgs a{keys, vals, c->buf[0], c->here, c->first};
+  if (vals) pack_kernel<true><<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+  else pack_kernel<false><<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+int launch_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals) {
+  const UnpackArgs a{c->buf[c->cur], keys, vals, c->here};
+  const int grid = io_grid(c, c->here);
+  if (keys && vals) unpack_kernel<true, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
+  else if (keys) unpack_kernel<true, false><<<grid, IO_THREADS, 0, c->stream>>>(a);
+  else unpack_kernel<false, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1012,6 +1062,7 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   CUC(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   CUC(cudaEventCreate(&c->ev_start));
   CUC(cudaEventCreate(&c->ev_stop));
+  CUC(cudaEventCreateWithFlags(&c->ev_caller, cudaEventDisableTiming));
   const size_t shard_bytes = (size_t)std::max<int64_t>(c->per, 1) * sizeof(Elt);
   CUC(cudaMalloc(&c->buf[0], shard_bytes));
   CUC(cudaMalloc(&c->buf[1], shard_bytes));
@@ -1187,6 +1238,7 @@ void lsb_destroy(lsb_ctx* c) {
   if (c->host_skip) cudaFreeHost(c->host_skip);
   if (c->ev_start) cudaEventDestroy(c->ev_start);
   if (c->ev_stop) cudaEventDestroy(c->ev_stop);
+  if (c->ev_caller) cudaEventDestroy(c->ev_caller);
   if (c->stream) cudaStreamDestroy(c->stream);
   delete c;
 }
@@ -1364,6 +1416,32 @@ int lsb_sort_host(lsb_ctx* c, const lsb_elt* host_in, lsb_elt* host_out, int64_t
   if (count) CU(c, cudaMemcpyAsync(c->buf[0], host_in, (size_t)count * sizeof(Elt), cudaMemcpyHostToDevice, c->stream));
   if ((rc = lsb_sort(c, st))) return rc;
   if (count) CU(c, cudaMemcpyAsync(host_out, c->buf[c->cur], (size_t)count * sizeof(Elt), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaStreamSynchronize(c->stream));
+  return LSB_OK;
+}
+
+int lsb_sort_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out, uint64_t* vals_out,
+                    int64_t count, void* stream, lsb_stats* st) {
+  int rc = check_ready(c);
+  if (rc) return rc;
+  if (count != c->here) return fail(c, LSB_ERR_ARG, "lsb_sort_device: count must equal this shard's size");
+  CU(c, cudaSetDevice(c->cfg.device));
+  if (count) {
+    if (!keys_in) return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_in is NULL");
+    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_out and vals_out are both NULL");
+    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
+    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
+    for (int i = 0; i < 4; i++)
+      if ((rc = check_device_array(c, ptrs[i], names[i], count))) return rc;
+    if (keys_out && vals_out && ranges_overlap(keys_out, (size_t)count * sizeof(uint64_t), vals_out, (size_t)count * sizeof(uint64_t)))
+      return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_out and vals_out overlap");
+  }
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  c->cur = 0;
+  if (count && (rc = launch_pack(c, keys_in, vals_in))) return rc;
+  if ((rc = lsb_sort(c, st))) return rc;
+  if (count && (rc = launch_unpack(c, keys_out, vals_out))) return rc;
   CU(c, cudaStreamSynchronize(c->stream));
   return LSB_OK;
 }

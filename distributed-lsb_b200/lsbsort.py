@@ -107,6 +107,7 @@ def load_library():
     L.lsb_sort.argtypes = [vp, ctypes.POINTER(Stats)]
     L.lsb_pass.argtypes = [vp, ci, ctypes.POINTER(Stats)]
     L.lsb_sort_host.argtypes = [vp, vp, vp, i64, ctypes.POINTER(Stats)]
+    L.lsb_sort_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, ctypes.POINTER(Stats)]
     L.lsb_histogram.argtypes = [vp, ci, vp]
     L.lsb_starts.argtypes = [vp, ci, vp]
     L.lsb_num_passes.argtypes = [vp]
@@ -176,6 +177,7 @@ class DistributedSorter:
         self.n, self.world_size, self.world_rank = n, world_size, world_rank
         self.per, self.here, self.first_global = per.value, here.value, first.value
         self.radix_bits = radix_bits
+        self.device, self.flags = device, flags
 
     create = classmethod(lambda cls, *a, **k: cls(*a, **k))
 
@@ -249,6 +251,39 @@ class DistributedSorter:
                                           ctypes.byref(st)), "lsb_sort_host")
         return st
 
+    def sort_device(self, keys, vals=None, keys_out=None, vals_out=None, stream=None):
+        """CUDA tensors in, CUDA tensors out, no host copy (lsb_sort_device).  `keys`: 1-D contiguous uint64, int64 or
+        float64 tensor of `here` elements on this sorter's device, of the dtype its key-type flags name; `vals`: the same
+        shape with any 8-byte dtype, or None for the global input index (torch.int64: the stable argsort).  keys_out /
+        vals_out: a tensor to write (may be the input itself: in place), None to allocate one, False for none (not
+        both).  The library waits for the work queued on `stream` (default: the current stream) before it reads the
+        inputs and returns when the outputs are written.  Returns (keys_out, vals_out, Stats of the sort itself)."""
+        torch = _torch()
+        n = self.here
+        if keys_out is False and vals_out is False:
+            raise ValueError("sort_device: keys_out and vals_out cannot both be False")
+        _check_vector(torch, keys, "keys", n, self.device, key_flags=self.flags & (FLAG_KEY_I64 | FLAG_KEY_F64))
+        if vals is not None:
+            _check_vector(torch, vals, "vals", n, self.device)
+        if keys_out is None:
+            keys_out = torch.empty_like(keys)
+        elif keys_out is not False:
+            _check_vector(torch, keys_out, "keys_out", n, self.device)
+            if keys_out.dtype != keys.dtype:
+                raise TypeError(f"sort_device: keys_out must have the keys' dtype {keys.dtype}, not {keys_out.dtype}")
+        if vals_out is None:
+            vals_out = torch.empty_like(vals) if vals is not None else torch.empty(n, dtype=torch.int64, device=keys.device)
+        elif vals_out is not False:
+            _check_vector(torch, vals_out, "vals_out", n, self.device)
+        if stream is None:
+            stream = torch.cuda.current_stream(keys.device)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        ptr = lambda t: t.data_ptr() if t is not None and t is not False else None  # noqa: E731
+        st = Stats()
+        self._check(self._L.lsb_sort_device(self._ctx, ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out), n, handle,
+                                            ctypes.byref(st)), "lsb_sort_device")
+        return (keys_out if keys_out is not False else None), (vals_out if vals_out is not False else None), st
+
     # -- test hooks -----------------------------------------------------------------------
     def num_passes(self):
         return self._L.lsb_num_passes(self._ctx)
@@ -302,3 +337,61 @@ def sort_pairs(keys, vals=None, descending=False, device=0):
     with DistributedSorter(n, ranks=1, device=device, flags=flags) as s:
         s.sort_host(recs, out)
     return out["key"].view(keys.dtype).copy(), out["val"].view(vals.dtype).copy()
+
+
+def _torch():
+    import torch  # only the tensor entry points need it
+    return torch
+
+
+def _key_dtype_flags(torch):
+    return {torch.uint64: 0, torch.int64: FLAG_KEY_I64, torch.float64: FLAG_KEY_F64}
+
+
+def _check_vector(torch, t, name, n=None, device=None, key_flags=None):
+    """TypeError / ValueError unless `t` is a 1-D contiguous CUDA tensor of 8-byte elements (of n elements on `device`,
+    and of the key dtype that `key_flags` names, when given)"""
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name} must be a torch.Tensor, not {type(t).__name__}")
+    if key_flags is not None:
+        dtypes = _key_dtype_flags(torch)
+        if t.dtype not in dtypes:
+            raise TypeError(f"{name} must be torch.uint64, int64 or float64, not {t.dtype}")
+        if dtypes[t.dtype] != key_flags:
+            raise TypeError(f"{name}: dtype {t.dtype} does not match the sorter's key-type flags ({key_flags})")
+    elif t.element_size() != 8:
+        raise TypeError(f"{name} must have an 8-byte dtype, not {t.dtype}")
+    if t.dim() != 1:
+        raise ValueError(f"{name} must be 1-D, not of shape {tuple(t.shape)}")
+    if not t.is_contiguous():
+        raise ValueError(f"{name} must be contiguous")
+    if n is not None and t.numel() != n:
+        raise ValueError(f"{name} has {t.numel()} elements, the shard {n}")
+    if not t.is_cuda:
+        raise ValueError(f"{name} must be a CUDA tensor, not on {t.device}")
+    if device is not None and t.device.index != device:
+        raise ValueError(f"{name} is on {t.device}, the sorter on cuda:{device}")
+
+
+def sort_tensor(keys, vals=None, descending=False):
+    """torch.sort(keys, stable=True, descending=descending) for a 1-D CUDA tensor of uint64, int64 or float64 keys, on
+    that tensor's GPU, with no host copy: returns (sorted keys, vals permuted the same way), or (sorted keys, int64
+    indices) without vals.  The order is torch's and numpy's: NaNs last (first when descending), -0.0 == +0.0, equal
+    keys in input order; key bits are never rewritten.  Makes a one-GPU sorter for the call."""
+    torch = _torch()
+    if not isinstance(keys, torch.Tensor):
+        raise TypeError(f"keys must be a torch.Tensor, not {type(keys).__name__}")
+    dtypes = _key_dtype_flags(torch)
+    if keys.dtype not in dtypes:
+        raise TypeError(f"keys must be torch.uint64, int64 or float64, not {keys.dtype}")
+    keys = keys.contiguous()
+    _check_vector(torch, keys, "keys", key_flags=dtypes[keys.dtype])
+    if vals is not None:
+        if not isinstance(vals, torch.Tensor):
+            raise TypeError(f"vals must be a torch.Tensor, not {type(vals).__name__}")
+        vals = vals.contiguous()
+        _check_vector(torch, vals, "vals", keys.numel(), keys.device.index)
+    flags = dtypes[keys.dtype] | (FLAG_DESCENDING if descending else 0)
+    with DistributedSorter(keys.numel(), ranks=1, device=keys.device.index, flags=flags) as s:
+        k, v, _ = s.sort_device(keys, vals)
+    return k, v

@@ -221,6 +221,18 @@ int lsb_pass(lsb_ctx* ctx, int digit, lsb_stats* stats);
 int lsb_sort_host(lsb_ctx* ctx, const lsb_elt* host_in, lsb_elt* host_out, int64_t count,
                   lsb_stats* stats);
 
+/* mySort on device memory: pack keys_in[0..count) and vals_in (NULL: the global input index, i.e. the stable argsort)
+ * into this shard, sort as lsb_sort does, and write the sorted keys and/or values to keys_out / vals_out (either may be
+ * NULL, not both).  count must equal `here`; all pointers are device memory of this context's device, 8-byte aligned;
+ * outputs may alias inputs (in place), keys_out and vals_out must not overlap.  The library's stream first waits for
+ * everything already queued on `stream` (a cudaStream_t of the caller, NULL = the legacy default stream), so a producer
+ * on that stream needs no synchronise.  Synchronous on return; afterwards the shard holds the sorted records, so
+ * lsb_verify_device / lsb_checksum / lsb_download work as after lsb_sort.  stats describes the sort between pack and
+ * unpack, as lsb_sort_host's excludes its copies.  With count == 0 the pointers are not looked at.  Bad pointers or
+ * count: LSB_ERR_ARG.  Collective. */
+int lsb_sort_device(lsb_ctx* ctx, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
+                    uint64_t* vals_out, int64_t count, void* stream, lsb_stats* stats);
+
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
 /* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard; d is the
