@@ -20,6 +20,7 @@ from .lsbsort import (  # noqa: F401
     library_path,
     load_library,
     sort_pairs,
+    sort_segments,
     sort_tensor,
     tune,
 )

@@ -26,6 +26,7 @@
 #include "lsb_kernels.cuh"
 #include "lsb_onepass.cuh"
 #include "lsb_io.cuh"
+#include "lsb_segments.cuh"
 
 #include <nccl.h>  // types only: the library itself is bound at run time, see NcclApi
 #include <dlfcn.h>
@@ -902,6 +903,17 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
   return LSB_OK;
 }
 
+// the passes [d0, d1) of lsb_sort in the context's pass shape
+int run_passes(lsb_ctx* c, int d0, int d1, int* subpasses) {
+  c->dense_ready_digit = -1;
+  if (!c->two_level) return passes_single(c, d0, d1, subpasses);
+  int rc = plan_fusion(c);
+  if (rc) return rc;
+  for (int d = d0; d < d1; d++)
+    if ((rc = pass_global(c, d, subpasses, d + 1 < d1))) return rc;
+  return LSB_OK;
+}
+
 int check_ready(lsb_ctx* c) {
   if (!c) return LSB_ERR_ARG;
   if (c->G > 1 && !c->comm_ready) return fail(c, LSB_ERR_STATE, "world_size > 1: call lsb_comm_init first");
@@ -916,21 +928,21 @@ inline bool ranges_overlap(const void* a, size_t a_bytes, const void* b, size_t 
 }
 
 // NULL or 8-byte-aligned device memory of this context's device that is not one of its own shards
-int check_device_array(lsb_ctx* c, const void* p, const char* name, int64_t count) {
+int check_device_array(lsb_ctx* c, const char* fn, const void* p, const char* name, int64_t count) {
   if (!p) return LSB_OK;
-  if ((uintptr_t)p & 7) return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not 8-byte aligned");
+  const std::string where = std::string(fn) + ": " + name;
+  if ((uintptr_t)p & 7) return fail(c, LSB_ERR_ARG, where + " is not 8-byte aligned");
   cudaPointerAttributes at;
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
     cudaGetLastError();  // not sticky: clear it so that the next launch check does not report it
-    return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not CUDA memory");
+    return fail(c, LSB_ERR_ARG, where + " is not CUDA memory");
   }
   if (at.type != cudaMemoryTypeDevice || at.device != c->cfg.device)
-    return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " is not device memory of device " +
-                                    std::to_string(c->cfg.device));
+    return fail(c, LSB_ERR_ARG, where + " is not device memory of device " + std::to_string(c->cfg.device));
   const size_t shard_bytes = (size_t)std::max<int64_t>(c->per, 1) * sizeof(Elt);
   for (int b = 0; b < 2; b++)
     if (ranges_overlap(p, (size_t)count * sizeof(uint64_t), c->buf[b], shard_bytes))
-      return fail(c, LSB_ERR_ARG, std::string("lsb_sort_device: ") + name + " overlaps the context's own shards");
+      return fail(c, LSB_ERR_ARG, where + " overlaps the context's own shards");
   return LSB_OK;
 }
 
@@ -952,6 +964,67 @@ int launch_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals) {
   if (keys && vals) unpack_kernel<true, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
   else if (keys) unpack_kernel<true, false><<<grid, IO_THREADS, 0, c->stream>>>(a);
   else unpack_kernel<false, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+// ---- lsb_sort_segments_device: offsets check, pack with segment ids, retag, unpack (lsb_segments.cuh) -------------------
+
+// The segment passes sort the retagged key word as a uint64, ascending: the key-order flags are lifted for their
+// duration and back in force when the scope ends, on every return path.  (The one-pass kernel's residency, taken at
+// lsb_create for the context's instantiation, holds for the plain one too: every instantiation is bounded by the same
+// __launch_bounds__ and dynamic shared memory.)
+struct PlainKeyOrder {
+  lsb_ctx* c;
+  uint32_t saved;
+  explicit PlainKeyOrder(lsb_ctx* ctx) : c(ctx), saved(ctx->cfg.flags) { c->cfg.flags &= ~KEY_ORDER_FLAGS; }
+  ~PlainKeyOrder() { c->cfg.flags = saved; }
+};
+
+// offsets[0] == 0, offsets[nseg] == count, non-decreasing: one flag read back (host_small[16], from small[60])
+int segsort_check(lsb_ctx* c, const int64_t* offsets, int64_t nseg, int64_t count, bool* ok) {
+  int* bad = reinterpret_cast<int*>(c->small + 60);
+  CU(c, cudaMemsetAsync(bad, 0, sizeof(int), c->stream));
+  const SegsortCheckArgs a{offsets, nseg, count, bad};
+  segsort_check_kernel<<<io_grid(c, nseg), IO_THREADS, 0, c->stream>>>(a);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  CU(c, cudaMemcpyAsync(c->host_small + 16, bad, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaStreamSynchronize(c->stream));
+  *ok = *reinterpret_cast<const int*>(c->host_small + 16) == 0;
+  return LSB_OK;
+}
+
+int launch_segsort_pack(lsb_ctx* c, const uint64_t* keys, const int64_t* offsets, int64_t nseg, int idxbits) {
+  const SegsortPackArgs a{keys, offsets, c->buf[0], c->here, nseg, idxbits};
+  segsort_pack_kernel<<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+int launch_segsort_retag(lsb_ctx* c, int idxbits, int segw) {
+  const SegsortRetagArgs a{c->buf[c->cur], c->here, idxbits, segw};
+  segsort_retag_kernel<<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+int launch_segsort_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals, const uint64_t* vals_in, const int64_t* offsets,
+                          bool local, int segw) {
+  const SegsortUnpackArgs a{c->buf[c->cur], keys, vals, vals_in, offsets, c->here, segw};
+  const int grid = io_grid(c, c->here);
+  const int mode = !vals ? SEGSORT_VALS_NONE : vals_in ? SEGSORT_VALS_GATHER : local ? SEGSORT_VALS_LOCAL : SEGSORT_VALS_GLOBAL;
+#define LSB_SEG_UNPACK(K, V) segsort_unpack_kernel<K, V><<<grid, IO_THREADS, 0, c->stream>>>(a)
+  switch (mode) {
+    case SEGSORT_VALS_NONE: LSB_SEG_UNPACK(true, SEGSORT_VALS_NONE); break;
+    case SEGSORT_VALS_GATHER: if (keys) LSB_SEG_UNPACK(true, SEGSORT_VALS_GATHER); else LSB_SEG_UNPACK(false, SEGSORT_VALS_GATHER); break;
+    case SEGSORT_VALS_LOCAL: if (keys) LSB_SEG_UNPACK(true, SEGSORT_VALS_LOCAL); else LSB_SEG_UNPACK(false, SEGSORT_VALS_LOCAL); break;
+    default: if (keys) LSB_SEG_UNPACK(true, SEGSORT_VALS_GLOBAL); else LSB_SEG_UNPACK(false, SEGSORT_VALS_GLOBAL); break;
+  }
+#undef LSB_SEG_UNPACK
+  c->launches++;
   CU(c, cudaGetLastError());
   return LSB_OK;
 }
@@ -1381,15 +1454,8 @@ int lsb_sort(lsb_ctx* c, lsb_stats* st) {
   if (rc) return rc;
   CU(c, cudaSetDevice(c->cfg.device));
   if ((rc = begin_call(c))) return rc;
-  c->dense_ready_digit = -1;
   int subpasses = 0;
-  if (!c->two_level) {
-    if ((rc = passes_single(c, 0, c->npasses, &subpasses))) return rc;
-  } else {
-    if ((rc = plan_fusion(c))) return rc;
-    for (int d = 0; d < c->npasses; d++)
-      if ((rc = pass_global(c, d, &subpasses, true))) return rc;
-  }
+  if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
   return end_call(c, st, c->npasses, subpasses);
 }
 
@@ -1432,7 +1498,7 @@ int lsb_sort_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in
     const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
     const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
     for (int i = 0; i < 4; i++)
-      if ((rc = check_device_array(c, ptrs[i], names[i], count))) return rc;
+      if ((rc = check_device_array(c, "lsb_sort_device", ptrs[i], names[i], count))) return rc;
     if (keys_out && vals_out && ranges_overlap(keys_out, (size_t)count * sizeof(uint64_t), vals_out, (size_t)count * sizeof(uint64_t)))
       return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_out and vals_out overlap");
   }
@@ -1444,6 +1510,70 @@ int lsb_sort_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in
   if (count && (rc = launch_unpack(c, keys_out, vals_out))) return rc;
   CU(c, cudaStreamSynchronize(c->stream));
   return LSB_OK;
+}
+
+int lsb_sort_segments_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
+                             uint64_t* vals_out, int64_t count, const int64_t* seg_offsets, int64_t num_segments,
+                             uint32_t seg_flags, void* stream, lsb_stats* st) {
+  static const char* fn = "lsb_sort_segments_device";
+  if (!c) return LSB_ERR_ARG;
+  if (c->G > 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": one GPU only (world_size > 1)");
+  int rc = check_ready(c);
+  if (rc) return rc;
+  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
+  if (num_segments < 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": num_segments must be >= 1");
+  if (seg_flags & ~LSB_SEG_LOCAL_INDEX) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown seg_flags");
+  const SegsortLayout lay = segsort_layout(count, num_segments, c->cfg.radix_bits);
+  if (!lay.fits)
+    return fail(c, LSB_ERR_ARG, std::string(fn) + ": segment id and input index need " + std::to_string(lay.segw + lay.idxbits) +
+                                    " bits of one key word (> 64)");
+  CU(c, cudaSetDevice(c->cfg.device));
+  const size_t bytes = (size_t)count * sizeof(uint64_t), off_bytes = (size_t)(num_segments + 1) * sizeof(int64_t);
+  if (count) {
+    if (!keys_in || !seg_offsets) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in or seg_offsets is NULL");
+    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
+    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
+    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
+    for (int i = 0; i < 4; i++)
+      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count))) return rc;
+    if ((rc = check_device_array(c, fn, seg_offsets, "seg_offsets", num_segments + 1))) return rc;
+    // keys_in is consumed by the pack, so keys_out may alias it; vals_in and the offsets are read by the unpack
+    const void* outs[2] = {keys_out, vals_out};
+    for (int i = 0; i < 2; i++) {
+      if (!outs[i]) continue;
+      if ((i == 0 && vals_out && ranges_overlap(keys_out, bytes, vals_out, bytes)) ||
+          (vals_in && ranges_overlap(outs[i], bytes, vals_in, bytes)) || ranges_overlap(outs[i], bytes, seg_offsets, off_bytes))
+        return fail(c, LSB_ERR_ARG, std::string(fn) + ": " + names[2 + i] + " overlaps another output, vals_in or seg_offsets");
+    }
+  }
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  if ((rc = begin_call(c))) return rc;
+  if (count) {
+    bool ok = false;
+    if ((rc = segsort_check(c, seg_offsets, num_segments, count, &ok))) return rc;
+    if (!ok) return fail(c, LSB_ERR_ARG, std::string(fn) + ": seg_offsets must rise from 0 to count (offsets[0] == 0, "
+                                           "offsets[num_segments] == count, non-decreasing)");
+  }
+  c->cur = 0;
+  if (count) {  // one segment: lsb_sort_device's records, {key, vals_in or the index}
+    rc = lay.segbits ? launch_segsort_pack(c, keys_in, seg_offsets, num_segments, lay.idxbits) : launch_pack(c, keys_in, vals_in);
+    if (lay.segbits == 0) c->launches++;
+    if (rc) return rc;
+  }
+  int subpasses = 0;
+  if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
+  if (lay.segbits) {
+    if (count && (rc = launch_segsort_retag(c, lay.idxbits, lay.segw))) return rc;
+    PlainKeyOrder plain(c);
+    if ((rc = run_passes(c, 0, lay.passes, &subpasses))) return rc;
+  }
+  if (count) {
+    if (lay.segbits) rc = launch_segsort_unpack(c, keys_out, vals_out, vals_in, seg_offsets, seg_flags & LSB_SEG_LOCAL_INDEX, lay.segw);
+    else if ((rc = launch_unpack(c, keys_out, vals_out)) == LSB_OK) c->launches++;
+    if (rc) return rc;
+  }
+  return end_call(c, st, c->npasses + lay.passes, subpasses);
 }
 
 // The two test hooks run the PRODUCTION count and scan kernels of the pass shape in use.

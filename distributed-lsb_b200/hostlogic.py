@@ -108,6 +108,25 @@ def part_boundaries(per, V, ramp=1.3):
     return out
 
 
+def bit_width(x):
+    return int(x).bit_length() if x > 0 else 0
+
+
+def segsort_layout(count, num_segments, radix_bits):
+    """bit layout of a segmented sort (segsort_layout in csrc/lsb_segments.cuh): (idxbits, segbits, segw, passes, fits).
+    The packed record carries the input index in idxbits = max(1, bits(count - 1)) bits below the segment id; after the
+    key passes the key word becomes seg | idx << segw, segw = the segment id's segbits = bits(num_segments - 1) rounded
+    up to whole digits, and the segment id is sorted by passes = segw / radix_bits more passes.  fits: both fields share
+    one 64-bit word (all zero and False for num_segments < 1)."""
+    if count < 0 or num_segments < 1 or not 1 <= radix_bits <= 16:
+        return 0, 0, 0, 0, False
+    idxbits = max(1, bit_width(count - 1))
+    segbits = bit_width(num_segments - 1)
+    passes = div_ceil(segbits, radix_bits)
+    segw = passes * radix_bits
+    return idxbits, segbits, segw, passes, segw + idxbits <= 64
+
+
 # ---- the one-pass kernel's work order (csrc/lsb_onepass.cuh), restated for tests ---------------------------------
 def onepass_ticket(t, nsuper, t1, lead, tiles_last=None):
     """ticket t of the one-pass kernel -> ("K1", supertile, tile) | ("K2", supertile, segment) | None (no such item).

@@ -32,6 +32,7 @@ FLAG_NO_SKIP = 8
 FLAG_KEY_I64 = 16
 FLAG_KEY_F64 = 32
 FLAG_DESCENDING = 64
+SEG_LOCAL_INDEX = 1  # lsb_sort_segments_device without vals_in: index within the segment, not the global input index
 KEY_DTYPE_FLAGS = {np.dtype(np.uint64): 0, np.dtype(np.int64): FLAG_KEY_I64, np.dtype(np.float64): FLAG_KEY_F64}
 
 
@@ -108,6 +109,7 @@ def load_library():
     L.lsb_pass.argtypes = [vp, ci, ctypes.POINTER(Stats)]
     L.lsb_sort_host.argtypes = [vp, vp, vp, i64, ctypes.POINTER(Stats)]
     L.lsb_sort_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, ctypes.POINTER(Stats)]
+    L.lsb_sort_segments_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, i64, ctypes.c_uint32, vp, ctypes.POINTER(Stats)]
     L.lsb_histogram.argtypes = [vp, ci, vp]
     L.lsb_starts.argtypes = [vp, ci, vp]
     L.lsb_num_passes.argtypes = [vp]
@@ -251,6 +253,54 @@ class DistributedSorter:
                                           ctypes.byref(st)), "lsb_sort_host")
         return st
 
+    def _outputs(self, what, keys, vals, keys_out, vals_out):
+        """checked keys_out / vals_out of sort_device and sort_segments: None allocates, False means none"""
+        torch = _torch()
+        n = self.here
+        if keys_out is False and vals_out is False:
+            raise ValueError(f"{what}: keys_out and vals_out cannot both be False")
+        _check_vector(torch, keys, "keys", n, self.device, key_flags=self.flags & (FLAG_KEY_I64 | FLAG_KEY_F64))
+        if vals is not None:
+            _check_vector(torch, vals, "vals", n, self.device)
+        if keys_out is None:
+            keys_out = torch.empty_like(keys)
+        elif keys_out is not False:
+            _check_vector(torch, keys_out, "keys_out", n, self.device)
+            if keys_out.dtype != keys.dtype:
+                raise TypeError(f"{what}: keys_out must have the keys' dtype {keys.dtype}, not {keys_out.dtype}")
+        if vals_out is None:
+            vals_out = torch.empty_like(vals) if vals is not None else torch.empty(n, dtype=torch.int64, device=keys.device)
+        elif vals_out is not False:
+            _check_vector(torch, vals_out, "vals_out", n, self.device)
+        return keys_out, vals_out
+
+    def sort_segments(self, keys, offsets, vals=None, keys_out=None, vals_out=None, local_index=False, stream=None):
+        """Every segment of a device array sorted at once (lsb_sort_segments_device): segment s is keys[offsets[s] :
+        offsets[s+1]], and the result is the stable sort by (segment, key) -- each segment in this sorter's key order,
+        the segments in ascending order.  `offsets`: 1-D contiguous int64 CUDA tensor of >= 2 elements on this sorter's
+        device, rising from 0 to `here` (the library checks its contents).  keys, vals, outputs and stream as in
+        sort_device; without vals, vals_out receives the input index of every key, or with local_index=True its index
+        within its segment (what torch.sort(dim=-1) returns for rows).  Returns (keys_out, vals_out, Stats)."""
+        torch = _torch()
+        if not isinstance(offsets, torch.Tensor):
+            raise TypeError(f"offsets must be a torch.Tensor, not {type(offsets).__name__}")
+        if offsets.dtype != torch.int64:
+            raise TypeError(f"offsets must be torch.int64, not {offsets.dtype}")
+        if offsets.dim() != 1 or offsets.numel() < 2:
+            raise ValueError(f"offsets must be 1-D with at least 2 elements (one segment), not of shape {tuple(offsets.shape)}")
+        _check_vector(torch, offsets, "offsets", None, self.device)
+        keys_out, vals_out = self._outputs("sort_segments", keys, vals, keys_out, vals_out)
+        if stream is None:
+            stream = torch.cuda.current_stream(keys.device)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        ptr = lambda t: t.data_ptr() if t is not None and t is not False else None  # noqa: E731
+        st = Stats()
+        self._check(self._L.lsb_sort_segments_device(self._ctx, ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out),
+                                                     self.here, offsets.data_ptr(), offsets.numel() - 1,
+                                                     SEG_LOCAL_INDEX if local_index else 0, handle, ctypes.byref(st)),
+                    "lsb_sort_segments_device")
+        return (keys_out if keys_out is not False else None), (vals_out if vals_out is not False else None), st
+
     def sort_device(self, keys, vals=None, keys_out=None, vals_out=None, stream=None):
         """CUDA tensors in, CUDA tensors out, no host copy (lsb_sort_device).  `keys`: 1-D contiguous uint64, int64 or
         float64 tensor of `here` elements on this sorter's device, of the dtype its key-type flags name; `vals`: the same
@@ -260,21 +310,7 @@ class DistributedSorter:
         inputs and returns when the outputs are written.  Returns (keys_out, vals_out, Stats of the sort itself)."""
         torch = _torch()
         n = self.here
-        if keys_out is False and vals_out is False:
-            raise ValueError("sort_device: keys_out and vals_out cannot both be False")
-        _check_vector(torch, keys, "keys", n, self.device, key_flags=self.flags & (FLAG_KEY_I64 | FLAG_KEY_F64))
-        if vals is not None:
-            _check_vector(torch, vals, "vals", n, self.device)
-        if keys_out is None:
-            keys_out = torch.empty_like(keys)
-        elif keys_out is not False:
-            _check_vector(torch, keys_out, "keys_out", n, self.device)
-            if keys_out.dtype != keys.dtype:
-                raise TypeError(f"sort_device: keys_out must have the keys' dtype {keys.dtype}, not {keys_out.dtype}")
-        if vals_out is None:
-            vals_out = torch.empty_like(vals) if vals is not None else torch.empty(n, dtype=torch.int64, device=keys.device)
-        elif vals_out is not False:
-            _check_vector(torch, vals_out, "vals_out", n, self.device)
+        keys_out, vals_out = self._outputs("sort_device", keys, vals, keys_out, vals_out)
         if stream is None:
             stream = torch.cuda.current_stream(keys.device)
         handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
@@ -394,4 +430,53 @@ def sort_tensor(keys, vals=None, descending=False):
     flags = dtypes[keys.dtype] | (FLAG_DESCENDING if descending else 0)
     with DistributedSorter(keys.numel(), ranks=1, device=keys.device.index, flags=flags) as s:
         k, v, _ = s.sort_device(keys, vals)
+    return k, v
+
+
+def sort_segments(keys, offsets=None, vals=None, descending=False):
+    """Sort many groups of a CUDA tensor at once, on that tensor's GPU, with no host copy.  Keys are uint64, int64 or
+    float64, sorted stably in numpy's and torch's order (NaNs last, first when descending; -0.0 == +0.0; equal keys in
+    input order; key bits never rewritten).
+      2-D keys [B, L], no offsets: every row sorted, as torch.sort(keys, dim=-1, stable=True, descending=...) does:
+        returns (sorted keys [B, L], int64 indices within the row [B, L]), or vals [B, L] permuted within the rows.
+      1-D keys with offsets (1-D int64 CUDA tensor of S + 1 elements rising from 0 to len(keys); empty segments
+        allowed): segment s = keys[offsets[s] : offsets[s+1]] sorted, the segments in place: returns (sorted keys,
+        int64 input indices), or vals permuted the same way.
+    Anything else is a ValueError.  Makes a one-GPU sorter for the call."""
+    torch = _torch()
+    if not isinstance(keys, torch.Tensor):
+        raise TypeError(f"keys must be a torch.Tensor, not {type(keys).__name__}")
+    dtypes = _key_dtype_flags(torch)
+    if keys.dtype not in dtypes:
+        raise TypeError(f"keys must be torch.uint64, int64 or float64, not {keys.dtype}")
+    if vals is not None and not isinstance(vals, torch.Tensor):
+        raise TypeError(f"vals must be a torch.Tensor, not {type(vals).__name__}")
+    if vals is not None and vals.shape != keys.shape:
+        raise ValueError(f"vals must have the keys' shape {tuple(keys.shape)}, not {tuple(vals.shape)}")
+    if keys.dim() == 2 and offsets is None:
+        rows, width = keys.shape
+        if not keys.is_cuda:
+            raise ValueError(f"keys must be a CUDA tensor, not on {keys.device}")
+        if rows == 0:
+            return keys.clone(), (vals.clone() if vals is not None else torch.empty_like(keys, dtype=torch.int64))
+        offsets = torch.arange(rows + 1, dtype=torch.int64, device=keys.device) * width
+        k, v = _sort_segments_1d(torch, keys.reshape(-1), offsets, None if vals is None else vals.reshape(-1), descending,
+                                 local_index=True)
+        return k.view(rows, width), v.view(rows, width)
+    if keys.dim() == 1 and offsets is not None:
+        return _sort_segments_1d(torch, keys, offsets, vals, descending, local_index=False)
+    raise ValueError("sort_segments takes 2-D keys without offsets (rows) or 1-D keys with offsets, not "
+                     f"{keys.dim()}-D keys {'with' if offsets is not None else 'without'} offsets")
+
+
+def _sort_segments_1d(torch, keys, offsets, vals, descending, local_index):
+    keys = keys.contiguous()
+    dtypes = _key_dtype_flags(torch)
+    _check_vector(torch, keys, "keys", key_flags=dtypes[keys.dtype])
+    if vals is not None:
+        vals = vals.contiguous()
+        _check_vector(torch, vals, "vals", keys.numel(), keys.device.index)
+    flags = dtypes[keys.dtype] | (FLAG_DESCENDING if descending else 0)
+    with DistributedSorter(keys.numel(), ranks=1, device=keys.device.index, flags=flags) as s:
+        k, v, _ = s.sort_segments(keys, offsets, vals, local_index=local_index)
     return k, v

@@ -233,6 +233,28 @@ int lsb_sort_host(lsb_ctx* ctx, const lsb_elt* host_in, lsb_elt* host_out, int64
 int lsb_sort_device(lsb_ctx* ctx, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
                     uint64_t* vals_out, int64_t count, void* stream, lsb_stats* stats);
 
+/* Segmented sort on device memory: segment s is the input positions [seg_offsets[s], seg_offsets[s+1]) (num_segments
+ * segments, empty ones allowed), and the result is the stable sort by (s, order_key(key)): every segment sorted in the
+ * context's key order, the segments themselves in ascending order (as torch.sort(x2d, dim=-1[, descending=True]) sorts
+ * rows).  keys_out[i] is the key of output position i; vals_out[i] is vals_in[j] for the input position j it came from
+ * (a gather within the segment), or without vals_in the index j itself -- or j - seg_offsets[s] with
+ * LSB_SEG_LOCAL_INDEX, the index within its segment that torch.sort(dim=-1) returns.
+ * The contract of lsb_sort_device otherwise: count == here, at least one output, 8-byte aligned device memory of the
+ * context's device that is not one of its shards, the caller's stream is waited on, synchronous on return, and with
+ * count == 0 no pointer is looked at.  keys_out may alias keys_in; an output must not overlap the other output, vals_in
+ * or seg_offsets.  seg_offsets (num_segments + 1 int64) is checked on the device before any key is read: offsets[0] == 0,
+ * offsets[num_segments] == count, non-decreasing.  LSB_ERR_ARG for world_size > 1 (one GPU only), num_segments < 1,
+ * offsets that fail the check, overlapping outputs, unknown seg_flags, and when the segment id and the input index do
+ * not fit one 64-bit word: radix_bits * ceil(bits(num_segments - 1) / radix_bits) + max(1, bits(count - 1)) > 64 (never
+ * at radix 16 with count <= 2^32).  Method: the passes of lsb_sort on the keys, then ceil(bits(num_segments - 1) /
+ * radix_bits) more on the segment id (uint64 ascending, same pass shape, same skip rule); stats covers the whole call
+ * from the pack to the unpack (passes, skipped and subpasses count both kinds).  Afterwards the shard holds internal
+ * records: what lsb_download, lsb_checksum and lsb_verify_device report is unspecified until the next sort. */
+#define LSB_SEG_LOCAL_INDEX 1u  /* without vals_in: index within the segment instead of the global input index */
+int lsb_sort_segments_device(lsb_ctx* ctx, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
+                             uint64_t* vals_out, int64_t count, const int64_t* seg_offsets, int64_t num_segments,
+                             uint32_t seg_flags, void* stream, lsb_stats* stats);
+
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
 /* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard; d is the
