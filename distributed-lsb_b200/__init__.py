@@ -12,6 +12,7 @@ from .lsbsort import (  # noqa: F401
     ELT,
     DistributedSorter,
     LsbError,
+    argsort,
     Stats,
     Verify,
     abi_symbols,
@@ -19,6 +20,7 @@ from .lsbsort import (  # noqa: F401
     header_symbols,
     library_path,
     load_library,
+    sort,
     sort_pairs,
     sort_segments,
     sort_tensor,

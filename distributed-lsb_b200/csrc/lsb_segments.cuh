@@ -5,11 +5,15 @@
 // K2 segments.  The sort between them is lsb_sort's, unchanged:
 //
 //   segsort_check_kernel   offsets[0] == 0, offsets[S] == count, non-decreasing              -> one flag
-//   segsort_pack_kernel    dst[i] = {key[i], i | seg(i) << idxbits}                           (24 B/element + offsets)
+//   segsort_pack_kernel    dst[i] = {key_word(key[i]), i | seg(i) << idxbits}                 (24 B/element + offsets)
 //   ... the key passes of lsb_sort (every pass shape and key order) ...
 //   segsort_retag_kernel   {key, idx | seg << idxbits} -> {seg | idx << segw, key}, in place  (32 B/element)
 //   ... segw / radix_bits passes on the low digits of the new key word, uint64 ascending ...
-//   segsort_unpack_kernel  keys_out[i] = val word; vals_out[i] = vals_in[idx] | idx - offsets[seg] | idx
+//   segsort_unpack_kernel  keys_out[i] = key of the val word; vals_out[i] = vals_in[idx] | idx - offsets[seg] | idx
+//
+// The key word is the 8-byte key itself, or for a narrow key type (lsb_sort_segments_device_typed) narrow_key_word:
+// the pack templated on the LSB_KEY_* type reads W-bit keys, the unpack templated on KBYTES writes the word's high half.
+// The key passes then cover the low W bits only; the retag and the segment passes move the whole word unchanged.
 //
 // The key passes leave equal (key) records in index order, so after the stable segment passes every segment holds its
 // records sorted by key and ties in input order: the stable sort by (seg, key).  A single segment (segbits == 0) needs
@@ -102,17 +106,19 @@ __device__ __forceinline__ void segsort_search(const int64_t* off, int64_t nseg,
 }
 
 struct SegsortPackArgs {
-  const uint64_t* keys;
+  const void* keys;
   const int64_t* offsets;  // [nseg + 1], checked by segsort_check_kernel
   Elt* dst;                // shard buf[0]
   int64_t count;
   int64_t nseg;
   int idxbits;
+  uint32_t flags;          // narrow KT: the key order (DESCENDING) applied to the key word
 };
 
 // Warp w of a CTA handles the 32 consecutive elements base + lane of each of its IO_U groups.  Two lanes find the
 // segments of the group's first and last element in all of offsets (one lockstep search); every lane then searches only
 // between those two, which for segments of >= 32 elements is zero or one step.
+template <int KT>
 __global__ void __launch_bounds__(IO_THREADS) segsort_pack_kernel(const SegsortPackArgs a) {
   const int lane = threadIdx.x & 31;
   const int64_t stride = (int64_t)gridDim.x * IO_THREADS;
@@ -123,7 +129,7 @@ __global__ void __launch_bounds__(IO_THREADS) segsort_pack_kernel(const SegsortP
 #pragma unroll
     for (int u = 0; u < IO_U; u++) {
       const int64_t i = base + u * stride + lane;
-      k[u] = i < a.count ? ld_stream_u64(a.keys + i) : 0;
+      k[u] = i < a.count ? ld_key_word<KT>(a.keys, i, a.flags) : 0;
       t[u] = min(base + u * stride + ((lane & 1) ? 31 : 0), last);  // even lanes: first element, odd lanes: last
       s[u] = 0;
     }
@@ -172,7 +178,7 @@ enum SegsortVals { SEGSORT_VALS_NONE = 0, SEGSORT_VALS_GATHER = 1, SEGSORT_VALS_
 
 struct SegsortUnpackArgs {
   const Elt* src;          // shard buf[cur] after the segment passes: {seg | idx << segw, key}
-  uint64_t* keys;          // KEYS only
+  void* keys;              // KEYS only
   uint64_t* vals;          // VALS != NONE only
   const uint64_t* vals_in; // GATHER
   const int64_t* offsets;  // LOCAL
@@ -180,7 +186,7 @@ struct SegsortUnpackArgs {
   int segw;
 };
 
-template <bool KEYS, int VALS>
+template <int KBYTES, bool KEYS, int VALS>
 __global__ void __launch_bounds__(IO_THREADS) segsort_unpack_kernel(const SegsortUnpackArgs a) {
   const int64_t stride = (int64_t)gridDim.x * IO_THREADS;
   const uint64_t seg_mask = (1ULL << a.segw) - 1;
@@ -201,7 +207,7 @@ __global__ void __launch_bounds__(IO_THREADS) segsort_unpack_kernel(const Segsor
 #pragma unroll
     for (int u = 0; u < IO_U; u++) {
       if (i + u * stride >= a.count) continue;
-      if (KEYS) a.keys[i + u * stride] = e[u].val;
+      if (KEYS) st_key<KBYTES>(a.keys, i + u * stride, e[u].val);
       if (VALS != SEGSORT_VALS_NONE) a.vals[i + u * stride] = v[u];
     }
   }

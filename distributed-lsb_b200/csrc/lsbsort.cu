@@ -93,6 +93,7 @@ struct lsb_ctx {
   int G = 1, my = 0;
   int64_t n = 0, per = 0, here = 0, first = 0, per_stream = 0;
   int npasses = 0;
+  int key_bits = 64;                  // bits of the key word the passes sort (narrower only inside a narrow-key call)
   cudaStream_t stream = nullptr;
   Elt* buf[2] = {nullptr, nullptr};  // A, B
   int cur = 0;                        // which of buf[] holds the data
@@ -235,7 +236,7 @@ inline bool ordered(const lsb_ctx* c) { return (c->cfg.flags & KEY_ORDER_FLAGS) 
 PassPlan plan_pass(const lsb_ctx* c, int digit) {
   PassPlan p;
   p.shift = c->cfg.radix_bits * digit;
-  p.bits = std::min<int>(c->cfg.radix_bits, 64 - p.shift);
+  p.bits = std::min<int>(c->cfg.radix_bits, c->key_bits - p.shift);
   // one-pass kernel: low BYTE, then the rest; two-step shape: balanced split (longer runs per bin)
   if (p.bits <= 8) p.lo_bits = 0;
   else p.lo_bits = (c->cfg.flags & LSB_FLAG_ONE_PASS) ? 8 : p.bits / 2;
@@ -927,11 +928,11 @@ inline bool ranges_overlap(const void* a, size_t a_bytes, const void* b, size_t 
   return x < y + b_bytes && y < x + a_bytes;
 }
 
-// NULL or 8-byte-aligned device memory of this context's device that is not one of its own shards
-int check_device_array(lsb_ctx* c, const char* fn, const void* p, const char* name, int64_t count) {
+// NULL or device memory of this context's device, aligned to its element width, that is not one of its own shards
+int check_device_array(lsb_ctx* c, const char* fn, const void* p, const char* name, int64_t count, int elt_bytes = 8) {
   if (!p) return LSB_OK;
   const std::string where = std::string(fn) + ": " + name;
-  if ((uintptr_t)p & 7) return fail(c, LSB_ERR_ARG, where + " is not 8-byte aligned");
+  if ((uintptr_t)p & (elt_bytes - 1)) return fail(c, LSB_ERR_ARG, where + " is not " + std::to_string(elt_bytes) + "-byte aligned");
   cudaPointerAttributes at;
   if (cudaPointerGetAttributes(&at, p) != cudaSuccess) {
     cudaGetLastError();  // not sticky: clear it so that the next launch check does not report it
@@ -941,7 +942,7 @@ int check_device_array(lsb_ctx* c, const char* fn, const void* p, const char* na
     return fail(c, LSB_ERR_ARG, where + " is not device memory of device " + std::to_string(c->cfg.device));
   const size_t shard_bytes = (size_t)std::max<int64_t>(c->per, 1) * sizeof(Elt);
   for (int b = 0; b < 2; b++)
-    if (ranges_overlap(p, (size_t)count * sizeof(uint64_t), c->buf[b], shard_bytes))
+    if (ranges_overlap(p, (size_t)count * elt_bytes, c->buf[b], shard_bytes))
       return fail(c, LSB_ERR_ARG, where + " overlaps the context's own shards");
   return LSB_OK;
 }
@@ -950,20 +951,45 @@ int io_grid(const lsb_ctx* c, int64_t count) {
   return (int)std::min<int64_t>((int64_t)c->num_sms * IO_CTAS_PER_SM, div_ceil(count, IO_THREADS));
 }
 
-int launch_pack(lsb_ctx* c, const uint64_t* keys, const uint64_t* vals) {
-  const PackArgs a{keys, vals, c->buf[0], c->here, c->first};
-  if (vals) pack_kernel<true><<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
-  else pack_kernel<false><<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+// expands LSB_KT_CALL(KT) for the key type `key_type` (checked by the caller: LSB_KEY_CONTEXT .. LSB_KEY_BF16)
+#define LSB_KT_SWITCH(key_type)                   \
+  switch (key_type) {                             \
+    case LSB_KEY_U32: LSB_KT_CALL(LSB_KEY_U32); break; \
+    case LSB_KEY_I32: LSB_KT_CALL(LSB_KEY_I32); break; \
+    case LSB_KEY_F32: LSB_KT_CALL(LSB_KEY_F32); break; \
+    case LSB_KEY_U16: LSB_KT_CALL(LSB_KEY_U16); break; \
+    case LSB_KEY_I16: LSB_KT_CALL(LSB_KEY_I16); break; \
+    case LSB_KEY_F16: LSB_KT_CALL(LSB_KEY_F16); break; \
+    case LSB_KEY_BF16: LSB_KT_CALL(LSB_KEY_BF16); break; \
+    default: LSB_KT_CALL(LSB_KEY_CONTEXT); break;      \
+  }
+
+// flags: the key order of the call (a narrow key's DESCENDING goes into its key word)
+int launch_pack(lsb_ctx* c, uint32_t key_type, const void* keys, const uint64_t* vals, uint32_t flags) {
+  const PackArgs a{keys, vals, c->buf[0], c->here, c->first, flags};
+  const int grid = io_grid(c, c->here);
+#define LSB_KT_CALL(KT)                                                    \
+  if (vals) pack_kernel<KT, true><<<grid, IO_THREADS, 0, c->stream>>>(a); \
+  else pack_kernel<KT, false><<<grid, IO_THREADS, 0, c->stream>>>(a)
+  LSB_KT_SWITCH(key_type)
+#undef LSB_KT_CALL
   CU(c, cudaGetLastError());
   return LSB_OK;
 }
 
-int launch_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals) {
+template <int KBYTES>
+void launch_unpack_kernel(const UnpackArgs& a, int grid, cudaStream_t stream) {
+  if (a.keys && a.vals) unpack_kernel<KBYTES, true, true><<<grid, IO_THREADS, 0, stream>>>(a);
+  else if (a.keys) unpack_kernel<KBYTES, true, false><<<grid, IO_THREADS, 0, stream>>>(a);
+  else unpack_kernel<KBYTES, false, true><<<grid, IO_THREADS, 0, stream>>>(a);
+}
+
+int launch_unpack(lsb_ctx* c, int key_bytes, void* keys, uint64_t* vals) {
   const UnpackArgs a{c->buf[c->cur], keys, vals, c->here};
   const int grid = io_grid(c, c->here);
-  if (keys && vals) unpack_kernel<true, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
-  else if (keys) unpack_kernel<true, false><<<grid, IO_THREADS, 0, c->stream>>>(a);
-  else unpack_kernel<false, true><<<grid, IO_THREADS, 0, c->stream>>>(a);
+  if (key_bytes == 8) launch_unpack_kernel<8>(a, grid, c->stream);
+  else if (key_bytes == 4) launch_unpack_kernel<4>(a, grid, c->stream);
+  else launch_unpack_kernel<2>(a, grid, c->stream);
   CU(c, cudaGetLastError());
   return LSB_OK;
 }
@@ -981,6 +1007,28 @@ struct PlainKeyOrder {
   ~PlainKeyOrder() { c->cfg.flags = saved; }
 };
 
+// The key passes of a narrow key (bits < 64): the pack already wrote the order key into the low `bits` bits of the key
+// word, so for the guard's scope every pass reads the plan of a `bits`-bit uint64 ascending key: key_bits = bits (the
+// last digit is clamped to it: at radix 13 a 32-bit key is digits of 13, 13 and 6 bits, never 7 raw key bits),
+// npasses = ceil(bits / radix_bits) and the key-order flags lifted.  All three are back when the scope ends, on every
+// return path.  At 64 bits it changes nothing.
+struct NarrowKeyPasses {
+  lsb_ctx* c;
+  const int saved_bits, saved_npasses;
+  const uint32_t saved_flags;
+  NarrowKeyPasses(lsb_ctx* ctx, int bits) : c(ctx), saved_bits(ctx->key_bits), saved_npasses(ctx->npasses), saved_flags(ctx->cfg.flags) {
+    if (bits >= 64) return;
+    c->key_bits = bits;
+    c->npasses = (int)div_ceil(bits, c->cfg.radix_bits);
+    c->cfg.flags &= ~KEY_ORDER_FLAGS;
+  }
+  ~NarrowKeyPasses() {
+    c->key_bits = saved_bits;
+    c->npasses = saved_npasses;
+    c->cfg.flags = saved_flags;
+  }
+};
+
 // offsets[0] == 0, offsets[nseg] == count, non-decreasing: one flag read back (host_small[16], from small[60])
 int segsort_check(lsb_ctx* c, const int64_t* offsets, int64_t nseg, int64_t count, bool* ok) {
   int* bad = reinterpret_cast<int*>(c->small + 60);
@@ -995,9 +1043,13 @@ int segsort_check(lsb_ctx* c, const int64_t* offsets, int64_t nseg, int64_t coun
   return LSB_OK;
 }
 
-int launch_segsort_pack(lsb_ctx* c, const uint64_t* keys, const int64_t* offsets, int64_t nseg, int idxbits) {
-  const SegsortPackArgs a{keys, offsets, c->buf[0], c->here, nseg, idxbits};
-  segsort_pack_kernel<<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+int launch_segsort_pack(lsb_ctx* c, uint32_t key_type, const void* keys, const int64_t* offsets, int64_t nseg, int idxbits,
+                        uint32_t flags) {
+  const SegsortPackArgs a{keys, offsets, c->buf[0], c->here, nseg, idxbits, flags};
+  const int grid = io_grid(c, c->here);
+#define LSB_KT_CALL(KT) segsort_pack_kernel<KT><<<grid, IO_THREADS, 0, c->stream>>>(a)
+  LSB_KT_SWITCH(key_type)
+#undef LSB_KT_CALL
   c->launches++;
   CU(c, cudaGetLastError());
   return LSB_OK;
@@ -1011,12 +1063,10 @@ int launch_segsort_retag(lsb_ctx* c, int idxbits, int segw) {
   return LSB_OK;
 }
 
-int launch_segsort_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals, const uint64_t* vals_in, const int64_t* offsets,
-                          bool local, int segw) {
-  const SegsortUnpackArgs a{c->buf[c->cur], keys, vals, vals_in, offsets, c->here, segw};
-  const int grid = io_grid(c, c->here);
-  const int mode = !vals ? SEGSORT_VALS_NONE : vals_in ? SEGSORT_VALS_GATHER : local ? SEGSORT_VALS_LOCAL : SEGSORT_VALS_GLOBAL;
-#define LSB_SEG_UNPACK(K, V) segsort_unpack_kernel<K, V><<<grid, IO_THREADS, 0, c->stream>>>(a)
+template <int KBYTES>
+void launch_segsort_unpack_kernel(const SegsortUnpackArgs& a, int grid, int mode, cudaStream_t stream) {
+#define LSB_SEG_UNPACK(K, V) segsort_unpack_kernel<KBYTES, K, V><<<grid, IO_THREADS, 0, stream>>>(a)
+  const bool keys = a.keys != nullptr;
   switch (mode) {
     case SEGSORT_VALS_NONE: LSB_SEG_UNPACK(true, SEGSORT_VALS_NONE); break;
     case SEGSORT_VALS_GATHER: if (keys) LSB_SEG_UNPACK(true, SEGSORT_VALS_GATHER); else LSB_SEG_UNPACK(false, SEGSORT_VALS_GATHER); break;
@@ -1024,9 +1074,134 @@ int launch_segsort_unpack(lsb_ctx* c, uint64_t* keys, uint64_t* vals, const uint
     default: if (keys) LSB_SEG_UNPACK(true, SEGSORT_VALS_GLOBAL); else LSB_SEG_UNPACK(false, SEGSORT_VALS_GLOBAL); break;
   }
 #undef LSB_SEG_UNPACK
+}
+
+int launch_segsort_unpack(lsb_ctx* c, int key_bytes, void* keys, uint64_t* vals, const uint64_t* vals_in,
+                          const int64_t* offsets, bool local, int segw) {
+  const SegsortUnpackArgs a{c->buf[c->cur], keys, vals, vals_in, offsets, c->here, segw};
+  const int grid = io_grid(c, c->here);
+  const int mode = !vals ? SEGSORT_VALS_NONE : vals_in ? SEGSORT_VALS_GATHER : local ? SEGSORT_VALS_LOCAL : SEGSORT_VALS_GLOBAL;
+  if (key_bytes == 8) launch_segsort_unpack_kernel<8>(a, grid, mode, c->stream);
+  else if (key_bytes == 4) launch_segsort_unpack_kernel<4>(a, grid, mode, c->stream);
+  else launch_segsort_unpack_kernel<2>(a, grid, mode, c->stream);
   c->launches++;
   CU(c, cudaGetLastError());
   return LSB_OK;
+}
+
+// the refusals the typed entry points add to the 8-byte ones; on success *key_bytes is the key width in bytes
+int check_key_type(lsb_ctx* c, const char* fn, uint32_t key_type, int* key_bytes) {
+  const int bits = key_type_bits(key_type);
+  if (!bits) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown key_type " + std::to_string(key_type));
+  if (bits < 64 && (c->cfg.flags & (LSB_FLAG_KEY_I64 | LSB_FLAG_KEY_F64)))
+    return fail(c, LSB_ERR_ARG, std::string(fn) + ": a narrow key_type needs a context without LSB_FLAG_KEY_I64 / LSB_FLAG_KEY_F64");
+  *key_bytes = bits / 8;
+  return LSB_OK;
+}
+
+int sort_device(lsb_ctx* c, const char* fn, uint32_t key_type, const void* keys_in, const uint64_t* vals_in, void* keys_out,
+                uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
+  int rc = check_ready(c);
+  if (rc) return rc;
+  int kb = 8;
+  if ((rc = check_key_type(c, fn, key_type, &kb))) return rc;
+  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
+  CU(c, cudaSetDevice(c->cfg.device));
+  if (count) {
+    if (!keys_in) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in is NULL");
+    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
+    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
+    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
+    const int widths[4] = {kb, 8, kb, 8};
+    for (int i = 0; i < 4; i++)
+      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count, widths[i]))) return rc;
+    if (keys_out && vals_out && ranges_overlap(keys_out, (size_t)count * kb, vals_out, (size_t)count * sizeof(uint64_t)))
+      return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out overlap");
+  }
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  c->cur = 0;
+  if (count && (rc = launch_pack(c, key_type, keys_in, vals_in, c->cfg.flags))) return rc;
+  {
+    NarrowKeyPasses narrow(c, kb * 8);
+    if ((rc = lsb_sort(c, st))) return rc;
+  }
+  if (count && (rc = launch_unpack(c, kb, keys_out, vals_out))) return rc;
+  CU(c, cudaStreamSynchronize(c->stream));
+  return LSB_OK;
+}
+
+int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const void* keys_in, const uint64_t* vals_in,
+                         void* keys_out, uint64_t* vals_out, int64_t count, const int64_t* seg_offsets, int64_t num_segments,
+                         uint32_t seg_flags, void* stream, lsb_stats* st) {
+  if (!c) return LSB_ERR_ARG;
+  if (c->G > 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": one GPU only (world_size > 1)");
+  int rc = check_ready(c);
+  if (rc) return rc;
+  int kb = 8;
+  if ((rc = check_key_type(c, fn, key_type, &kb))) return rc;
+  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
+  if (num_segments < 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": num_segments must be >= 1");
+  if (seg_flags & ~LSB_SEG_LOCAL_INDEX) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown seg_flags");
+  const SegsortLayout lay = segsort_layout(count, num_segments, c->cfg.radix_bits);
+  if (!lay.fits)
+    return fail(c, LSB_ERR_ARG, std::string(fn) + ": segment id and input index need " + std::to_string(lay.segw + lay.idxbits) +
+                                    " bits of one key word (> 64)");
+  CU(c, cudaSetDevice(c->cfg.device));
+  const size_t bytes = (size_t)count * sizeof(uint64_t), kbytes = (size_t)count * kb;
+  const size_t off_bytes = (size_t)(num_segments + 1) * sizeof(int64_t);
+  if (count) {
+    if (!keys_in || !seg_offsets) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in or seg_offsets is NULL");
+    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
+    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
+    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
+    const int widths[4] = {kb, 8, kb, 8};
+    for (int i = 0; i < 4; i++)
+      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count, widths[i]))) return rc;
+    if ((rc = check_device_array(c, fn, seg_offsets, "seg_offsets", num_segments + 1))) return rc;
+    // keys_in is consumed by the pack, so keys_out may alias it; vals_in and the offsets are read by the unpack
+    const void* outs[2] = {keys_out, vals_out};
+    const size_t out_bytes[2] = {kbytes, bytes};
+    for (int i = 0; i < 2; i++) {
+      if (!outs[i]) continue;
+      if ((i == 0 && vals_out && ranges_overlap(keys_out, kbytes, vals_out, bytes)) ||
+          (vals_in && ranges_overlap(outs[i], out_bytes[i], vals_in, bytes)) || ranges_overlap(outs[i], out_bytes[i], seg_offsets, off_bytes))
+        return fail(c, LSB_ERR_ARG, std::string(fn) + ": " + names[2 + i] + " overlaps another output, vals_in or seg_offsets");
+    }
+  }
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  if ((rc = begin_call(c))) return rc;
+  if (count) {
+    bool ok = false;
+    if ((rc = segsort_check(c, seg_offsets, num_segments, count, &ok))) return rc;
+    if (!ok) return fail(c, LSB_ERR_ARG, std::string(fn) + ": seg_offsets must rise from 0 to count (offsets[0] == 0, "
+                                           "offsets[num_segments] == count, non-decreasing)");
+  }
+  c->cur = 0;
+  if (count) {  // one segment: lsb_sort_device's records, {key word, vals_in or the index}
+    rc = lay.segbits ? launch_segsort_pack(c, key_type, keys_in, seg_offsets, num_segments, lay.idxbits, c->cfg.flags)
+                     : launch_pack(c, key_type, keys_in, vals_in, c->cfg.flags);
+    if (lay.segbits == 0) c->launches++;
+    if (rc) return rc;
+  }
+  int subpasses = 0, key_passes = 0;
+  {
+    NarrowKeyPasses narrow(c, kb * 8);
+    key_passes = c->npasses;
+    if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
+  }
+  if (lay.segbits) {
+    if (count && (rc = launch_segsort_retag(c, lay.idxbits, lay.segw))) return rc;
+    PlainKeyOrder plain(c);
+    if ((rc = run_passes(c, 0, lay.passes, &subpasses))) return rc;
+  }
+  if (count) {
+    if (lay.segbits) rc = launch_segsort_unpack(c, kb, keys_out, vals_out, vals_in, seg_offsets, seg_flags & LSB_SEG_LOCAL_INDEX, lay.segw);
+    else if ((rc = launch_unpack(c, kb, keys_out, vals_out)) == LSB_OK) c->launches++;
+    if (rc) return rc;
+  }
+  return end_call(c, st, key_passes + lay.passes, subpasses);
 }
 
 }  // namespace
@@ -1488,92 +1663,26 @@ int lsb_sort_host(lsb_ctx* c, const lsb_elt* host_in, lsb_elt* host_out, int64_t
 
 int lsb_sort_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out, uint64_t* vals_out,
                     int64_t count, void* stream, lsb_stats* st) {
-  int rc = check_ready(c);
-  if (rc) return rc;
-  if (count != c->here) return fail(c, LSB_ERR_ARG, "lsb_sort_device: count must equal this shard's size");
-  CU(c, cudaSetDevice(c->cfg.device));
-  if (count) {
-    if (!keys_in) return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_in is NULL");
-    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_out and vals_out are both NULL");
-    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
-    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
-    for (int i = 0; i < 4; i++)
-      if ((rc = check_device_array(c, "lsb_sort_device", ptrs[i], names[i], count))) return rc;
-    if (keys_out && vals_out && ranges_overlap(keys_out, (size_t)count * sizeof(uint64_t), vals_out, (size_t)count * sizeof(uint64_t)))
-      return fail(c, LSB_ERR_ARG, "lsb_sort_device: keys_out and vals_out overlap");
-  }
-  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
-  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
-  c->cur = 0;
-  if (count && (rc = launch_pack(c, keys_in, vals_in))) return rc;
-  if ((rc = lsb_sort(c, st))) return rc;
-  if (count && (rc = launch_unpack(c, keys_out, vals_out))) return rc;
-  CU(c, cudaStreamSynchronize(c->stream));
-  return LSB_OK;
+  return sort_device(c, "lsb_sort_device", LSB_KEY_CONTEXT, keys_in, vals_in, keys_out, vals_out, count, stream, st);
+}
+
+int lsb_sort_device_typed(lsb_ctx* c, uint32_t key_type, const void* keys_in, const uint64_t* vals_in, void* keys_out,
+                          uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
+  return sort_device(c, "lsb_sort_device_typed", key_type, keys_in, vals_in, keys_out, vals_out, count, stream, st);
 }
 
 int lsb_sort_segments_device(lsb_ctx* c, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
                              uint64_t* vals_out, int64_t count, const int64_t* seg_offsets, int64_t num_segments,
                              uint32_t seg_flags, void* stream, lsb_stats* st) {
-  static const char* fn = "lsb_sort_segments_device";
-  if (!c) return LSB_ERR_ARG;
-  if (c->G > 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": one GPU only (world_size > 1)");
-  int rc = check_ready(c);
-  if (rc) return rc;
-  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
-  if (num_segments < 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": num_segments must be >= 1");
-  if (seg_flags & ~LSB_SEG_LOCAL_INDEX) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown seg_flags");
-  const SegsortLayout lay = segsort_layout(count, num_segments, c->cfg.radix_bits);
-  if (!lay.fits)
-    return fail(c, LSB_ERR_ARG, std::string(fn) + ": segment id and input index need " + std::to_string(lay.segw + lay.idxbits) +
-                                    " bits of one key word (> 64)");
-  CU(c, cudaSetDevice(c->cfg.device));
-  const size_t bytes = (size_t)count * sizeof(uint64_t), off_bytes = (size_t)(num_segments + 1) * sizeof(int64_t);
-  if (count) {
-    if (!keys_in || !seg_offsets) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in or seg_offsets is NULL");
-    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
-    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
-    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
-    for (int i = 0; i < 4; i++)
-      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count))) return rc;
-    if ((rc = check_device_array(c, fn, seg_offsets, "seg_offsets", num_segments + 1))) return rc;
-    // keys_in is consumed by the pack, so keys_out may alias it; vals_in and the offsets are read by the unpack
-    const void* outs[2] = {keys_out, vals_out};
-    for (int i = 0; i < 2; i++) {
-      if (!outs[i]) continue;
-      if ((i == 0 && vals_out && ranges_overlap(keys_out, bytes, vals_out, bytes)) ||
-          (vals_in && ranges_overlap(outs[i], bytes, vals_in, bytes)) || ranges_overlap(outs[i], bytes, seg_offsets, off_bytes))
-        return fail(c, LSB_ERR_ARG, std::string(fn) + ": " + names[2 + i] + " overlaps another output, vals_in or seg_offsets");
-    }
-  }
-  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
-  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
-  if ((rc = begin_call(c))) return rc;
-  if (count) {
-    bool ok = false;
-    if ((rc = segsort_check(c, seg_offsets, num_segments, count, &ok))) return rc;
-    if (!ok) return fail(c, LSB_ERR_ARG, std::string(fn) + ": seg_offsets must rise from 0 to count (offsets[0] == 0, "
-                                           "offsets[num_segments] == count, non-decreasing)");
-  }
-  c->cur = 0;
-  if (count) {  // one segment: lsb_sort_device's records, {key, vals_in or the index}
-    rc = lay.segbits ? launch_segsort_pack(c, keys_in, seg_offsets, num_segments, lay.idxbits) : launch_pack(c, keys_in, vals_in);
-    if (lay.segbits == 0) c->launches++;
-    if (rc) return rc;
-  }
-  int subpasses = 0;
-  if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
-  if (lay.segbits) {
-    if (count && (rc = launch_segsort_retag(c, lay.idxbits, lay.segw))) return rc;
-    PlainKeyOrder plain(c);
-    if ((rc = run_passes(c, 0, lay.passes, &subpasses))) return rc;
-  }
-  if (count) {
-    if (lay.segbits) rc = launch_segsort_unpack(c, keys_out, vals_out, vals_in, seg_offsets, seg_flags & LSB_SEG_LOCAL_INDEX, lay.segw);
-    else if ((rc = launch_unpack(c, keys_out, vals_out)) == LSB_OK) c->launches++;
-    if (rc) return rc;
-  }
-  return end_call(c, st, c->npasses + lay.passes, subpasses);
+  return sort_segments_device(c, "lsb_sort_segments_device", LSB_KEY_CONTEXT, keys_in, vals_in, keys_out, vals_out, count,
+                              seg_offsets, num_segments, seg_flags, stream, st);
+}
+
+int lsb_sort_segments_device_typed(lsb_ctx* c, uint32_t key_type, const void* keys_in, const uint64_t* vals_in,
+                                   void* keys_out, uint64_t* vals_out, int64_t count, const int64_t* seg_offsets,
+                                   int64_t num_segments, uint32_t seg_flags, void* stream, lsb_stats* st) {
+  return sort_segments_device(c, "lsb_sort_segments_device_typed", key_type, keys_in, vals_in, keys_out, vals_out, count,
+                              seg_offsets, num_segments, seg_flags, stream, st);
 }
 
 // The two test hooks run the PRODUCTION count and scan kernels of the pass shape in use.

@@ -32,16 +32,19 @@ def global_to_local(per, glb):
     return rank, glb - rank * per
 
 
-def num_passes(radix_bits):
-    return div_ceil(64, radix_bits)  # N_DIGITS (:22), ceil as chpl/arkouda-radix-sort.chpl:78-79
+def num_passes(radix_bits, key_bits=64):
+    """N_DIGITS (:22), ceil as chpl/arkouda-radix-sort.chpl:78-79; key_bits = 32 / 16 for a narrow key type"""
+    return div_ceil(key_bits, radix_bits)
 
 
-def plan_pass(radix_bits, digit, one_pass=False):
+def plan_pass(radix_bits, digit, one_pass=False, key_bits=64):
     """(shift, bits, lo_bits, hi_bits) of reference pass `digit`: a digit wider than 8 bits is sorted as a
     stable low-sub-digit step followed by a stable high-sub-digit step, split evenly (fewer bins per step =
-    longer runs per bin); LSB_FLAG_ONE_PASS sorts it by its low byte (K1) and then by the rest (K2)"""
+    longer runs per bin); LSB_FLAG_ONE_PASS sorts it by its low byte (K1) and then by the rest (K2).  The last digit
+    is clamped to the key's width: key_bits = 32 / 16 for a narrow key type, whose order key fills the low key_bits
+    bits of the key word (plan_pass in csrc/lsbsort.cu)"""
     shift = radix_bits * digit
-    bits = min(radix_bits, 64 - shift)
+    bits = min(radix_bits, key_bits - shift)
     lo = 0 if bits <= 8 else (8 if one_pass else bits // 2)
     return shift, bits, lo, bits - lo
 

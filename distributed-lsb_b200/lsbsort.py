@@ -34,6 +34,9 @@ FLAG_KEY_F64 = 32
 FLAG_DESCENDING = 64
 SEG_LOCAL_INDEX = 1  # lsb_sort_segments_device without vals_in: index within the segment, not the global input index
 KEY_DTYPE_FLAGS = {np.dtype(np.uint64): 0, np.dtype(np.int64): FLAG_KEY_I64, np.dtype(np.float64): FLAG_KEY_F64}
+# key types of lsb_sort_device_typed / lsb_sort_segments_device_typed (LSB_KEY_*), by torch dtype name
+KEY_CONTEXT = 0
+NARROW_KEY_TYPES = {"uint32": 1, "int32": 2, "float32": 3, "uint16": 4, "int16": 5, "float16": 6, "bfloat16": 7}
 
 
 class LsbError(RuntimeError):
@@ -110,6 +113,9 @@ def load_library():
     L.lsb_sort_host.argtypes = [vp, vp, vp, i64, ctypes.POINTER(Stats)]
     L.lsb_sort_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, ctypes.POINTER(Stats)]
     L.lsb_sort_segments_device.argtypes = [vp, vp, vp, vp, vp, i64, vp, i64, ctypes.c_uint32, vp, ctypes.POINTER(Stats)]
+    L.lsb_sort_device_typed.argtypes = [vp, ctypes.c_uint32, vp, vp, vp, vp, i64, vp, ctypes.POINTER(Stats)]
+    L.lsb_sort_segments_device_typed.argtypes = [vp, ctypes.c_uint32, vp, vp, vp, vp, i64, vp, i64, ctypes.c_uint32, vp,
+                                                 ctypes.POINTER(Stats)]
     L.lsb_histogram.argtypes = [vp, ci, vp]
     L.lsb_starts.argtypes = [vp, ci, vp]
     L.lsb_num_passes.argtypes = [vp]
@@ -162,10 +168,22 @@ class PinnedBuffer:
 
 
 class DistributedSorter:
-    """One process's view of the distributed arrays A and B (one shard of each on one GPU)."""
+    """One process's view of the distributed arrays A and B (one shard of each on one GPU).
+
+    key_dtype: None for the 8-byte key the flags name, or one of torch.uint32, int32, float32, uint16, int16, float16,
+    bfloat16: sort_device / sort_segments then take keys (and keys_out) of exactly that dtype and sort them in
+    ceil(W / radix_bits) passes (lsb_sort_device_typed); flags may add FLAG_DESCENDING but no 8-byte key type."""
+
+    key_dtype = None
 
     def __init__(self, n, ranks=0, world_size=1, world_rank=0, device=0, radix_bits=16, seed_base=0,
-                 key_mask=0xFFFFFFFFFFFFFFFF, and_draws=1, flags=0):
+                 key_mask=0xFFFFFFFFFFFFFFFF, and_draws=1, flags=0, key_dtype=None):
+        if key_dtype is not None:
+            torch = _torch()
+            if _narrow_key_type(torch, key_dtype) is None:
+                raise TypeError(f"key_dtype must be None or one of torch.{', torch.'.join(NARROW_KEY_TYPES)}, not {key_dtype}")
+            if flags & (FLAG_KEY_I64 | FLAG_KEY_F64):
+                raise ValueError(f"key_dtype {key_dtype} excludes the 8-byte key-type flags FLAG_KEY_I64 / FLAG_KEY_F64")
         self._L = load_library()
         self._ctx = ctypes.c_void_p()
         cfg = _Config(n=n, ranks=ranks, world_size=world_size, world_rank=world_rank, device=device,
@@ -180,6 +198,7 @@ class DistributedSorter:
         self.per, self.here, self.first_global = per.value, here.value, first.value
         self.radix_bits = radix_bits
         self.device, self.flags = device, flags
+        self.key_dtype = key_dtype
 
     create = classmethod(lambda cls, *a, **k: cls(*a, **k))
 
@@ -259,13 +278,16 @@ class DistributedSorter:
         n = self.here
         if keys_out is False and vals_out is False:
             raise ValueError(f"{what}: keys_out and vals_out cannot both be False")
-        _check_vector(torch, keys, "keys", n, self.device, key_flags=self.flags & (FLAG_KEY_I64 | FLAG_KEY_F64))
+        if self.key_dtype is None:
+            _check_vector(torch, keys, "keys", n, self.device, key_flags=self.flags & (FLAG_KEY_I64 | FLAG_KEY_F64))
+        else:
+            _check_vector(torch, keys, "keys", n, self.device, dtype=self.key_dtype)
         if vals is not None:
             _check_vector(torch, vals, "vals", n, self.device)
         if keys_out is None:
             keys_out = torch.empty_like(keys)
         elif keys_out is not False:
-            _check_vector(torch, keys_out, "keys_out", n, self.device)
+            _check_vector(torch, keys_out, "keys_out", n, self.device, dtype=self.key_dtype)
             if keys_out.dtype != keys.dtype:
                 raise TypeError(f"{what}: keys_out must have the keys' dtype {keys.dtype}, not {keys_out.dtype}")
         if vals_out is None:
@@ -295,15 +317,19 @@ class DistributedSorter:
         handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
         ptr = lambda t: t.data_ptr() if t is not None and t is not False else None  # noqa: E731
         st = Stats()
-        self._check(self._L.lsb_sort_segments_device(self._ctx, ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out),
-                                                     self.here, offsets.data_ptr(), offsets.numel() - 1,
-                                                     SEG_LOCAL_INDEX if local_index else 0, handle, ctypes.byref(st)),
-                    "lsb_sort_segments_device")
+        args = (ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out), self.here, offsets.data_ptr(), offsets.numel() - 1,
+                SEG_LOCAL_INDEX if local_index else 0, handle, ctypes.byref(st))
+        if self.key_dtype is None:
+            self._check(self._L.lsb_sort_segments_device(self._ctx, *args), "lsb_sort_segments_device")
+        else:
+            key_type = _narrow_key_type(torch, self.key_dtype)
+            self._check(self._L.lsb_sort_segments_device_typed(self._ctx, key_type, *args), "lsb_sort_segments_device_typed")
         return (keys_out if keys_out is not False else None), (vals_out if vals_out is not False else None), st
 
     def sort_device(self, keys, vals=None, keys_out=None, vals_out=None, stream=None):
         """CUDA tensors in, CUDA tensors out, no host copy (lsb_sort_device).  `keys`: 1-D contiguous uint64, int64 or
-        float64 tensor of `here` elements on this sorter's device, of the dtype its key-type flags name; `vals`: the same
+        float64 tensor of `here` elements on this sorter's device, of the dtype its key-type flags name (of key_dtype
+        when the sorter has one: lsb_sort_device_typed); `vals`: the same
         shape with any 8-byte dtype, or None for the global input index (torch.int64: the stable argsort).  keys_out /
         vals_out: a tensor to write (may be the input itself: in place), None to allocate one, False for none (not
         both).  The library waits for the work queued on `stream` (default: the current stream) before it reads the
@@ -316,8 +342,12 @@ class DistributedSorter:
         handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
         ptr = lambda t: t.data_ptr() if t is not None and t is not False else None  # noqa: E731
         st = Stats()
-        self._check(self._L.lsb_sort_device(self._ctx, ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out), n, handle,
-                                            ctypes.byref(st)), "lsb_sort_device")
+        args = (ptr(keys), ptr(vals), ptr(keys_out), ptr(vals_out), n, handle, ctypes.byref(st))
+        if self.key_dtype is None:
+            self._check(self._L.lsb_sort_device(self._ctx, *args), "lsb_sort_device")
+        else:
+            key_type = _narrow_key_type(torch, self.key_dtype)
+            self._check(self._L.lsb_sort_device_typed(self._ctx, key_type, *args), "lsb_sort_device_typed")
         return (keys_out if keys_out is not False else None), (vals_out if vals_out is not False else None), st
 
     # -- test hooks -----------------------------------------------------------------------
@@ -384,12 +414,20 @@ def _key_dtype_flags(torch):
     return {torch.uint64: 0, torch.int64: FLAG_KEY_I64, torch.float64: FLAG_KEY_F64}
 
 
-def _check_vector(torch, t, name, n=None, device=None, key_flags=None):
-    """TypeError / ValueError unless `t` is a 1-D contiguous CUDA tensor of 8-byte elements (of n elements on `device`,
-    and of the key dtype that `key_flags` names, when given)"""
+def _narrow_key_type(torch, dtype):
+    """LSB_KEY_* of a narrow torch dtype, None for any other"""
+    return NARROW_KEY_TYPES.get(str(dtype).replace("torch.", "")) if isinstance(dtype, torch.dtype) else None
+
+
+def _check_vector(torch, t, name, n=None, device=None, key_flags=None, dtype=None):
+    """TypeError / ValueError unless `t` is a 1-D contiguous CUDA tensor of 8-byte elements, or of exactly `dtype` when
+    given (of n elements on `device`, and of the key dtype that `key_flags` names, when given)"""
     if not isinstance(t, torch.Tensor):
         raise TypeError(f"{name} must be a torch.Tensor, not {type(t).__name__}")
-    if key_flags is not None:
+    if dtype is not None:
+        if t.dtype != dtype:
+            raise TypeError(f"{name} must be {dtype}, the sorter's key_dtype, not {t.dtype}")
+    elif key_flags is not None:
         dtypes = _key_dtype_flags(torch)
         if t.dtype not in dtypes:
             raise TypeError(f"{name} must be torch.uint64, int64 or float64, not {t.dtype}")
@@ -480,3 +518,49 @@ def _sort_segments_1d(torch, keys, offsets, vals, descending, local_index):
     with DistributedSorter(keys.numel(), ranks=1, device=keys.device.index, flags=flags) as s:
         k, v, _ = s.sort_segments(keys, offsets, vals, local_index=local_index)
     return k, v
+
+
+def sort(input, dim=-1, descending=False, stable=False):
+    """torch.sort for a CUDA tensor of uint64, int64, float64, uint32, int32, float32, uint16, int16, float16 or bfloat16
+    keys, of any rank and `dim`, on that tensor's GPU: returns torch.return_types.sort(values, indices).  The result is
+    always the stable sort (also a valid answer for stable=False), in numpy's and torch's order: NaNs last (first when
+    descending), -0.0 == +0.0, equal keys in input order; key bits are never rewritten, and a W-bit key takes
+    ceil(W / 16) passes.  One row (1-D input, or every other dimension of size 1) is one sort_device; more rows are
+    sorted at once by sort_segments with `dim` moved last.  Makes a one-GPU sorter for the call."""
+    torch = _torch()
+    values, indices = _sort_rows(torch, input, dim, descending, keys=True)
+    return torch.return_types.sort((values, indices))
+
+
+def argsort(input, dim=-1, descending=False, stable=False):
+    """torch.argsort: the indices of sort(input, dim, descending), without writing the sorted keys"""
+    return _sort_rows(_torch(), input, dim, descending, keys=False)[1]
+
+
+def _sort_rows(torch, x, dim, descending, keys):
+    if not isinstance(x, torch.Tensor):
+        raise TypeError(f"input must be a torch.Tensor, not {type(x).__name__}")
+    wide = _key_dtype_flags(torch)
+    if x.dtype not in wide and _narrow_key_type(torch, x.dtype) is None:
+        raise TypeError(f"input must be torch.uint64, int64, float64, torch.{', torch.'.join(NARROW_KEY_TYPES)}, not {x.dtype}")
+    if not x.is_cuda:
+        raise ValueError(f"input must be a CUDA tensor, not on {x.device}")
+    nd = max(x.dim(), 1)
+    if isinstance(dim, bool) or not isinstance(dim, int) or not -nd <= dim < nd:
+        raise ValueError(f"dim must be an int in [{-nd}, {nd - 1}] for a {x.dim()}-D input, not {dim!r}")
+    if x.dim() == 0 or x.numel() == 0:  # as torch answers: the input itself, index 0 / nothing
+        return (x.clone() if keys else None), torch.zeros_like(x, dtype=torch.int64)
+    d = dim % nd
+    rows = x.movedim(d, -1).contiguous()
+    shape, width = rows.shape, rows.shape[-1]
+    flat = rows.view(-1)
+    flags = wide.get(x.dtype, 0) | (FLAG_DESCENDING if descending else 0)
+    key_dtype = None if x.dtype in wide else x.dtype
+    with DistributedSorter(flat.numel(), ranks=1, device=x.device.index, flags=flags, key_dtype=key_dtype) as s:
+        if flat.numel() == width:
+            k, v, _ = s.sort_device(flat, keys_out=None if keys else False)
+        else:
+            offsets = torch.arange(flat.numel() // width + 1, dtype=torch.int64, device=x.device) * width
+            k, v, _ = s.sort_segments(flat, offsets, keys_out=None if keys else False, local_index=True)
+    back = lambda t: t.view(shape).movedim(-1, d).contiguous()  # noqa: E731
+    return (back(k) if keys else None), back(v)

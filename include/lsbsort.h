@@ -114,6 +114,29 @@ typedef struct lsb_config {
 #define LSB_FLAG_KEY_F64 32u     /* key is an IEEE-754 binary64                                 */
 #define LSB_FLAG_DESCENDING 64u  /* largest first                                               */
 
+/*
+ * Key types of lsb_sort_device_typed / lsb_sort_segments_device_typed.  LSB_KEY_CONTEXT is the 8-byte key the
+ * context's flags name.  The others are narrow keys of W = 32 or 16 bits, W / 8 bytes each in the caller's arrays,
+ * aligned to their own width:
+ *   LSB_KEY_U32 / LSB_KEY_U16:  order k
+ *   LSB_KEY_I32 / LSB_KEY_I16:  order k ^ signbit (two's complement)
+ *   LSB_KEY_F32 / LSB_KEY_F16 / LSB_KEY_BF16 (exponent/mantissa 8/23, 5/10, 8/7 bits): the LSB_FLAG_KEY_F64 rule at
+ *     width W: -0 as +0, every NaN as all ones, any other value k ^ (sign ? all ones : signbit)
+ *   LSB_FLAG_DESCENDING: the complement of that within W bits.
+ * The order is numpy's and torch's stable one, as for the 8-byte keys.  A narrow key travels in the record's key word
+ * as (uint64)k << 32 | order_W(k); the sort takes ceil(W / radix_bits) passes over the low W bits only (uint64
+ * ascending: the order was applied by the pack), and the key written back is the word's high half, so key bits are
+ * never rewritten.  A narrow type needs a context without LSB_FLAG_KEY_I64 / LSB_FLAG_KEY_F64.
+ */
+#define LSB_KEY_CONTEXT 0   /* 8-byte key ordered by the context's flags: exactly lsb_sort_device */
+#define LSB_KEY_U32 1
+#define LSB_KEY_I32 2
+#define LSB_KEY_F32 3
+#define LSB_KEY_U16 4
+#define LSB_KEY_I16 5
+#define LSB_KEY_F16 6
+#define LSB_KEY_BF16 7
+
 /* what lsb_sort / lsb_pass measured, device time from CUDA events on the sort stream */
 typedef struct lsb_stats {
   double device_ms;       /* whole call: first kernel start -> last kernel end             */
@@ -254,6 +277,20 @@ int lsb_sort_device(lsb_ctx* ctx, const uint64_t* keys_in, const uint64_t* vals_
 int lsb_sort_segments_device(lsb_ctx* ctx, const uint64_t* keys_in, const uint64_t* vals_in, uint64_t* keys_out,
                              uint64_t* vals_out, int64_t count, const int64_t* seg_offsets, int64_t num_segments,
                              uint32_t seg_flags, void* stream, lsb_stats* stats);
+
+/* lsb_sort_device and lsb_sort_segments_device for keys of type key_type (LSB_KEY_*): keys_in and keys_out are arrays
+ * of W-bit keys aligned to W / 8 bytes; values and indices stay 8-byte.  With LSB_KEY_CONTEXT they are exactly the two
+ * calls above.  A narrow type sorts in ceil(W / radix_bits) key passes (lsb_stats.passes counts them, plus any segment
+ * passes), every pass shape and the skip rule as for 8-byte keys.  Contracts as above (multi-GPU: each rank passes its
+ * shard; the segmented form is one GPU only), with the pointer and overlap checks on the real byte widths of each
+ * array.  LSB_ERR_ARG also for an unknown key_type, a narrow type on a context with LSB_FLAG_KEY_I64 or
+ * LSB_FLAG_KEY_F64, and a key pointer not aligned to its width.  After a narrow call the shard holds internal records:
+ * what lsb_download, lsb_checksum and lsb_verify_device report is unspecified until the next sort. */
+int lsb_sort_device_typed(lsb_ctx* ctx, uint32_t key_type, const void* keys_in, const uint64_t* vals_in, void* keys_out,
+                          uint64_t* vals_out, int64_t count, void* stream, lsb_stats* stats);
+int lsb_sort_segments_device_typed(lsb_ctx* ctx, uint32_t key_type, const void* keys_in, const uint64_t* vals_in,
+                                   void* keys_out, uint64_t* vals_out, int64_t count, const int64_t* seg_offsets,
+                                   int64_t num_segments, uint32_t seg_flags, void* stream, lsb_stats* stats);
 
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
