@@ -93,7 +93,6 @@ struct lsb_ctx {
   int G = 1, my = 0;
   int64_t n = 0, per = 0, here = 0, first = 0, per_stream = 0;
   int npasses = 0;
-  int key_bits = 64;                  // bits of the key word the passes sort (narrower only inside a narrow-key call)
   cudaStream_t stream = nullptr;
   Elt* buf[2] = {nullptr, nullptr};  // A, B
   int cur = 0;                        // which of buf[] holds the data
@@ -230,13 +229,31 @@ int fail(lsb_ctx* c, int code, const std::string& msg) {
 inline int64_t div_ceil(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 constexpr uint32_t KEY_ORDER_FLAGS = LSB_FLAG_KEY_I64 | LSB_FLAG_KEY_F64 | LSB_FLAG_DESCENDING;
-// digits come from order_key(key) (the ORD = true instantiation of every digit-reading kernel), not from the raw key
-inline bool ordered(const lsb_ctx* c) { return (c->cfg.flags & KEY_ORDER_FLAGS) != 0; }
 
-PassPlan plan_pass(const lsb_ctx* c, int digit) {
+// What one run of passes sorts: the low `bits` bits of the key word, read through order_key(key, korder) when korder
+// is not 0 (the ORD = true instantiation of every digit-reading kernel), as the raw uint64 otherwise.  The one-pass
+// kernel's residency, taken at lsb_create for the context's instantiation, holds for the other one too: both are
+// bounded by the same __launch_bounds__ and dynamic shared memory.
+struct KeyPlan {
+  int bits;         // 64, or W for a narrow key (the last digit is clamped to it)
+  uint32_t korder;  // the context's key-order flags, or 0 when the key word already holds the order key
+};
+
+KeyPlan context_plan(const lsb_ctx* c) { return {64, c->cfg.flags & KEY_ORDER_FLAGS}; }
+
+// A narrow key's pack writes its order key into the low W bits of the key word: its passes sort those as a uint64
+// ascending.  At radix 13 a 32-bit key is digits of 13, 13 and 6 bits, never 7 raw key bits.
+KeyPlan key_type_plan(const lsb_ctx* c, uint32_t key_type) {
+  const int bits = key_type_bits(key_type);
+  return bits < 64 ? KeyPlan{bits, 0} : context_plan(c);
+}
+
+int num_passes(const lsb_ctx* c, const KeyPlan& k) { return (int)div_ceil(k.bits, c->cfg.radix_bits); }
+
+PassPlan plan_pass(const lsb_ctx* c, const KeyPlan& k, int digit) {
   PassPlan p;
   p.shift = c->cfg.radix_bits * digit;
-  p.bits = std::min<int>(c->cfg.radix_bits, c->key_bits - p.shift);
+  p.bits = std::min<int>(c->cfg.radix_bits, k.bits - p.shift);
   // one-pass kernel: low BYTE, then the rest; two-step shape: balanced split (longer runs per bin)
   if (p.bits <= 8) p.lo_bits = 0;
   else p.lo_bits = (c->cfg.flags & LSB_FLAG_ONE_PASS) ? 8 : p.bits / 2;
@@ -323,8 +340,8 @@ int end_call(lsb_ctx* c, lsb_stats* st, int passes, int subpasses) {
 // counts of `ndig` digits over src[0, m) in ONE read (localShuffle's count loop, :226-229):
 // digit i of width bits[i] at shift[i] is accumulated into out[out_off[i] ...] (u64 or u32
 // bins, the caller zeroes them).  Digits are packed into at most 4 roles of <= 65 536 bins.
-int launch_digit_hist(lsb_ctx* c, const Elt* src, int64_t m, const int* shift, const int* bits, const int* out_off, int ndig,
-                      void* out, bool out_u32) {
+int launch_digit_hist(lsb_ctx* c, uint32_t korder, const Elt* src, int64_t m, const int* shift, const int* bits, const int* out_off,
+                      int ndig, void* out, bool out_u32) {
   for (int first = 0; first < ndig;) {
     DigitHistArgs a;
     memset(&a, 0, sizeof(a));
@@ -332,7 +349,7 @@ int launch_digit_hist(lsb_ctx* c, const Elt* src, int64_t m, const int* shift, c
     a.m = m;
     a.out = out;
     a.out_u32 = out_u32 ? 1 : 0;
-    a.korder = c->cfg.flags;
+    a.korder = korder;
     int nd = 0, role = 0, role_bins = 0;
     a.role_first[0] = 0;
     while (first + nd < ndig && nd < DH_MAX_DIGITS) {
@@ -357,7 +374,7 @@ int launch_digit_hist(lsb_ctx* c, const Elt* src, int64_t m, const int* shift, c
       bool one_each = true;
       for (int r = 0; r < a.nroles; r++) one_each = one_each && (a.role_first[r + 1] - a.role_first[r] == 1);
       const int grid = groups * a.nroles;
-      if (ordered(c)) {
+      if (korder) {
         if (one_each) digit_hist_kernel<1, true><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
         else digit_hist_kernel<0, true><<<grid, DH_THREADS, DH_SMEM, c->stream>>>(a);
       } else {
@@ -398,7 +415,7 @@ void launch_subdigit_hist_kernel(const HistArgs& a, int grid, bool bytes, cudaSt
 }
 
 // 256-bin histograms of up to HIST_MAX_SUB sub-digits in one read + their exclusive scans (two-step shape)
-int launch_subdigit_hist(lsb_ctx* c, const Elt* src, const SubPass* subs, int nsub) {
+int launch_subdigit_hist(lsb_ctx* c, uint32_t korder, const Elt* src, const SubPass* subs, int nsub) {
   CU(c, cudaMemsetAsync(c->hist, 0, sizeof(unsigned long long) * 256 * HIST_MAX_SUB, c->stream));
   if (c->here > 0) {
     HistArgs a;
@@ -411,11 +428,11 @@ int launch_subdigit_hist(lsb_ctx* c, const Elt* src, const SubPass* subs, int ns
       a.mask[s] = (1u << subs[s].bits) - 1;
     }
     a.out = c->hist;
-    a.korder = c->cfg.flags;
+    a.korder = korder;
     const int grid = (int)std::min<int64_t>((int64_t)c->num_sms * 4, div_ceil(c->here, HIST_THREADS));
     bool bytes = true;  // sub-digits are exactly bytes 0..nsub-1 of the key (radix 8 and 16)
     for (int s = 0; s < nsub; s++) bytes = bytes && subs[s].shift == 8 * s && subs[s].bits == 8;
-    if (ordered(c)) launch_subdigit_hist_kernel<true>(a, grid, bytes, c->stream);
+    if (korder) launch_subdigit_hist_kernel<true>(a, grid, bytes, c->stream);
     else launch_subdigit_hist_kernel<false>(a, grid, bytes, c->stream);
     c->launches++;
   }
@@ -446,7 +463,7 @@ int launch_scan(lsb_ctx* c, const unsigned long long* counts, int nb, int G, int
 
 // one stable counting-sort step on <= 8 bits over src[0, m): the whole pass for digits of <= 8
 // bits, half a pass in the two-step shape.  bases[bin] = first output index of the bin.
-int launch_partition(lsb_ctx* c, const Elt* src, int64_t m, int shift, int bits, const int64_t* seg_start,
+int launch_partition(lsb_ctx* c, uint32_t korder, const Elt* src, int64_t m, int shift, int bits, const int64_t* seg_start,
                      const uint32_t* seg_tile_start, const int64_t* bases, Elt* dst) {
   if (c->gen > 126) {  // tags exhausted: wipe the look-back words and start over
     CU(c, cudaMemsetAsync(c->lookback, 0, c->lookback_tiles * 256 * sizeof(uint64_t), c->stream));
@@ -474,17 +491,17 @@ int launch_partition(lsb_ctx* c, const Elt* src, int64_t m, int shift, int bits,
   a.world = 1;
   a.dst[0] = dst;
   a.prof = c->op_prof;
-  a.direct = g_tune.pt_direct;
-  a.log_chunks = g_tune.pt_chunks;
+  a.direct = c->tune.pt_direct;
+  a.log_chunks = c->tune.pt_chunks;
   a.d_begin = 0;
   a.d_end = m;
-  a.pf_tiles = g_tune.pt_pf_tiles > 0 ? g_tune.pt_pf_tiles : std::max(1, c->num_sms / 2);
-  a.korder = c->cfg.flags;
+  a.pf_tiles = c->tune.pt_pf_tiles > 0 ? c->tune.pt_pf_tiles : std::max(1, c->num_sms / 2);
+  a.korder = korder;
   c->part_elems += m;
   if (m > 0) {
     const unsigned grid = (unsigned)div_ceil(m, c->tile);
-    const bool l2pf = a.direct && g_tune.pt_variant;  // the prefetch needs blockIdx-ordered tiles
-    if (ordered(c)) {
+    const bool l2pf = a.direct && c->tune.pt_variant;  // the prefetch needs blockIdx-ordered tiles
+    if (korder) {
       if (l2pf) partition_kernel<TileCfg, true, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
       else partition_kernel<TileCfg, false, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
     } else {
@@ -499,8 +516,8 @@ int launch_partition(lsb_ctx* c, const Elt* src, int64_t m, int shift, int bits,
 
 // one stable scatter on a digit of 9..16 bits over src[0, m) -> dst: starts[d] + add is the first
 // output index of digit d (natural digit order); `ctas_per_sm` 0 = as many as stay resident
-int launch_onepass(lsb_ctx* c, const Elt* src, Elt* dst, int64_t m, int shift, int bits, const int64_t* starts, long long add,
-                   int ctas_per_sm) {
+int launch_onepass(lsb_ctx* c, uint32_t korder, const Elt* src, Elt* dst, int64_t m, int shift, int bits, const int64_t* starts,
+                   long long add, int ctas_per_sm) {
   c->part_elems += m;
   if (m > 0) {
     const int T1 = c->tune.op_t1, NX = c->tune.op_nx;
@@ -547,18 +564,18 @@ int launch_onepass(lsb_ctx* c, const Elt* src, Elt* dst, int64_t m, int shift, i
     a.biglist = ctl + o_biglist;
     a.timeout_ns = (unsigned long long)c->tune.timeout_ms * 1000000ULL;
     a.prof = c->op_prof;
-    a.korder = c->cfg.flags;
+    a.korder = korder;
     const int per_sm = ctas_per_sm > 0 ? std::min(ctas_per_sm, c->op_resident) : c->op_resident;
     // every claimed item must belong to a resident CTA: never launch more CTAs than fit
     const int64_t useful = div_ceil(m, c->op_tile) + 256;
     const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((int64_t)c->num_sms * per_sm, useful));
     const bool byte = (shift % 8) == 0 && bits == 16;  // both digit halves are whole bytes of the key
     if (c->tune.op_cfg == 1) {
-      if (ordered(c)) onepass_kernel<TileCfgS, false, true><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
+      if (korder) onepass_kernel<TileCfgS, false, true><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
       else if (byte) onepass_kernel<TileCfgS, true, false><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
       else onepass_kernel<TileCfgS, false, false><<<grid, TileCfgS::THREADS, TileCfgS::SMEM, c->stream>>>(a);
     } else {
-      if (ordered(c)) onepass_kernel<TileCfg, false, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
+      if (korder) onepass_kernel<TileCfg, false, true><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
       else if (byte) onepass_kernel<TileCfg, true, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
       else onepass_kernel<TileCfg, false, false><<<grid, TileCfg::THREADS, TileCfg::SMEM, c->stream>>>(a);
     }
@@ -581,15 +598,15 @@ int64_t part_len(const lsb_ctx* c, int q) {
 
 // virtual-rank counts of digit `digit` for every part of every GPU -> c_all[G*V][nb]
 // (localShuffle's counts, :226-229, per part; then the count exchange of :327-383)
-int count_parts(lsb_ctx* c, int digit) {
-  const PassPlan p = plan_pass(c, digit);
+int count_parts(lsb_ctx* c, const KeyPlan& k, int digit) {
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits, V = c->V;
   CU(c, cudaMemsetAsync(c->dense_local, 0, sizeof(unsigned) * (size_t)V * nb, c->stream));
   for (int q = 0; q < V; q++) {
     const int64_t m = part_len(c, q);
     if (m <= 0) continue;
     const int off = q * nb;
-    int rc = launch_digit_hist(c, c->buf[c->cur] + c->pstart[q], m, &p.shift, &p.bits, &off, 1, c->dense_local, true);
+    int rc = launch_digit_hist(c, k.korder, c->buf[c->cur] + c->pstart[q], m, &p.shift, &p.bits, &off, 1, c->dense_local, true);
     if (rc) return rc;
   }
   if (c->G > 1) {
@@ -603,8 +620,8 @@ int count_parts(lsb_ctx* c, int digit) {
 // c_all -> mybase_v[q][d] (global output index of part q's first element of digit d: the
 // reference's exclusive scan in digit-major / rank-minor order, :327-479, over virtual ranks),
 // sent[] (:553-554), localbase_v and the bases of the local step(s) of every part
-int part_offsets(lsb_ctx* c, int digit) {
-  const PassPlan p = plan_pass(c, digit);
+int part_offsets(lsb_ctx* c, const KeyPlan& k, int digit) {
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits, V = c->V;
   CU(c, cudaMemsetAsync(c->small, 0, 8 * sizeof(unsigned long long), c->stream));
   VrScanArgs v;
@@ -638,8 +655,8 @@ int part_offsets(lsb_ctx* c, int digit) {
 }
 
 // c_all (counts of every virtual rank) -> does one digit value hold all n elements?
-int digit_is_constant(lsb_ctx* c, int digit, bool* constant) {
-  const PassPlan p = plan_pass(c, digit);
+int digit_is_constant(lsb_ctx* c, const KeyPlan& k, int digit, bool* constant) {
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits;
   VrScanArgs v;
   memset(&v, 0, sizeof(v));
@@ -661,22 +678,23 @@ int digit_is_constant(lsb_ctx* c, int digit, bool* constant) {
 
 // Which passes may have their digit counted by the previous pass's exchange kernel: digits of >= 12 bits that
 // take >= 2048 distinct values among the first 65 536 elements of every shard (a digit's distribution does not
-// change when the array is permuted, so the input is as good a sample as any).  One host sync, before pass 0.
-int plan_fusion(lsb_ctx* c) {
+// change when the array is permuted, so the input is as good a sample as any).  One host sync, before pass 0.  Every
+// digit of the plan is sampled, whichever of its passes the caller runs.
+int plan_fusion(lsb_ctx* c, const KeyPlan& k) {
   unsigned* d = c->fuse_live;
-  const int m = (int)std::min<int64_t>(c->here, 65536);
-  for (int p = 0; p < c->npasses; p++) {
-    const PassPlan q = plan_pass(c, p);
+  const int m = (int)std::min<int64_t>(c->here, 65536), np = num_passes(c, k);
+  for (int p = 0; p < np; p++) {
+    const PassPlan q = plan_pass(c, k, p);
     const uint32_t mask = (uint32_t)((1u << q.bits) - 1);
-    if (ordered(c)) live_bins_kernel<true><<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, mask, d + p, c->cfg.flags);
+    if (k.korder) live_bins_kernel<true><<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, mask, d + p, k.korder);
     else live_bins_kernel<false><<<1, 1024, 0, c->stream>>>(c->buf[c->cur], m, q.shift, mask, d + p, 0);
     c->launches++;
   }
   CU(c, cudaGetLastError());
-  if (c->G > 1) NC(c, g_nccl.AllReduce(d, d, (size_t)c->npasses, ncclUint32, ncclMin, c->comm, c->stream));
-  CU(c, cudaMemcpyAsync(c->host_skip, d, sizeof(unsigned) * c->npasses, cudaMemcpyDeviceToHost, c->stream));
+  if (c->G > 1) NC(c, g_nccl.AllReduce(d, d, (size_t)np, ncclUint32, ncclMin, c->comm, c->stream));
+  CU(c, cudaMemcpyAsync(c->host_skip, d, sizeof(unsigned) * np, cudaMemcpyDeviceToHost, c->stream));
   CU(c, cudaStreamSynchronize(c->stream));
-  for (int p = 0; p < c->npasses; p++) c->fuse_ok[p] = plan_pass(c, p).bits >= 12 && c->host_skip[p] >= 2048;
+  for (int p = 0; p < np; p++) c->fuse_ok[p] = plan_pass(c, k, p).bits >= 12 && c->host_skip[p] >= 2048;
   return LSB_OK;
 }
 
@@ -685,13 +703,13 @@ int plan_fusion(lsb_ctx* c) {
 //   passes: produced by the previous pass's exchange kernel), so
 //     part q:   local stable sort by the digit (compute stream)  ->  exchange (exchange stream)
 //   and the exchange of part q overlaps the local sort of part q+1.
-int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
-  const PassPlan p = plan_pass(c, digit);
+int pass_global(lsb_ctx* c, const KeyPlan& k, int digit, int* subpasses, bool fuse_next) {
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits;
   const int V = c->V;
   int rc;
   if (c->dense_ready_digit != digit) {  // nobody has counted this digit yet
-    if ((rc = count_parts(c, digit))) return rc;
+    if ((rc = count_parts(c, k, digit))) return rc;
     if ((rc = phase_mark(c, 0))) return rc;
   }
   c->dense_ready_digit = -1;
@@ -699,7 +717,7 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
     // a digit that is constant over the WHOLE array makes the pass the identity (every GPU sees the same
     // counts of all virtual ranks, so every GPU takes the same decision)
     bool constant = false;
-    if ((rc = digit_is_constant(c, digit, &constant))) return rc;
+    if ((rc = digit_is_constant(c, k, digit, &constant))) return rc;
     if (constant) {  // identity pass: every element stays where it is (sendCounts: everything to myself)
       c->skipped++;
       unsigned long long* sent = c->host_small + 140;
@@ -708,7 +726,7 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
       return phase_mark(c, 1);
     }
   }
-  if ((rc = part_offsets(c, digit))) return rc;
+  if ((rc = part_offsets(c, k, digit))) return rc;
   if ((rc = phase_mark(c, 1))) return rc;
 
   // The exchange kernel counts the NEXT pass's digit per (destination GPU, destination part) with one L2 atomic per
@@ -717,9 +735,9 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
   // counted by the shared-memory count kernel at the start of their own pass instead (one extra 16 B/element read).
   int next_nb = 0, next_shift = 0;
   // ... and wide digits that are narrow in THIS data (skewed keys), judged from a sample at the start of the sort
-  const bool has_next = fuse_next && digit + 1 < c->npasses && c->fuse_ok[digit + 1];
+  const bool has_next = fuse_next && digit + 1 < num_passes(c, k) && c->fuse_ok[digit + 1];
   if (has_next) {
-    const PassPlan q = plan_pass(c, digit + 1);
+    const PassPlan q = plan_pass(c, k, digit + 1);
     next_nb = 1 << q.bits;
     next_shift = q.shift;
     CU(c, cudaMemsetAsync(c->next_dense, 0, sizeof(unsigned) * (size_t)c->G * V * next_nb, c->stream));
@@ -737,9 +755,9 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
     const uint32_t* tiles = c->seg_tiles + 2 * (1 + q);
     const Elt* sorted;
     if (two_step) {  // low step into the scratch, high step back in place
-      if ((rc = launch_partition(c, part, m, p.shift, p.lo_bits, segs, tiles, c->bases_v + ((size_t)q * 2 + 0) * 257, c->scratch[0])))
+      if ((rc = launch_partition(c, k.korder, part, m, p.shift, p.lo_bits, segs, tiles, c->bases_v + ((size_t)q * 2 + 0) * 257, c->scratch[0])))
         return rc;
-      if ((rc = launch_partition(c, c->scratch[0], m, p.shift + p.lo_bits, p.hi_bits, segs, tiles,
+      if ((rc = launch_partition(c, k.korder, c->scratch[0], m, p.shift + p.lo_bits, p.hi_bits, segs, tiles,
                                  c->bases_v + ((size_t)q * 2 + 1) * 257, part)))
         return rc;
       sorted = part;
@@ -747,8 +765,8 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
     } else {  // one launch; its output lives in an alternating scratch until it has been exchanged
       Elt* out = c->scratch[slot];
       if (prev_x >= 0) CU(c, cudaStreamWaitEvent(c->stream, c->ev_x[prev_x], 0));  // scratch[slot] was read by that exchange
-      if (p.lo_bits) rc = launch_onepass(c, part, out, m, p.shift, p.bits, c->localbase_v + (size_t)q * nb, 0, c->tune.op_ctas_mgpu);
-      else rc = launch_partition(c, part, m, p.shift, p.hi_bits, segs, tiles, c->bases_v + ((size_t)q * 2 + 1) * 257, out);
+      if (p.lo_bits) rc = launch_onepass(c, k.korder, part, out, m, p.shift, p.bits, c->localbase_v + (size_t)q * nb, 0, c->tune.op_ctas_mgpu);
+      else rc = launch_partition(c, k.korder, part, m, p.shift, p.hi_bits, segs, tiles, c->bases_v + ((size_t)q * 2 + 1) * 257, out);
       if (rc) return rc;
       sorted = out;
       (*subpasses)++;
@@ -779,12 +797,12 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
     x.next_nb = next_nb;
     for (int i = 0; i <= LSB_MAX_PARTS; i++) x.pstart[i] = c->pstart[std::min(i, V)];
     x.next_dense = c->next_dense;
-    x.korder = c->cfg.flags;
+    x.korder = k.korder;
     // 512 threads next to partition_kernel CTAs that come and go; 256 fit beside three resident one-pass CTAs
     const int ex_threads = c->tune.ex_threads ? c->tune.ex_threads : ((c->cfg.flags & LSB_FLAG_ONE_PASS) ? 256 : 512);
     const int ex_u = c->tune.ex_u == 8 ? 8 : 4;
     const int grid = (int)std::min<int64_t>((int64_t)c->num_sms * c->tune.ex_ctas, div_ceil(m, (int64_t)ex_threads * ex_u));
-    if (ordered(c)) {
+    if (k.korder) {
       if (ex_threads == 256) exchange_vr_kernel<256, 4, true><<<grid, 256, 0, c->xstream>>>(x);
       else if (ex_u == 8) exchange_vr_kernel<512, 8, true><<<grid, 512, 0, c->xstream>>>(x);
       else exchange_vr_kernel<512, 4, true><<<grid, 512, 0, c->xstream>>>(x);
@@ -827,19 +845,19 @@ int pass_global(lsb_ctx* c, int digit, int* subpasses, bool fuse_next) {
 
 // passes [d0, d1) on one GPU: one read counts the digits of every pass, then one launch per pass
 // (LSB_FLAG_ONE_PASS) or per 8-bit step (default) that reads the shard once and writes it once
-int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
+int passes_single(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) {
   if (!(c->cfg.flags & LSB_FLAG_ONE_PASS)) {
     // two-step shape: one histogram read for all sub-digits, then one HBM -> HBM step per sub-digit
     std::vector<SubPass> subs;
     for (int d = d0; d < d1; d++) {
-      const PassPlan p = plan_pass(c, d);
+      const PassPlan p = plan_pass(c, k, d);
       if (p.lo_bits) subs.push_back({p.shift, p.lo_bits});
       subs.push_back({p.shift + p.lo_bits, p.hi_bits});
     }
     int rc;
     for (size_t s0 = 0; s0 < subs.size(); s0 += HIST_MAX_SUB) {
       const int ns = (int)std::min<size_t>(HIST_MAX_SUB, subs.size() - s0);
-      if ((rc = launch_subdigit_hist(c, c->buf[c->cur], subs.data() + s0, ns))) return rc;
+      if ((rc = launch_subdigit_hist(c, k.korder, c->buf[c->cur], subs.data() + s0, ns))) return rc;
       const bool may_skip = !(c->cfg.flags & LSB_FLAG_NO_SKIP) && c->here > 0;
       if (may_skip) {  // a digit that is constant over the shard makes its stable step the identity
         CU(c, cudaMemcpyAsync(c->host_hist, c->hist, sizeof(unsigned long long) * 256 * ns, cudaMemcpyDeviceToHost, c->stream));
@@ -852,7 +870,7 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
           for (int b = 0; b < 256; b++) constant = constant || c->host_hist[s * 256 + b] == (unsigned long long)c->here;
           if (constant) { c->skipped++; continue; }
         }
-        if ((rc = launch_partition(c, c->buf[c->cur], c->here, sp.shift, sp.bits, c->seg_start, c->seg_tiles, c->scan_out + (size_t)s * 257, c->buf[c->cur ^ 1])))
+        if ((rc = launch_partition(c, k.korder, c->buf[c->cur], c->here, sp.shift, sp.bits, c->seg_start, c->seg_tiles, c->scan_out + (size_t)s * 257, c->buf[c->cur ^ 1])))
           return rc;
         c->cur ^= 1;
         (*subpasses)++;
@@ -864,7 +882,7 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
   int shift[64], bits[64], off[64], meta[128];
   int total = 0;
   for (int i = 0; i < np; i++) {
-    const PassPlan p = plan_pass(c, d0 + i);
+    const PassPlan p = plan_pass(c, k, d0 + i);
     shift[i] = p.shift;
     bits[i] = p.bits;
     off[i] = total;
@@ -874,7 +892,7 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
   }
   int rc;
   CU(c, cudaMemsetAsync(c->hist16, 0, sizeof(unsigned long long) * total, c->stream));
-  if ((rc = launch_digit_hist(c, c->buf[c->cur], c->here, shift, bits, off, np, c->hist16, false))) return rc;
+  if ((rc = launch_digit_hist(c, k.korder, c->buf[c->cur], c->here, shift, bits, off, np, c->hist16, false))) return rc;
   if ((rc = phase_mark(c, 0))) return rc;
   for (int i = 0; i < np; i++)
     if ((rc = launch_scan(c, c->hist16 + off[i], 1 << bits[i], 1, 0, c->starts16 + off[i], nullptr))) return rc;
@@ -889,13 +907,13 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
   if ((rc = phase_mark(c, 1))) return rc;
   for (int i = 0; i < np; i++) {
     if (may_skip && c->host_skip[i]) { c->skipped++; continue; }
-    const PassPlan p = plan_pass(c, d0 + i);
+    const PassPlan p = plan_pass(c, k, d0 + i);
     const int64_t* starts = c->starts16 + off[i];
     if (p.lo_bits == 0) {
-      rc = launch_partition(c, c->buf[c->cur], c->here, p.shift, p.bits, c->seg_start, c->seg_tiles, starts, c->buf[c->cur ^ 1]);
+      rc = launch_partition(c, k.korder, c->buf[c->cur], c->here, p.shift, p.bits, c->seg_start, c->seg_tiles, starts, c->buf[c->cur ^ 1]);
       (*subpasses)++;
     } else {
-      rc = launch_onepass(c, c->buf[c->cur], c->buf[c->cur ^ 1], c->here, p.shift, p.bits, starts, 0, 0);
+      rc = launch_onepass(c, k.korder, c->buf[c->cur], c->buf[c->cur ^ 1], c->here, p.shift, p.bits, starts, 0, 0);
       (*subpasses)++;
     }
     if (rc) return rc;
@@ -904,14 +922,14 @@ int passes_single(lsb_ctx* c, int d0, int d1, int* subpasses) {
   return LSB_OK;
 }
 
-// the passes [d0, d1) of lsb_sort in the context's pass shape
-int run_passes(lsb_ctx* c, int d0, int d1, int* subpasses) {
+// the passes [d0, d1) of the plan `k` in the context's pass shape
+int run_passes(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) {
   c->dense_ready_digit = -1;
-  if (!c->two_level) return passes_single(c, d0, d1, subpasses);
-  int rc = plan_fusion(c);
+  if (!c->two_level) return passes_single(c, k, d0, d1, subpasses);
+  int rc = plan_fusion(c, k);
   if (rc) return rc;
   for (int d = d0; d < d1; d++)
-    if ((rc = pass_global(c, d, subpasses, d + 1 < d1))) return rc;
+    if ((rc = pass_global(c, k, d, subpasses, d + 1 < d1))) return rc;
   return LSB_OK;
 }
 
@@ -919,6 +937,17 @@ int check_ready(lsb_ctx* c) {
   if (!c) return LSB_ERR_ARG;
   if (c->G > 1 && !c->comm_ready) return fail(c, LSB_ERR_STATE, "world_size > 1: call lsb_comm_init first");
   return LSB_OK;
+}
+
+// lsb_sort with the plan `k`: the context's, or a narrow-key call's own for the records it packed
+int sort_shard(lsb_ctx* c, const KeyPlan& k, lsb_stats* st) {
+  CU(c, cudaSetDevice(c->cfg.device));
+  int rc = begin_call(c);
+  if (rc) return rc;
+  int subpasses = 0;
+  const int np = num_passes(c, k);
+  if ((rc = run_passes(c, k, 0, np, &subpasses))) return rc;
+  return end_call(c, st, np, subpasses);
 }
 
 // ---- lsb_sort_device: the caller's arrays <-> the shard's records --------------------------------------------------------
@@ -973,6 +1002,7 @@ int launch_pack(lsb_ctx* c, uint32_t key_type, const void* keys, const uint64_t*
   else pack_kernel<KT, false><<<grid, IO_THREADS, 0, c->stream>>>(a)
   LSB_KT_SWITCH(key_type)
 #undef LSB_KT_CALL
+  c->launches++;
   CU(c, cudaGetLastError());
   return LSB_OK;
 }
@@ -990,44 +1020,12 @@ int launch_unpack(lsb_ctx* c, int key_bytes, void* keys, uint64_t* vals) {
   if (key_bytes == 8) launch_unpack_kernel<8>(a, grid, c->stream);
   else if (key_bytes == 4) launch_unpack_kernel<4>(a, grid, c->stream);
   else launch_unpack_kernel<2>(a, grid, c->stream);
+  c->launches++;
   CU(c, cudaGetLastError());
   return LSB_OK;
 }
 
 // ---- lsb_sort_segments_device: offsets check, pack with segment ids, retag, unpack (lsb_segments.cuh) -------------------
-
-// The segment passes sort the retagged key word as a uint64, ascending: the key-order flags are lifted for their
-// duration and back in force when the scope ends, on every return path.  (The one-pass kernel's residency, taken at
-// lsb_create for the context's instantiation, holds for the plain one too: every instantiation is bounded by the same
-// __launch_bounds__ and dynamic shared memory.)
-struct PlainKeyOrder {
-  lsb_ctx* c;
-  uint32_t saved;
-  explicit PlainKeyOrder(lsb_ctx* ctx) : c(ctx), saved(ctx->cfg.flags) { c->cfg.flags &= ~KEY_ORDER_FLAGS; }
-  ~PlainKeyOrder() { c->cfg.flags = saved; }
-};
-
-// The key passes of a narrow key (bits < 64): the pack already wrote the order key into the low `bits` bits of the key
-// word, so for the guard's scope every pass reads the plan of a `bits`-bit uint64 ascending key: key_bits = bits (the
-// last digit is clamped to it: at radix 13 a 32-bit key is digits of 13, 13 and 6 bits, never 7 raw key bits),
-// npasses = ceil(bits / radix_bits) and the key-order flags lifted.  All three are back when the scope ends, on every
-// return path.  At 64 bits it changes nothing.
-struct NarrowKeyPasses {
-  lsb_ctx* c;
-  const int saved_bits, saved_npasses;
-  const uint32_t saved_flags;
-  NarrowKeyPasses(lsb_ctx* ctx, int bits) : c(ctx), saved_bits(ctx->key_bits), saved_npasses(ctx->npasses), saved_flags(ctx->cfg.flags) {
-    if (bits >= 64) return;
-    c->key_bits = bits;
-    c->npasses = (int)div_ceil(bits, c->cfg.radix_bits);
-    c->cfg.flags &= ~KEY_ORDER_FLAGS;
-  }
-  ~NarrowKeyPasses() {
-    c->key_bits = saved_bits;
-    c->npasses = saved_npasses;
-    c->cfg.flags = saved_flags;
-  }
-};
 
 // offsets[0] == 0, offsets[nseg] == count, non-decreasing: one flag read back (host_small[16], from small[60])
 int segsort_check(lsb_ctx* c, const int64_t* offsets, int64_t nseg, int64_t count, bool* ok) {
@@ -1089,32 +1087,44 @@ int launch_segsort_unpack(lsb_ctx* c, int key_bytes, void* keys, uint64_t* vals,
   return LSB_OK;
 }
 
-// the refusals the typed entry points add to the 8-byte ones; on success *key_bytes is the key width in bytes
-int check_key_type(lsb_ctx* c, const char* fn, uint32_t key_type, int* key_bytes) {
+// The checks of the two device entry points, in the order they make them: first the context, the key type and the
+// count (on success *key_bytes is the key width in bytes) ...
+int check_call(lsb_ctx* c, const char* fn, uint32_t key_type, int64_t count, int* key_bytes) {
+  int rc = check_ready(c);
+  if (rc) return rc;
   const int bits = key_type_bits(key_type);
   if (!bits) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown key_type " + std::to_string(key_type));
   if (bits < 64 && (c->cfg.flags & (LSB_FLAG_KEY_I64 | LSB_FLAG_KEY_F64)))
     return fail(c, LSB_ERR_ARG, std::string(fn) + ": a narrow key_type needs a context without LSB_FLAG_KEY_I64 / LSB_FLAG_KEY_F64");
+  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
   *key_bytes = bits / 8;
+  return LSB_OK;
+}
+
+// ... then, for count > 0 and a non-NULL keys_in, the four arrays: an output at least, each of them NULL or device memory
+// that check_device_array accepts at its own width
+int check_arrays(lsb_ctx* c, const char* fn, int key_bytes, int64_t count, const void* keys_in, const uint64_t* vals_in,
+                 const void* keys_out, const uint64_t* vals_out) {
+  if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
+  const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
+  const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
+  const int widths[4] = {key_bytes, 8, key_bytes, 8};
+  for (int i = 0; i < 4; i++) {
+    const int rc = check_device_array(c, fn, ptrs[i], names[i], count, widths[i]);
+    if (rc) return rc;
+  }
   return LSB_OK;
 }
 
 int sort_device(lsb_ctx* c, const char* fn, uint32_t key_type, const void* keys_in, const uint64_t* vals_in, void* keys_out,
                 uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
-  int rc = check_ready(c);
-  if (rc) return rc;
   int kb = 8;
-  if ((rc = check_key_type(c, fn, key_type, &kb))) return rc;
-  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
+  int rc = check_call(c, fn, key_type, count, &kb);
+  if (rc) return rc;
   CU(c, cudaSetDevice(c->cfg.device));
   if (count) {
     if (!keys_in) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in is NULL");
-    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
-    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
-    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
-    const int widths[4] = {kb, 8, kb, 8};
-    for (int i = 0; i < 4; i++)
-      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count, widths[i]))) return rc;
+    if ((rc = check_arrays(c, fn, kb, count, keys_in, vals_in, keys_out, vals_out))) return rc;
     if (keys_out && vals_out && ranges_overlap(keys_out, (size_t)count * kb, vals_out, (size_t)count * sizeof(uint64_t)))
       return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out overlap");
   }
@@ -1122,10 +1132,7 @@ int sort_device(lsb_ctx* c, const char* fn, uint32_t key_type, const void* keys_
   CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
   c->cur = 0;
   if (count && (rc = launch_pack(c, key_type, keys_in, vals_in, c->cfg.flags))) return rc;
-  {
-    NarrowKeyPasses narrow(c, kb * 8);
-    if ((rc = lsb_sort(c, st))) return rc;
-  }
+  if ((rc = sort_shard(c, key_type_plan(c, key_type), st))) return rc;
   if (count && (rc = launch_unpack(c, kb, keys_out, vals_out))) return rc;
   CU(c, cudaStreamSynchronize(c->stream));
   return LSB_OK;
@@ -1136,11 +1143,9 @@ int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const vo
                          uint32_t seg_flags, void* stream, lsb_stats* st) {
   if (!c) return LSB_ERR_ARG;
   if (c->G > 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": one GPU only (world_size > 1)");
-  int rc = check_ready(c);
-  if (rc) return rc;
   int kb = 8;
-  if ((rc = check_key_type(c, fn, key_type, &kb))) return rc;
-  if (count != c->here) return fail(c, LSB_ERR_ARG, std::string(fn) + ": count must equal this shard's size");
+  int rc = check_call(c, fn, key_type, count, &kb);
+  if (rc) return rc;
   if (num_segments < 1) return fail(c, LSB_ERR_ARG, std::string(fn) + ": num_segments must be >= 1");
   if (seg_flags & ~LSB_SEG_LOCAL_INDEX) return fail(c, LSB_ERR_ARG, std::string(fn) + ": unknown seg_flags");
   const SegsortLayout lay = segsort_layout(count, num_segments, c->cfg.radix_bits);
@@ -1152,21 +1157,17 @@ int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const vo
   const size_t off_bytes = (size_t)(num_segments + 1) * sizeof(int64_t);
   if (count) {
     if (!keys_in || !seg_offsets) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_in or seg_offsets is NULL");
-    if (!keys_out && !vals_out) return fail(c, LSB_ERR_ARG, std::string(fn) + ": keys_out and vals_out are both NULL");
-    const void* ptrs[4] = {keys_in, vals_in, keys_out, vals_out};
-    const char* names[4] = {"keys_in", "vals_in", "keys_out", "vals_out"};
-    const int widths[4] = {kb, 8, kb, 8};
-    for (int i = 0; i < 4; i++)
-      if ((rc = check_device_array(c, fn, ptrs[i], names[i], count, widths[i]))) return rc;
+    if ((rc = check_arrays(c, fn, kb, count, keys_in, vals_in, keys_out, vals_out))) return rc;
     if ((rc = check_device_array(c, fn, seg_offsets, "seg_offsets", num_segments + 1))) return rc;
     // keys_in is consumed by the pack, so keys_out may alias it; vals_in and the offsets are read by the unpack
     const void* outs[2] = {keys_out, vals_out};
+    const char* names[2] = {"keys_out", "vals_out"};
     const size_t out_bytes[2] = {kbytes, bytes};
     for (int i = 0; i < 2; i++) {
       if (!outs[i]) continue;
       if ((i == 0 && vals_out && ranges_overlap(keys_out, kbytes, vals_out, bytes)) ||
           (vals_in && ranges_overlap(outs[i], out_bytes[i], vals_in, bytes)) || ranges_overlap(outs[i], out_bytes[i], seg_offsets, off_bytes))
-        return fail(c, LSB_ERR_ARG, std::string(fn) + ": " + names[2 + i] + " overlaps another output, vals_in or seg_offsets");
+        return fail(c, LSB_ERR_ARG, std::string(fn) + ": " + names[i] + " overlaps another output, vals_in or seg_offsets");
     }
   }
   CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
@@ -1182,23 +1183,20 @@ int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const vo
   if (count) {  // one segment: lsb_sort_device's records, {key word, vals_in or the index}
     rc = lay.segbits ? launch_segsort_pack(c, key_type, keys_in, seg_offsets, num_segments, lay.idxbits, c->cfg.flags)
                      : launch_pack(c, key_type, keys_in, vals_in, c->cfg.flags);
-    if (lay.segbits == 0) c->launches++;
     if (rc) return rc;
   }
-  int subpasses = 0, key_passes = 0;
-  {
-    NarrowKeyPasses narrow(c, kb * 8);
-    key_passes = c->npasses;
-    if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
-  }
+  const KeyPlan keys = key_type_plan(c, key_type);
+  const int key_passes = num_passes(c, keys);
+  int subpasses = 0;
+  if ((rc = run_passes(c, keys, 0, key_passes, &subpasses))) return rc;
   if (lay.segbits) {
     if (count && (rc = launch_segsort_retag(c, lay.idxbits, lay.segw))) return rc;
-    PlainKeyOrder plain(c);
-    if ((rc = run_passes(c, 0, lay.passes, &subpasses))) return rc;
+    // the segment passes sort the low digits of the retagged key word as a uint64, ascending
+    if ((rc = run_passes(c, KeyPlan{64, 0}, 0, lay.passes, &subpasses))) return rc;
   }
   if (count) {
-    if (lay.segbits) rc = launch_segsort_unpack(c, kb, keys_out, vals_out, vals_in, seg_offsets, seg_flags & LSB_SEG_LOCAL_INDEX, lay.segw);
-    else if ((rc = launch_unpack(c, kb, keys_out, vals_out)) == LSB_OK) c->launches++;
+    rc = lay.segbits ? launch_segsort_unpack(c, kb, keys_out, vals_out, vals_in, seg_offsets, seg_flags & LSB_SEG_LOCAL_INDEX, lay.segw)
+                     : launch_unpack(c, kb, keys_out, vals_out);
     if (rc) return rc;
   }
   return end_call(c, st, key_passes + lay.passes, subpasses);
@@ -1292,7 +1290,7 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   if (c->here < 0) c->here = 0;
   c->first = c->per * c->my;
   c->per_stream = std::max<int64_t>(div_ceil(c->n, c->cfg.ranks), 1);
-  c->npasses = (64 + c->cfg.radix_bits - 1) / c->cfg.radix_bits;
+  c->npasses = num_passes(c, context_plan(c));
 
 #define CUC(expr)                                                                        \
   do {                                                                                   \
@@ -1356,9 +1354,9 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   // every claimed one-pass item must belong to a resident CTA: residency of the instantiation this context launches
   if (c->tune.op_cfg == 1) {
     c->op_tile = TileCfgS::TILE;
-    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, ordered(c) ? onepass_kernel<TileCfgS, false, true> : onepass_kernel<TileCfgS, true, false>, TileCfgS::THREADS, TileCfgS::SMEM));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, context_plan(c).korder ? onepass_kernel<TileCfgS, false, true> : onepass_kernel<TileCfgS, true, false>, TileCfgS::THREADS, TileCfgS::SMEM));
   } else {
-    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, ordered(c) ? onepass_kernel<TileCfg, false, true> : onepass_kernel<TileCfg, true, false>, TileCfg::THREADS, TileCfg::SMEM));
+    CUC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c->op_resident, context_plan(c).korder ? onepass_kernel<TileCfg, false, true> : onepass_kernel<TileCfg, true, false>, TileCfg::THREADS, TileCfg::SMEM));
   }
   if (c->tune.op_persist > 0) {
     int max_persist = 0;
@@ -1559,7 +1557,7 @@ int lsb_num_passes(const lsb_ctx* c) { return c ? c->npasses : LSB_ERR_ARG; }
 
 int lsb_digit_bits(const lsb_ctx* c, int digit) {
   if (!c || digit < 0 || digit >= c->npasses) return LSB_ERR_ARG;
-  return plan_pass(c, digit).bits;
+  return plan_pass(c, context_plan(c), digit).bits;
 }
 
 int lsb_generate(lsb_ctx* c) {
@@ -1625,13 +1623,8 @@ int lsb_host_free(void* ptr) {
 }
 
 int lsb_sort(lsb_ctx* c, lsb_stats* st) {
-  int rc = check_ready(c);
-  if (rc) return rc;
-  CU(c, cudaSetDevice(c->cfg.device));
-  if ((rc = begin_call(c))) return rc;
-  int subpasses = 0;
-  if ((rc = run_passes(c, 0, c->npasses, &subpasses))) return rc;
-  return end_call(c, st, c->npasses, subpasses);
+  const int rc = check_ready(c);
+  return rc ? rc : sort_shard(c, context_plan(c), st);
 }
 
 int lsb_pass(lsb_ctx* c, int digit, lsb_stats* st) {
@@ -1642,8 +1635,8 @@ int lsb_pass(lsb_ctx* c, int digit, lsb_stats* st) {
   if ((rc = begin_call(c))) return rc;
   c->dense_ready_digit = -1;
   int subpasses = 0;
-  if (!c->two_level) rc = passes_single(c, digit, digit + 1, &subpasses);
-  else rc = pass_global(c, digit, &subpasses, false);
+  if (!c->two_level) rc = passes_single(c, context_plan(c), digit, digit + 1, &subpasses);
+  else rc = pass_global(c, context_plan(c), digit, &subpasses, false);
   if (rc) return rc;
   return end_call(c, st, 1, subpasses);
 }
@@ -1689,10 +1682,11 @@ int lsb_sort_segments_device_typed(lsb_ctx* c, uint32_t key_type, const void* ke
 int lsb_histogram(lsb_ctx* c, int digit, int64_t* host_counts) {
   if (!c || !host_counts || digit < 0 || digit >= c->npasses) return fail(c, LSB_ERR_ARG, "lsb_histogram: argument");
   CU(c, cudaSetDevice(c->cfg.device));
-  const PassPlan p = plan_pass(c, digit);
+  const KeyPlan k = context_plan(c);
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits, zero = 0;
   CU(c, cudaMemsetAsync(c->hist16, 0, sizeof(unsigned long long) * nb, c->stream));
-  int rc = launch_digit_hist(c, c->buf[c->cur], c->here, &p.shift, &p.bits, &zero, 1, c->hist16, false);
+  int rc = launch_digit_hist(c, k.korder, c->buf[c->cur], c->here, &p.shift, &p.bits, &zero, 1, c->hist16, false);
   if (rc) return rc;
   CU(c, cudaMemcpyAsync(host_counts, c->hist16, sizeof(int64_t) * nb, cudaMemcpyDeviceToHost, c->stream));
   CU(c, cudaStreamSynchronize(c->stream));
@@ -1703,7 +1697,7 @@ int lsb_histogram(lsb_ctx* c, int digit, int64_t* host_counts) {
     int ns = 0;
     if (p.lo_bits) subs[ns++] = {p.shift, p.lo_bits};
     subs[ns++] = {p.shift + p.lo_bits, p.hi_bits};
-    if ((rc = launch_subdigit_hist(c, c->buf[c->cur], subs, ns))) return rc;
+    if ((rc = launch_subdigit_hist(c, k.korder, c->buf[c->cur], subs, ns))) return rc;
     CU(c, cudaMemcpyAsync(c->host_hist, c->hist, sizeof(unsigned long long) * 256 * ns, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     std::vector<unsigned long long> lo(256, 0), hi(256, 0);
@@ -1725,17 +1719,18 @@ int lsb_starts(lsb_ctx* c, int digit, int64_t* host_starts) {
   if (rc) return rc;
   if (!host_starts || digit < 0 || digit >= c->npasses) return fail(c, LSB_ERR_ARG, "lsb_starts: argument");
   CU(c, cudaSetDevice(c->cfg.device));
-  const PassPlan p = plan_pass(c, digit);
+  const KeyPlan k = context_plan(c);
+  const PassPlan p = plan_pass(c, k, digit);
   const int nb = 1 << p.bits, zero = 0;
   const int64_t* src;
   if (c->two_level) {
     // a shard's first element of digit d is its first part's first element of digit d
-    if ((rc = count_parts(c, digit))) return rc;
-    if ((rc = part_offsets(c, digit))) return rc;
+    if ((rc = count_parts(c, k, digit))) return rc;
+    if ((rc = part_offsets(c, k, digit))) return rc;
     src = c->mybase_v;
   } else {
     CU(c, cudaMemsetAsync(c->hist16, 0, sizeof(unsigned long long) * nb, c->stream));
-    if ((rc = launch_digit_hist(c, c->buf[c->cur], c->here, &p.shift, &p.bits, &zero, 1, c->hist16, false))) return rc;
+    if ((rc = launch_digit_hist(c, k.korder, c->buf[c->cur], c->here, &p.shift, &p.bits, &zero, 1, c->hist16, false))) return rc;
     if ((rc = launch_scan(c, c->hist16, nb, 1, 0, c->mybase, nullptr))) return rc;
     src = c->mybase;
   }
@@ -1749,7 +1744,8 @@ static int local_verify(lsb_ctx* c) {
   CU(c, cudaMemsetAsync(c->small + 40, 0, 8 * sizeof(unsigned long long), c->stream));
   if (c->here > 0) {
     int grid = (int)std::min<int64_t>((int64_t)c->num_sms * 8, div_ceil(c->here, 256));
-    if (ordered(c)) verify_kernel<true><<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40, c->cfg.flags);
+    const uint32_t korder = context_plan(c).korder;
+    if (korder) verify_kernel<true><<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40, korder);
     else verify_kernel<false><<<grid, 256, 0, c->stream>>>(c->buf[c->cur], c->here, c->small + 40, 0);
     CU(c, cudaGetLastError());
   }

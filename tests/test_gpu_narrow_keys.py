@@ -180,6 +180,51 @@ def test_reused_sorter(flags):
             assert torch.equal(k.view(torch.int16), k2.view(torch.int16)) and torch.equal(v, v2)
 
 
+@pytest.mark.parametrize("flags", [0, OP, TL])
+def test_narrow_calls_leave_the_context_plan(flags):
+    """Typed calls sort by their own plan (a float32 key at radix 13 is digits of 13, 13 and 6 bits, ascending in the
+    packed word) and leave the context's (five digits of a 64-bit word, descending): interleaved on one sorter, every
+    call returns what it returns on a fresh sorter."""
+    n, radix = P.SUPERTILE + 1, 13
+    rng = np.random.default_rng(18)
+    bits = NK.special_mix(n, "float32", seed=18)
+    kt = NK.to_device(torch, bits, "float32")
+    offsets = torch.from_numpy(np.concatenate([[0], np.sort(rng.integers(0, n, 99)), [n]]).astype(np.int64)).cuda()
+    recs = np.empty(n, dtype=L.ELT)
+    recs["key"] = KO.special_mix(n, seed=18)
+    recs["val"] = np.arange(n)
+
+    def typed(s):
+        k, v, st = s.sort_device(kt)
+        return NK.bits_of(torch, k), v.cpu().numpy(), st.passes
+
+    def segments(s):
+        k, v, st = s.sort_segments(kt, offsets)
+        return NK.bits_of(torch, k), v.cpu().numpy(), st.passes
+
+    def records(s):
+        s.upload(recs)
+        st = s.my_sort()
+        return s.download().view(np.uint64), st.passes
+
+    def plan(s):
+        return s.num_passes(), [s.digit_bits(d) for d in range(s.num_passes())]
+
+    def sorter():
+        return lsb.DistributedSorter(n, ranks=1, radix_bits=radix, flags=flags | DESC, key_dtype=torch.float32)
+
+    with sorter() as s:
+        for call in [typed, records, segments, plan, records, typed, segments, records, plan]:
+            got = call(s)
+            with sorter() as fresh:
+                want = call(fresh)
+            assert all(np.array_equal(a, b) for a, b in zip(got, want)), call.__name__
+        assert plan(s) == (5, [13, 13, 13, 13, 12])
+        k, v, passes = typed(s)
+        perm = NK.argsort(bits, "float32", True)
+        assert np.array_equal(k, bits[perm]) and np.array_equal(v, perm) and passes == 3
+
+
 def test_waits_for_the_callers_stream():
     n = (1 << 20) + 7
     bits = NK.special_mix(n, "float32", seed=11)
