@@ -18,6 +18,7 @@ from .lsbsort import (  # noqa: F401
     abi_symbols,
     comm_unique_id,
     header_symbols,
+    lexsort,
     library_path,
     load_library,
     sort,

@@ -27,6 +27,7 @@
 #include "lsb_onepass.cuh"
 #include "lsb_io.cuh"
 #include "lsb_segments.cuh"
+#include "lsb_lexsort.cuh"
 
 #include <nccl.h>  // types only: the library itself is bound at run time, see NcclApi
 #include <dlfcn.h>
@@ -1202,6 +1203,101 @@ int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const vo
   return end_call(c, st, key_passes + lay.passes, subpasses);
 }
 
+// ---- lsb_lexsort_device: a round's pack, its passes, ..., the unpack (lsb_lexsort.cuh) ----------------------------------
+
+// the pack of round `r` of `cols`: into buf[0] for the first round, in place on buf[cur] for every later one
+int launch_lexsort_pack(lsb_ctx* c, const lsb_key_column* cols, const LexsortRound& r, bool gather) {
+  LexsortPackArgs a{};
+  int shift = 0;
+  for (int i = 0; i < r.ncols; i++) {
+    const lsb_key_column& k = cols[r.first + i];
+    a.col[i] = LexsortColumn{k.keys, k.key_type, k.flags, shift};
+    shift += key_type_bits(k.key_type);
+  }
+  a.buf = c->buf[gather ? c->cur : 0];
+  a.count = c->here;
+  const int grid = io_grid(c, c->here);
+#define LSB_LEX_PACK(N)                                                          \
+  if (gather) lexsort_pack_kernel<true, N><<<grid, IO_THREADS, 0, c->stream>>>(a); \
+  else lexsort_pack_kernel<false, N><<<grid, IO_THREADS, 0, c->stream>>>(a)
+  switch (r.ncols) {  // 1 .. LEXSORT_ROUND_COLUMNS (lexsort_rounds)
+    case 1: LSB_LEX_PACK(1); break;
+    case 2: LSB_LEX_PACK(2); break;
+    case 3: LSB_LEX_PACK(3); break;
+    default: LSB_LEX_PACK(4); break;
+  }
+#undef LSB_LEX_PACK
+  c->launches++;
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+int launch_lexsort_unpack(lsb_ctx* c, const uint64_t* vals_in, uint64_t* vals_out) {
+  if (!vals_in) return launch_unpack(c, 8, nullptr, vals_out);  // the input index in the val word
+  const LexsortUnpackArgs a{c->buf[c->cur], vals_in, vals_out, c->here};
+  lexsort_unpack_kernel<<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(a);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  return LSB_OK;
+}
+
+int lexsort_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32_t K, const uint64_t* vals_in,
+                   uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
+  if (!c) return LSB_ERR_ARG;
+  const std::string f(fn);
+  if (c->G > 1) return fail(c, LSB_ERR_ARG, f + ": one GPU only (world_size > 1)");
+  if (c->cfg.flags & KEY_ORDER_FLAGS)
+    return fail(c, LSB_ERR_ARG, f + ": the context has key-order flags (KEY_I64 / KEY_F64 / DESCENDING); the columns "
+                                    "carry their own");
+  if (K < 1 || !cols) return fail(c, LSB_ERR_ARG, f + ": needs num_columns >= 1 and a columns array");
+  std::vector<int> widths(K);
+  for (int i = 0; i < K; i++) {
+    const std::string col = f + ": column " + std::to_string(i);
+    widths[i] = key_type_bits(cols[i].key_type);
+    if (!widths[i]) return fail(c, LSB_ERR_ARG, col + ": unknown key_type " + std::to_string(cols[i].key_type));
+    const uint32_t allowed = widths[i] == 64 ? KEY_ORDER_FLAGS : LSB_FLAG_DESCENDING;
+    const uint32_t both = LSB_FLAG_KEY_I64 | LSB_FLAG_KEY_F64;
+    if ((cols[i].flags & ~allowed) || (cols[i].flags & both) == both)
+      return fail(c, LSB_ERR_ARG, col + ": flags " + std::to_string(cols[i].flags) + " are not " +
+                                      (widths[i] == 64 ? "DESCENDING plus at most one of KEY_I64 / KEY_F64" : "DESCENDING or 0"));
+  }
+  if (count != c->here) return fail(c, LSB_ERR_ARG, f + ": count must equal this shard's size");
+  std::vector<LexsortRound> rounds(K);
+  const int nr = lexsort_rounds(widths.data(), K, c->cfg.radix_bits, rounds.data());
+  CU(c, cudaSetDevice(c->cfg.device));
+  const size_t bytes = (size_t)count * sizeof(uint64_t);
+  if (count) {
+    for (int i = 0; i < K; i++) {
+      const std::string name = "column " + std::to_string(i);
+      if (!cols[i].keys) return fail(c, LSB_ERR_ARG, f + ": " + name + ": keys is NULL");
+      int rc = check_device_array(c, fn, cols[i].keys, name.c_str(), count, widths[i] / 8);
+      if (rc) return rc;
+    }
+    if (!vals_out) return fail(c, LSB_ERR_ARG, f + ": vals_out is NULL");
+    int rc = check_device_array(c, fn, vals_in, "vals_in", count);
+    if (!rc) rc = check_device_array(c, fn, vals_out, "vals_out", count);
+    if (rc) return rc;
+    if (vals_in && ranges_overlap(vals_out, bytes, vals_in, bytes)) return fail(c, LSB_ERR_ARG, f + ": vals_out overlaps vals_in");
+    for (int i = 0; i < K; i++)
+      if (ranges_overlap(vals_out, bytes, cols[i].keys, (size_t)count * (widths[i] / 8)))
+        return fail(c, LSB_ERR_ARG, f + ": vals_out overlaps column " + std::to_string(i));
+  }
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  int rc = begin_call(c);
+  if (rc) return rc;
+  c->cur = 0;
+  int passes = 0, subpasses = 0;
+  for (int r = 0; r < nr; r++) {
+    // the round's word holds its order keys: its passes sort the low `bits` bits as a uint64, ascending
+    if (count && (rc = launch_lexsort_pack(c, cols, rounds[r], r > 0))) return rc;
+    if ((rc = run_passes(c, KeyPlan{rounds[r].bits, 0}, 0, rounds[r].passes, &subpasses))) return rc;
+    passes += rounds[r].passes;
+  }
+  if (count && (rc = launch_lexsort_unpack(c, vals_in, vals_out))) return rc;
+  return end_call(c, st, passes, subpasses);
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1676,6 +1772,11 @@ int lsb_sort_segments_device_typed(lsb_ctx* c, uint32_t key_type, const void* ke
                                    int64_t num_segments, uint32_t seg_flags, void* stream, lsb_stats* st) {
   return sort_segments_device(c, "lsb_sort_segments_device_typed", key_type, keys_in, vals_in, keys_out, vals_out, count,
                               seg_offsets, num_segments, seg_flags, stream, st);
+}
+
+int lsb_lexsort_device(lsb_ctx* c, const lsb_key_column* columns, int32_t num_columns, const uint64_t* vals_in,
+                       uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
+  return lexsort_device(c, "lsb_lexsort_device", columns, num_columns, vals_in, vals_out, count, stream, st);
 }
 
 // The two test hooks run the PRODUCTION count and scan kernels of the pass shape in use.

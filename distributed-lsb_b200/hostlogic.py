@@ -130,6 +130,23 @@ def segsort_layout(count, num_segments, radix_bits):
     return idxbits, segbits, segw, passes, segw + idxbits <= 64
 
 
+
+def lexsort_rounds(widths, radix_bits):
+    """rounds of a sort by key columns of widths 64 / 32 / 16 bits, least significant first (lexsort_rounds in
+    csrc/lsb_lexsort.cuh): [(first, ncols, bits, passes)].  From column 0 on, the next column joins the current round while
+    the round's summed width stays <= 64 and it holds fewer than 4 columns; bits is that sum, passes = ceil(bits / radix).
+    Column first + c sits at the summed widths of the round's columns below it.  [] for no columns, a radix outside
+    1..16 or another width."""
+    if not widths or not 1 <= radix_bits <= 16 or any(w not in (16, 32, 64) for w in widths):
+        return []
+    rounds = []
+    for c, w in enumerate(widths):
+        if not rounds or rounds[-1][2] + w > 64 or rounds[-1][1] == 4:
+            rounds.append([c, 0, 0])
+        rounds[-1][1] += 1
+        rounds[-1][2] += w
+    return [(first, n, bits, div_ceil(bits, radix_bits)) for first, n, bits in rounds]
+
 # ---- the one-pass kernel's work order (csrc/lsb_onepass.cuh), restated for tests ---------------------------------
 def onepass_ticket(t, nsuper, t1, lead, tiles_last=None):
     """ticket t of the one-pass kernel -> ("K1", supertile, tile) | ("K2", supertile, segment) | None (no such item).

@@ -60,6 +60,11 @@ class Stats(ctypes.Structure):
                 ("kernel_launches", ctypes.c_int64)]
 
 
+class KeyColumn(ctypes.Structure):
+    """lsb_key_column: one key column of lsb_lexsort_device"""
+    _fields_ = [("keys", ctypes.c_void_p), ("key_type", ctypes.c_uint32), ("flags", ctypes.c_uint32)]
+
+
 class Verify(ctypes.Structure):
     _fields_ = [("order_violations", ctypes.c_int64), ("elements", ctypes.c_int64),
                 ("checksum", ctypes.c_uint64 * 4)]
@@ -116,6 +121,7 @@ def load_library():
     L.lsb_sort_device_typed.argtypes = [vp, ctypes.c_uint32, vp, vp, vp, vp, i64, vp, ctypes.POINTER(Stats)]
     L.lsb_sort_segments_device_typed.argtypes = [vp, ctypes.c_uint32, vp, vp, vp, vp, i64, vp, i64, ctypes.c_uint32, vp,
                                                  ctypes.POINTER(Stats)]
+    L.lsb_lexsort_device.argtypes = [vp, ctypes.POINTER(KeyColumn), ctypes.c_int32, vp, vp, i64, vp, ctypes.POINTER(Stats)]
     L.lsb_histogram.argtypes = [vp, ci, vp]
     L.lsb_starts.argtypes = [vp, ci, vp]
     L.lsb_num_passes.argtypes = [vp]
@@ -350,6 +356,40 @@ class DistributedSorter:
             self._check(self._L.lsb_sort_device_typed(self._ctx, key_type, *args), "lsb_sort_device_typed")
         return (keys_out if keys_out is not False else None), (vals_out if vals_out is not False else None), st
 
+    def lexsort_device(self, columns, vals=None, vals_out=None, descending=False, stream=None):
+        """The stable sort by several key columns (lsb_lexsort_device), np.lexsort's convention: columns[0] is the least
+        significant key, columns[-1] the primary.  `columns`: a sequence of 1-D contiguous CUDA tensors of `here`
+        elements on this sorter's device, each of uint64, int64, float64, uint32, int32, float32, uint16, int16, float16
+        or bfloat16 (the sorter's own key_dtype and flags play no part, and it must have no key-order flags).
+        `descending`: a bool for every column, or one bool per column.  Each column sorts in numpy's and torch's order:
+        NaNs last (first when descending), -0.0 == +0.0; elements equal in every column keep their input order.
+        `vals`: 8-byte tensor like a column, or None for the input index (torch.int64: what np.lexsort returns).
+        `vals_out`: a tensor to write, or None to allocate one.  Stream as in sort_device.  Returns (vals_out, Stats)."""
+        torch = _torch()
+        n = self.here
+        cols = _check_columns(torch, columns, n, self.device)
+        desc = _check_descending(descending, len(cols))
+        if vals is not None:
+            _check_vector(torch, vals, "vals", n, self.device)
+        if vals_out is None:
+            vals_out = torch.empty_like(vals) if vals is not None else torch.empty(n, dtype=torch.int64, device=cols[0].device)
+        else:
+            _check_vector(torch, vals_out, "vals_out", n, self.device)
+        if stream is None:
+            stream = torch.cuda.current_stream(cols[0].device)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        spec = (KeyColumn * len(cols))()
+        for c, (t, d) in enumerate(zip(cols, desc)):
+            narrow = _narrow_key_type(torch, t.dtype)
+            spec[c].keys = t.data_ptr() or None
+            spec[c].key_type = narrow if narrow is not None else KEY_CONTEXT
+            spec[c].flags = (0 if narrow is not None else _key_dtype_flags(torch)[t.dtype]) | (FLAG_DESCENDING if d else 0)
+        st = Stats()
+        ptr = lambda t: t.data_ptr() or None if t is not None else None  # noqa: E731
+        self._check(self._L.lsb_lexsort_device(self._ctx, spec, len(cols), ptr(vals), ptr(vals_out), n, handle,
+                                               ctypes.byref(st)), "lsb_lexsort_device")
+        return vals_out, st
+
     # -- test hooks -----------------------------------------------------------------------
     def num_passes(self):
         return self._L.lsb_num_passes(self._ctx)
@@ -518,6 +558,68 @@ def _sort_segments_1d(torch, keys, offsets, vals, descending, local_index):
     with DistributedSorter(keys.numel(), ranks=1, device=keys.device.index, flags=flags) as s:
         k, v, _ = s.sort_segments(keys, offsets, vals, local_index=local_index)
     return k, v
+
+
+def _check_columns(torch, columns, n=None, device=None):
+    """the key columns of a lexsort as a list: TypeError / ValueError unless `columns` is a non-empty sequence (not a
+    tensor) of 1-D contiguous CUDA tensors of one of the ten key dtypes, of n elements on `device` when given"""
+    if isinstance(columns, torch.Tensor) or not isinstance(columns, (list, tuple)):
+        raise TypeError(f"columns must be a list or tuple of tensors, not {type(columns).__name__}")
+    if not columns:
+        raise ValueError("columns is empty: a lexsort needs at least one key column")
+    for c, t in enumerate(columns):
+        if not isinstance(t, torch.Tensor):
+            raise TypeError(f"columns[{c}] must be a torch.Tensor, not {type(t).__name__}")
+        if t.dtype not in _key_dtype_flags(torch) and _narrow_key_type(torch, t.dtype) is None:
+            raise TypeError(f"columns[{c}] must be torch.uint64, int64, float64, torch.{', torch.'.join(NARROW_KEY_TYPES)}, "
+                            f"not {t.dtype}")
+        _check_vector(torch, t, f"columns[{c}]", n, device, dtype=t.dtype)
+    return list(columns)
+
+
+def _check_descending(descending, k):
+    """one bool per column from a bool or a sequence of k bools"""
+    if isinstance(descending, bool):
+        return [descending] * k
+    if not isinstance(descending, (list, tuple)) or not all(isinstance(d, bool) for d in descending):
+        raise TypeError(f"descending must be a bool or a list of bools, not {descending!r}")
+    if len(descending) != k:
+        raise ValueError(f"descending has {len(descending)} entries for {k} columns")
+    return list(descending)
+
+
+def lexsort(keys, descending=False, vals=None):
+    """np.lexsort for CUDA tensors, on their GPU, with no host copy: the permutation that sorts stably by the last key,
+    then the one before it, ..., then the first.  `keys`: a list or tuple of 1-D CUDA tensors of one length on one
+    device, or a 2-D CUDA tensor whose rows are the keys; each of uint64, int64, float64, uint32, int32, float32, uint16,
+    int16, float16 or bfloat16 (they may differ).  `descending`: a bool, or one bool per key.  Every key sorts in numpy's
+    and torch's order (NaNs last, first when descending; -0.0 == +0.0), and elements equal in every key keep their input
+    order.  Returns int64 indices, or `vals` (a tensor of 8-byte elements, one per key element) permuted.  Makes a
+    one-GPU sorter for the call."""
+    torch = _torch()
+    if isinstance(keys, torch.Tensor):
+        if keys.dim() != 2:
+            raise ValueError(f"keys must be a 2-D tensor (one key per row) or a list of 1-D tensors, not {keys.dim()}-D")
+        keys = list(keys.unbind(0))
+    if not isinstance(keys, (list, tuple)):
+        raise TypeError(f"keys must be a list or tuple of tensors or a 2-D tensor, not {type(keys).__name__}")
+    if not keys:
+        raise ValueError("lexsort needs at least one key")
+    keys = [k.contiguous() if isinstance(k, torch.Tensor) else k for k in keys]
+    _check_columns(torch, keys)
+    n, dev = keys[0].numel(), keys[0].device
+    for c, k in enumerate(keys):
+        if k.numel() != n or k.device != dev:
+            raise ValueError(f"keys[{c}] has {k.numel()} elements on {k.device}, keys[0] {n} on {dev}")
+    desc = _check_descending(descending, len(keys))
+    if vals is not None:
+        if not isinstance(vals, torch.Tensor):
+            raise TypeError(f"vals must be a torch.Tensor, not {type(vals).__name__}")
+        vals = vals.contiguous()
+        _check_vector(torch, vals, "vals", n, dev.index)
+    with DistributedSorter(n, ranks=1, device=dev.index) as s:
+        v, _ = s.lexsort_device(keys, vals, descending=desc)
+    return v
 
 
 def sort(input, dim=-1, descending=False, stable=False):

@@ -292,6 +292,41 @@ int lsb_sort_segments_device_typed(lsb_ctx* ctx, uint32_t key_type, const void* 
                                    void* keys_out, uint64_t* vals_out, int64_t count, const int64_t* seg_offsets,
                                    int64_t num_segments, uint32_t seg_flags, void* stream, lsb_stats* stats);
 
+/* One key column of lsb_lexsort_device.  An 8-byte column has key_type LSB_KEY_CONTEXT and names its type through its
+ * own flags (uint64, LSB_FLAG_KEY_I64 or LSB_FLAG_KEY_F64), never through the context's. */
+typedef struct lsb_key_column {
+  const void* keys;   /* count keys of key_type, device memory aligned to their width                     */
+  uint32_t key_type;  /* LSB_KEY_U32 .. LSB_KEY_BF16, or LSB_KEY_CONTEXT: an 8-byte key whose type the
+                         column's own flags name (uint64, LSB_FLAG_KEY_I64, LSB_FLAG_KEY_F64)               */
+  uint32_t flags;     /* LSB_FLAG_DESCENDING, plus LSB_FLAG_KEY_I64 or LSB_FLAG_KEY_F64 for 8-byte columns    */
+} lsb_key_column;
+
+/* Sort by several key columns on device memory, np.lexsort's convention: columns[0] is the least significant key and
+ * columns[num_columns - 1] the primary.  The result is the permutation j that sorts stably by
+ *   (order_{K-1}(col_{K-1}[j]), ..., order_1(col_1[j]), order_0(col_0[j])),
+ * order_c being the key order above of the column's type under its own flags: NaNs last (first when the column is
+ * descending), -0.0 == +0.0, a descending column the complement of its order key, and elements equal in every column
+ * in input order.  vals_out[i] is vals_in[j[i]], or without vals_in the input index j[i] itself (what np.lexsort
+ * returns).  The columns are never rewritten.
+ * Method: consecutive columns from columns[0] on share one key word while their widths (64 / 32 / 16 bits) sum to at
+ * most 64 and a word holds at most 4 of them; such a round is sorted by ceil(bits / radix_bits) stable passes on its
+ * packed order keys (uint64 ascending, the context's pass shape and skip rule), the least significant round first.
+ * Each later round repacks the records where they stand, reading its columns at the input index each record carries.
+ * So (int32, float32) or (bfloat16, int16, int32) take the 4 passes of one 64-bit sort at radix 16, (int64, int64) two
+ * rounds of 4.  stats covers the whole call: passes and skipped count the passes of every round.
+ * The contract of lsb_sort_segments_device otherwise: one GPU, count == here, the library's stream waits on `stream`,
+ * synchronous on return, and with count == 0 no device pointer is looked at.  Afterwards the shard holds internal
+ * records: what lsb_download, lsb_checksum and lsb_verify_device report is unspecified until the next sort.
+ * LSB_ERR_ARG, with a message naming the column where one applies, in this order: world_size > 1; a context with
+ * LSB_FLAG_KEY_I64, LSB_FLAG_KEY_F64 or LSB_FLAG_DESCENDING (the order comes from the columns only; the pass-shape
+ * flags and radix_bits apply as usual); num_columns < 1 or columns == NULL; an unknown key_type; column flags other
+ * than LSB_FLAG_DESCENDING (narrow column) or LSB_FLAG_DESCENDING plus one of LSB_FLAG_KEY_I64 / LSB_FLAG_KEY_F64
+ * (8-byte column); count != here; and for count > 0: a column with keys == NULL, or not aligned to its width, not
+ * device memory of the context's device, or overlapping the context's shards; vals_in failing the same checks at 8
+ * bytes; vals_out == NULL or failing them; vals_out overlapping vals_in or any column. */
+int lsb_lexsort_device(lsb_ctx* ctx, const lsb_key_column* columns, int32_t num_columns, const uint64_t* vals_in,
+                       uint64_t* vals_out, int64_t count, void* stream, lsb_stats* stats);
+
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
 /* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard; d is the
