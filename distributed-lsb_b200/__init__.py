@@ -26,4 +26,6 @@ from .lsbsort import (  # noqa: F401
     sort_segments,
     sort_tensor,
     tune,
+    unique,
+    unique_consecutive,
 )

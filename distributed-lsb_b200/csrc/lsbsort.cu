@@ -28,6 +28,7 @@
 #include "lsb_io.cuh"
 #include "lsb_segments.cuh"
 #include "lsb_lexsort.cuh"
+#include "lsb_unique.cuh"
 
 #include <nccl.h>  // types only: the library itself is bound at run time, see NcclApi
 #include <dlfcn.h>
@@ -1206,14 +1207,19 @@ int sort_segments_device(lsb_ctx* c, const char* fn, uint32_t key_type, const vo
 // ---- lsb_lexsort_device: a round's pack, its passes, ..., the unpack (lsb_lexsort.cuh) ----------------------------------
 
 // the pack of round `r` of `cols`: into buf[0] for the first round, in place on buf[cur] for every later one
-int launch_lexsort_pack(lsb_ctx* c, const lsb_key_column* cols, const LexsortRound& r, bool gather) {
-  LexsortPackArgs a{};
+// the columns of round `r` with their shifts in the round's word
+void round_columns(const lsb_key_column* cols, const LexsortRound& r, LexsortColumn* out) {
   int shift = 0;
   for (int i = 0; i < r.ncols; i++) {
     const lsb_key_column& k = cols[r.first + i];
-    a.col[i] = LexsortColumn{k.keys, k.key_type, k.flags, shift};
+    out[i] = LexsortColumn{k.keys, k.key_type, k.flags, shift};
     shift += key_type_bits(k.key_type);
   }
+}
+
+int launch_lexsort_pack(lsb_ctx* c, const lsb_key_column* cols, const LexsortRound& r, bool gather) {
+  LexsortPackArgs a{};
+  round_columns(cols, r, a.col);
   a.buf = c->buf[gather ? c->cur : 0];
   a.count = c->here;
   const int grid = io_grid(c, c->here);
@@ -1241,16 +1247,16 @@ int launch_lexsort_unpack(lsb_ctx* c, const uint64_t* vals_in, uint64_t* vals_ou
   return LSB_OK;
 }
 
-int lexsort_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32_t K, const uint64_t* vals_in,
-                   uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
-  if (!c) return LSB_ERR_ARG;
+// The checks of lsb_lexsort_device's context, columns and count, shared by lsb_unique_device: widths[i] is the bit
+// width of column i.  Sets the context's device.
+int check_columns(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32_t K, int64_t count, std::vector<int>& widths) {
   const std::string f(fn);
   if (c->G > 1) return fail(c, LSB_ERR_ARG, f + ": one GPU only (world_size > 1)");
   if (c->cfg.flags & KEY_ORDER_FLAGS)
     return fail(c, LSB_ERR_ARG, f + ": the context has key-order flags (KEY_I64 / KEY_F64 / DESCENDING); the columns "
                                     "carry their own");
   if (K < 1 || !cols) return fail(c, LSB_ERR_ARG, f + ": needs num_columns >= 1 and a columns array");
-  std::vector<int> widths(K);
+  widths.assign(K, 0);
   for (int i = 0; i < K; i++) {
     const std::string col = f + ": column " + std::to_string(i);
     widths[i] = key_type_bits(cols[i].key_type);
@@ -1262,19 +1268,47 @@ int lexsort_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32
                                       (widths[i] == 64 ? "DESCENDING plus at most one of KEY_I64 / KEY_F64" : "DESCENDING or 0"));
   }
   if (count != c->here) return fail(c, LSB_ERR_ARG, f + ": count must equal this shard's size");
-  std::vector<LexsortRound> rounds(K);
-  const int nr = lexsort_rounds(widths.data(), K, c->cfg.radix_bits, rounds.data());
   CU(c, cudaSetDevice(c->cfg.device));
+  for (int i = 0; count && i < K; i++) {
+    const std::string name = "column " + std::to_string(i);
+    if (!cols[i].keys) return fail(c, LSB_ERR_ARG, f + ": " + name + ": keys is NULL");
+    int rc = check_device_array(c, fn, cols[i].keys, name.c_str(), count, widths[i] / 8);
+    if (rc) return rc;
+  }
+  return LSB_OK;
+}
+
+// The packs and passes of every round, least significant first: afterwards buf[cur] holds {the last round's word, the
+// input index} of every record in lexsort order.  passes counts the passes of every round.
+int sort_columns(lsb_ctx* c, const lsb_key_column* cols, const std::vector<LexsortRound>& rounds, int* passes, int* subpasses) {
+  c->cur = 0;
+  for (size_t r = 0; r < rounds.size(); r++) {
+    // the round's word holds its order keys: its passes sort the low `bits` bits as a uint64, ascending
+    int rc;
+    if (c->here && (rc = launch_lexsort_pack(c, cols, rounds[r], r > 0))) return rc;
+    if ((rc = run_passes(c, KeyPlan{rounds[r].bits, 0}, 0, rounds[r].passes, subpasses))) return rc;
+    *passes += rounds[r].passes;
+  }
+  return LSB_OK;
+}
+
+std::vector<LexsortRound> column_rounds(const lsb_ctx* c, const std::vector<int>& widths) {
+  std::vector<LexsortRound> rounds(widths.size());
+  rounds.resize(lexsort_rounds(widths.data(), (int)widths.size(), c->cfg.radix_bits, rounds.data()));
+  return rounds;
+}
+
+int lexsort_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32_t K, const uint64_t* vals_in,
+                   uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
+  if (!c) return LSB_ERR_ARG;
+  const std::string f(fn);
+  std::vector<int> widths;
+  int rc = check_columns(c, fn, cols, K, count, widths);
+  if (rc) return rc;
   const size_t bytes = (size_t)count * sizeof(uint64_t);
   if (count) {
-    for (int i = 0; i < K; i++) {
-      const std::string name = "column " + std::to_string(i);
-      if (!cols[i].keys) return fail(c, LSB_ERR_ARG, f + ": " + name + ": keys is NULL");
-      int rc = check_device_array(c, fn, cols[i].keys, name.c_str(), count, widths[i] / 8);
-      if (rc) return rc;
-    }
     if (!vals_out) return fail(c, LSB_ERR_ARG, f + ": vals_out is NULL");
-    int rc = check_device_array(c, fn, vals_in, "vals_in", count);
+    rc = check_device_array(c, fn, vals_in, "vals_in", count);
     if (!rc) rc = check_device_array(c, fn, vals_out, "vals_out", count);
     if (rc) return rc;
     if (vals_in && ranges_overlap(vals_out, bytes, vals_in, bytes)) return fail(c, LSB_ERR_ARG, f + ": vals_out overlaps vals_in");
@@ -1284,18 +1318,128 @@ int lexsort_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32
   }
   CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
   CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
-  int rc = begin_call(c);
-  if (rc) return rc;
-  c->cur = 0;
+  if ((rc = begin_call(c))) return rc;
   int passes = 0, subpasses = 0;
-  for (int r = 0; r < nr; r++) {
-    // the round's word holds its order keys: its passes sort the low `bits` bits as a uint64, ascending
-    if (count && (rc = launch_lexsort_pack(c, cols, rounds[r], r > 0))) return rc;
-    if ((rc = run_passes(c, KeyPlan{rounds[r].bits, 0}, 0, rounds[r].passes, &subpasses))) return rc;
-    passes += rounds[r].passes;
-  }
+  if ((rc = sort_columns(c, cols, column_rounds(c, widths), &passes, &subpasses))) return rc;
   if (count && (rc = launch_lexsort_unpack(c, vals_in, vals_out))) return rc;
   return end_call(c, st, passes, subpasses);
+}
+
+// ---- lsb_unique_device: lexsort's rounds (sorted mode), head flags, tile counts and their scan, the outputs -------------
+// (lsb_unique.cuh)
+
+template <bool SORTED>
+void launch_unique_flag_kernel(const UniqueFlagArgs& a, int ncols, int grid, cudaStream_t stream) {
+#define LSB_UNIQ_FLAG(N) unique_flag_kernel<SORTED, N><<<grid, IO_THREADS, 0, stream>>>(a)
+  switch (ncols) {  // 1 .. LEXSORT_ROUND_COLUMNS
+    case 1: LSB_UNIQ_FLAG(1); break;
+    case 2: LSB_UNIQ_FLAG(2); break;
+    case 3: LSB_UNIQ_FLAG(3); break;
+    default: LSB_UNIQ_FLAG(4); break;
+  }
+#undef LSB_UNIQ_FLAG
+}
+
+template <int PHASE>
+void launch_unique_tile_kernel(const UniqueTileArgs& a, int ncols, int grid, cudaStream_t stream) {
+#define LSB_UNIQ_TILE(N) unique_tile_kernel<PHASE, N><<<grid, UNIQUE_THREADS, 0, stream>>>(a)
+  switch (ncols) {  // 0: the sorted records; 1 .. LEXSORT_ROUND_COLUMNS: the last round's columns
+    case 0: LSB_UNIQ_TILE(0); break;
+    case 1: LSB_UNIQ_TILE(1); break;
+    case 2: LSB_UNIQ_TILE(2); break;
+    case 3: LSB_UNIQ_TILE(3); break;
+    default: LSB_UNIQ_TILE(4); break;
+  }
+#undef LSB_UNIQ_TILE
+}
+
+// count >= 1.  Sorted mode reads buf[cur], the records of sort_columns; both modes keep their scratch in buf[cur ^ 1].
+// U goes to small[24] on the device and comes back to host_small[24] before the call's final synchronise.
+int launch_unique(lsb_ctx* c, const lsb_key_column* cols, const std::vector<LexsortRound>& rounds, bool sorted,
+                  int64_t* index_out, int64_t* inverse_out, int64_t* counts_out) {
+  const UniqueScratch s = unique_scratch(c->buf[c->cur ^ 1], c->here);
+  int64_t* u = reinterpret_cast<int64_t*>(c->small + 24);
+  for (size_t r = 0; r + 1 < rounds.size(); r++) {
+    UniqueFlagArgs f{};
+    round_columns(cols, rounds[r], f.col);
+    f.rec = c->buf[c->cur];
+    f.diff = s.diff;
+    f.count = c->here;
+    f.first = r == 0;
+    if (sorted) launch_unique_flag_kernel<true>(f, rounds[r].ncols, io_grid(c, c->here), c->stream);
+    else launch_unique_flag_kernel<false>(f, rounds[r].ncols, io_grid(c, c->here), c->stream);
+    c->launches++;
+    CU(c, cudaGetLastError());
+  }
+  UniqueTileArgs a{};
+  a.rec = c->buf[c->cur];
+  if (!sorted) round_columns(cols, rounds.back(), a.col);
+  a.diff = rounds.size() > 1 ? s.diff : nullptr;
+  a.count = c->here;
+  a.totals = s.totals;
+  a.bases = s.bases;
+  a.index_out = index_out;
+  a.inverse_out = inverse_out;
+  a.ends = counts_out ? s.ends : nullptr;
+  a.num_unique = u;
+  const int ncols = sorted ? 0 : rounds.back().ncols;
+  launch_unique_tile_kernel<0>(a, ncols, (int)s.tiles, c->stream);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  // one CTA walks all count / UNIQUE_TILE totals, more than the sort's tables it was sized for: 1.0 ms at 2^30, under 1 %
+  // of the call (DESIGN.md §4g)
+  int rc = launch_scan(c, s.totals, (int)s.tiles, 1, 0, s.bases, nullptr);
+  if (rc) return rc;
+  launch_unique_tile_kernel<1>(a, ncols, (int)s.tiles, c->stream);
+  c->launches++;
+  CU(c, cudaGetLastError());
+  if (counts_out) {
+    const UniqueCountsArgs k{s.ends, u, counts_out, c->here};
+    unique_counts_kernel<<<io_grid(c, c->here), IO_THREADS, 0, c->stream>>>(k);
+    c->launches++;
+    CU(c, cudaGetLastError());
+  }
+  CU(c, cudaMemcpyAsync(c->host_small + 24, u, sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+  return LSB_OK;
+}
+
+int unique_device(lsb_ctx* c, const char* fn, const lsb_key_column* cols, int32_t K, uint32_t unique_flags,
+                  int64_t* index_out, int64_t* inverse_out, int64_t* counts_out, int64_t count, int64_t* num_unique,
+                  void* stream, lsb_stats* st) {
+  if (!c) return LSB_ERR_ARG;
+  const std::string f(fn);
+  std::vector<int> widths;
+  int rc = check_columns(c, fn, cols, K, count, widths);
+  if (rc) return rc;
+  if (unique_flags & ~LSB_UNIQUE_CONSECUTIVE)
+    return fail(c, LSB_ERR_ARG, f + ": unknown unique_flags " + std::to_string(unique_flags));
+  if (!num_unique) return fail(c, LSB_ERR_ARG, f + ": num_unique is NULL");
+  if (count) {
+    int64_t* outs[3] = {index_out, inverse_out, counts_out};
+    const char* names[3] = {"index_out", "inverse_out", "counts_out"};
+    const size_t bytes = (size_t)count * sizeof(int64_t);
+    for (int i = 0; i < 3; i++) {
+      if ((rc = check_device_array(c, fn, outs[i], names[i], count))) return rc;
+      if (!outs[i]) continue;
+      for (int j = 0; j < i; j++)
+        if (outs[j] && ranges_overlap(outs[i], bytes, outs[j], bytes))
+          return fail(c, LSB_ERR_ARG, f + ": " + names[i] + " overlaps " + names[j]);
+      for (int k = 0; k < K; k++)
+        if (ranges_overlap(outs[i], bytes, cols[k].keys, (size_t)count * (widths[k] / 8)))
+          return fail(c, LSB_ERR_ARG, f + ": " + names[i] + " overlaps column " + std::to_string(k));
+    }
+  }
+  const std::vector<LexsortRound> rounds = column_rounds(c, widths);
+  const bool sorted = !(unique_flags & LSB_UNIQUE_CONSECUTIVE);
+  CU(c, cudaEventRecord(c->ev_caller, (cudaStream_t)stream));
+  CU(c, cudaStreamWaitEvent(c->stream, c->ev_caller, 0));
+  if ((rc = begin_call(c))) return rc;
+  int passes = 0, subpasses = 0;
+  if (sorted && (rc = sort_columns(c, cols, rounds, &passes, &subpasses))) return rc;
+  if (count && (rc = launch_unique(c, cols, rounds, sorted, index_out, inverse_out, counts_out))) return rc;
+  if ((rc = end_call(c, st, passes, subpasses))) return rc;
+  *num_unique = count ? (int64_t)c->host_small[24] : 0;
+  return LSB_OK;
 }
 
 }  // namespace
@@ -1777,6 +1921,13 @@ int lsb_sort_segments_device_typed(lsb_ctx* c, uint32_t key_type, const void* ke
 int lsb_lexsort_device(lsb_ctx* c, const lsb_key_column* columns, int32_t num_columns, const uint64_t* vals_in,
                        uint64_t* vals_out, int64_t count, void* stream, lsb_stats* st) {
   return lexsort_device(c, "lsb_lexsort_device", columns, num_columns, vals_in, vals_out, count, stream, st);
+}
+
+int lsb_unique_device(lsb_ctx* c, const lsb_key_column* columns, int32_t num_columns, uint32_t unique_flags,
+                      int64_t* index_out, int64_t* inverse_out, int64_t* counts_out, int64_t count, int64_t* num_unique,
+                      void* stream, lsb_stats* st) {
+  return unique_device(c, "lsb_unique_device", columns, num_columns, unique_flags, index_out, inverse_out, counts_out,
+                       count, num_unique, stream, st);
 }
 
 // The two test hooks run the PRODUCTION count and scan kernels of the pass shape in use.

@@ -32,6 +32,7 @@ FLAG_NO_SKIP = 8
 FLAG_KEY_I64 = 16
 FLAG_KEY_F64 = 32
 FLAG_DESCENDING = 64
+UNIQUE_CONSECUTIVE = 1  # lsb_unique_device: groups are runs of equal adjacent elements, in input order
 SEG_LOCAL_INDEX = 1  # lsb_sort_segments_device without vals_in: index within the segment, not the global input index
 KEY_DTYPE_FLAGS = {np.dtype(np.uint64): 0, np.dtype(np.int64): FLAG_KEY_I64, np.dtype(np.float64): FLAG_KEY_F64}
 # key types of lsb_sort_device_typed / lsb_sort_segments_device_typed (LSB_KEY_*), by torch dtype name
@@ -122,6 +123,8 @@ def load_library():
     L.lsb_sort_segments_device_typed.argtypes = [vp, ctypes.c_uint32, vp, vp, vp, vp, i64, vp, i64, ctypes.c_uint32, vp,
                                                  ctypes.POINTER(Stats)]
     L.lsb_lexsort_device.argtypes = [vp, ctypes.POINTER(KeyColumn), ctypes.c_int32, vp, vp, i64, vp, ctypes.POINTER(Stats)]
+    L.lsb_unique_device.argtypes = [vp, ctypes.POINTER(KeyColumn), ctypes.c_int32, ctypes.c_uint32, vp, vp, vp, i64,
+                                    ctypes.POINTER(i64), vp, ctypes.POINTER(Stats)]
     L.lsb_histogram.argtypes = [vp, ci, vp]
     L.lsb_starts.argtypes = [vp, ci, vp]
     L.lsb_num_passes.argtypes = [vp]
@@ -378,17 +381,50 @@ class DistributedSorter:
         if stream is None:
             stream = torch.cuda.current_stream(cols[0].device)
         handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
-        spec = (KeyColumn * len(cols))()
-        for c, (t, d) in enumerate(zip(cols, desc)):
-            narrow = _narrow_key_type(torch, t.dtype)
-            spec[c].keys = t.data_ptr() or None
-            spec[c].key_type = narrow if narrow is not None else KEY_CONTEXT
-            spec[c].flags = (0 if narrow is not None else _key_dtype_flags(torch)[t.dtype]) | (FLAG_DESCENDING if d else 0)
         st = Stats()
         ptr = lambda t: t.data_ptr() or None if t is not None else None  # noqa: E731
-        self._check(self._L.lsb_lexsort_device(self._ctx, spec, len(cols), ptr(vals), ptr(vals_out), n, handle,
-                                               ctypes.byref(st)), "lsb_lexsort_device")
+        self._check(self._L.lsb_lexsort_device(self._ctx, _key_columns(torch, cols, desc), len(cols), ptr(vals),
+                                               ptr(vals_out), n, handle, ctypes.byref(st)), "lsb_lexsort_device")
         return vals_out, st
+
+    def unique_device(self, columns, descending=False, consecutive=False, index_out=None, inverse_out=None,
+                      counts_out=None, stream=None):
+        """The distinct elements of several key columns (lsb_unique_device): np.unique(return_index=True,
+        return_inverse=True, return_counts=True, equal_nan=True) over the rows (columns[K-1][j], ..., columns[0][j]), or
+        with consecutive=True torch.unique_consecutive's runs of equal adjacent rows.  `columns` and `descending` as in
+        lexsort_device (descending reverses the numbering of the groups of sorted mode).  Elements are equal when every
+        column's key is: all NaNs of a column are one value, and -0.0 == +0.0.  index_out / inverse_out / counts_out: an
+        int64 tensor of `here` elements to write, None to allocate one, False for none.  Groups are numbered in the
+        columns' lexsort order (consecutive: in input order); index_out[r] is the first input position of group r,
+        inverse_out[j] the group of element j and counts_out[r] the size of group r.  index and counts keep their full
+        length: their first num_unique entries are written.  Stream as in sort_device.  Returns (index_out, inverse_out,
+        counts_out, num_unique, Stats), None for an output not asked for."""
+        torch = _torch()
+        n = self.here
+        cols = _check_columns(torch, columns, n, self.device)
+        desc = _check_descending(descending, len(cols))
+        if not isinstance(consecutive, bool):
+            raise TypeError(f"consecutive must be a bool, not {consecutive!r}")
+        outs = []
+        for name, t in (("index_out", index_out), ("inverse_out", inverse_out), ("counts_out", counts_out)):
+            if t is None:
+                t = torch.empty(n, dtype=torch.int64, device=cols[0].device)
+            elif t is not False:
+                if not isinstance(t, torch.Tensor) or t.dtype != torch.int64:
+                    raise TypeError(f"{name} must be an int64 torch.Tensor, None or False, not {getattr(t, 'dtype', type(t).__name__)}")
+                _check_vector(torch, t, name, n, self.device)
+            outs.append(t)
+        if stream is None:
+            stream = torch.cuda.current_stream(cols[0].device)
+        handle = stream.cuda_stream if hasattr(stream, "cuda_stream") else int(stream)
+        st = Stats()
+        u = ctypes.c_int64()
+        ptrs = [t.data_ptr() or None if t is not False else None for t in outs]
+        self._check(self._L.lsb_unique_device(self._ctx, _key_columns(torch, cols, desc), len(cols),
+                                              UNIQUE_CONSECUTIVE if consecutive else 0, *ptrs, n, ctypes.byref(u),
+                                              handle, ctypes.byref(st)), "lsb_unique_device")
+        index, inverse, counts = (t if t is not False else None for t in outs)
+        return index, inverse, counts, u.value, st
 
     # -- test hooks -----------------------------------------------------------------------
     def num_passes(self):
@@ -577,6 +613,17 @@ def _check_columns(torch, columns, n=None, device=None):
     return list(columns)
 
 
+def _key_columns(torch, cols, desc):
+    """the lsb_key_column array of checked columns and their directions"""
+    spec = (KeyColumn * len(cols))()
+    for c, (t, d) in enumerate(zip(cols, desc)):
+        narrow = _narrow_key_type(torch, t.dtype)
+        spec[c].keys = t.data_ptr() or None
+        spec[c].key_type = narrow if narrow is not None else KEY_CONTEXT
+        spec[c].flags = (0 if narrow is not None else _key_dtype_flags(torch)[t.dtype]) | (FLAG_DESCENDING if d else 0)
+    return spec
+
+
 def _check_descending(descending, k):
     """one bool per column from a bool or a sequence of k bools"""
     if isinstance(descending, bool):
@@ -666,3 +713,72 @@ def _sort_rows(torch, x, dim, descending, keys):
             k, v, _ = s.sort_segments(flat, offsets, keys_out=None if keys else False, local_index=True)
     back = lambda t: t.view(shape).movedim(-1, d).contiguous()  # noqa: E731
     return (back(k) if keys else None), back(v)
+
+
+def unique(input, sorted=True, return_inverse=False, return_counts=False, dim=None, return_index=False):
+    """torch.unique for a CUDA tensor of uint64, int64, float64, uint32, int32, float32, uint16, int16, float16 or
+    bfloat16, on that tensor's GPU.  Returns the distinct values in ascending order, then with return_index the input
+    position of each one's first occurrence (np.unique's return_index, which torch lacks), with return_inverse the group
+    of every element (the input's shape; [input.size(dim)] with dim) and with return_counts the size of every group: a
+    tensor alone when no extra output is asked for, else a tuple in that order (numpy's).  dim=None flattens the input;
+    with dim=d the slices along d are the elements, compared lexicographically (input.select(d, i) flattened, its first
+    entry the primary key).  Values are equal as numpy's equal_nan=True has them: all NaNs are one value (torch counts
+    every NaN apart), and -0.0 == +0.0.  The values returned are input[index], the exact bits of each first occurrence.
+    sorted=False returns the sorted result too (a valid answer).  Makes a one-GPU sorter for the call."""
+    outs = _unique(_torch(), input, dim, False, return_index, return_inverse, return_counts)
+    return outs[0] if len(outs) == 1 else tuple(outs)
+
+
+def unique_consecutive(input, return_inverse=False, return_counts=False, dim=None):
+    """torch.unique_consecutive for a CUDA tensor of the dtypes of unique: the first element of every run of equal
+    adjacent elements (slices along dim with dim), with the group of every element and the length of every run, in
+    input order; no sort.  Equality as in unique (all NaNs one value, -0.0 == +0.0).  Makes a one-GPU sorter for the
+    call."""
+    outs = _unique(_torch(), input, dim, True, False, return_inverse, return_counts)
+    return outs[0] if len(outs) == 1 else tuple(outs)
+
+
+def _unique(torch, x, dim, consecutive, want_index, want_inverse, want_counts):
+    """[values, index?, inverse?, counts?] of unique / unique_consecutive"""
+    if not isinstance(x, torch.Tensor):
+        raise TypeError(f"input must be a torch.Tensor, not {type(x).__name__}")
+    if x.dtype not in _key_dtype_flags(torch) and _narrow_key_type(torch, x.dtype) is None:
+        raise TypeError(f"input must be torch.uint64, int64, float64, torch.{', torch.'.join(NARROW_KEY_TYPES)}, not {x.dtype}")
+    size, inverse_shape, columns = _unique_columns(torch, x, dim)
+    if not x.is_cuda:
+        raise ValueError(f"input must be a CUDA tensor, not on {x.device}")
+    if size == 0:  # what torch returns: no values (the empty slices along dim), no groups
+        empty = torch.empty(0, dtype=torch.int64, device=x.device)
+        inverse = torch.empty(inverse_shape, dtype=torch.int64, device=x.device)
+        return [x.reshape(-1) if dim is None else x.clone()] + [empty] * want_index + [inverse] * want_inverse \
+            + [empty] * want_counts
+    with DistributedSorter(size, ranks=1, device=x.device.index) as s:
+        index, inverse, counts, u, _ = s.unique_device(columns, consecutive=consecutive,
+                                                       inverse_out=None if want_inverse else False,
+                                                       counts_out=None if want_counts else False)
+    index = index[:u]
+    # gathered as signed integers of the element's width: torch indexes no unsigned CUDA tensor wider than a byte
+    bits = x.view({8: torch.int64, 4: torch.int32, 2: torch.int16}[x.element_size()])
+    values = (bits.reshape(-1)[index] if dim is None else bits.index_select(dim % x.dim(), index)).view(x.dtype)
+    return [values] + ([index] if want_index else []) + ([inverse.view(inverse_shape)] if want_inverse else []) \
+        + ([counts[:u]] if want_counts else [])
+
+
+def _unique_columns(torch, x, dim):
+    """(number of elements, shape of the inverse, key columns least significant first) of unique over x on x's device.
+    dim=None: the flattened input, one column.  dim=d: the slices x.select(d, i) are the elements, and column j holds
+    entry j of every flattened slice; entry 0 is the primary key, so it comes last.  IndexError for a dim out of range
+    (as torch), ValueError for empty slices along a dim of nonzero size (torch refuses them too)."""
+    if dim is None:
+        return x.numel(), x.shape, [x.reshape(-1).contiguous()]
+    if isinstance(dim, bool) or not isinstance(dim, int):
+        raise TypeError(f"dim must be None or an int, not {dim!r}")
+    if not -x.dim() <= dim < x.dim():
+        raise IndexError(f"dim {dim} is out of range for a {x.dim()}-D input")
+    size = x.shape[dim]
+    if size and x.numel() == 0:
+        raise ValueError(f"dim {dim}: the slices along it are empty (shape {tuple(x.shape)})")
+    if size == 0:
+        return 0, (0,), []
+    cols = x.movedim(dim, 0).reshape(size, -1).t().contiguous()  # one contiguous row per entry of a slice
+    return size, (size,), list(cols.unbind(0))[::-1]

@@ -327,6 +327,41 @@ typedef struct lsb_key_column {
 int lsb_lexsort_device(lsb_ctx* ctx, const lsb_key_column* columns, int32_t num_columns, const uint64_t* vals_in,
                        uint64_t* vals_out, int64_t count, void* stream, lsb_stats* stats);
 
+/* unique_flags of lsb_unique_device: groups are runs of equal adjacent elements, in input order (no sort) */
+#define LSB_UNIQUE_CONSECUTIVE 1u
+
+/* The distinct elements of K key columns on device memory (torch.unique / np.unique with equal_nan=True, and with
+ * LSB_UNIQUE_CONSECUTIVE torch.unique_consecutive).  Columns as in lsb_lexsort_device: columns[0] the least significant,
+ * each of any key type under its own flags.  Positions i and j are equal when order_c(col_c[i]) == order_c(col_c[j]) for
+ * every column c, order_c being the column's key order above: so all NaNs of a column are equal whatever their sign or
+ * payload, and -0.0 == +0.0.  A group is a maximal set of equal positions; U is the number of groups.
+ *   Sorted mode (unique_flags 0): groups are numbered 0 .. U-1 in the lexsort order of their keys.
+ *   LSB_UNIQUE_CONSECUTIVE: groups are the maximal runs of equal adjacent positions, numbered in input order; equal keys
+ *   in non-adjacent runs are separate groups.
+ * index_out[r] is the smallest input position of group r (its first occurrence), inverse_out[j] the group of position
+ * j, counts_out[r] the size of group r, and *num_unique = U.  Each of the three outputs may be NULL (all three: U only);
+ * they are int64 device memory of the context's device with room for count entries, of which index_out and counts_out
+ * get the first U only.  The columns are never rewritten.
+ * Method: sorted mode runs lsb_lexsort_device's packs and passes.  Position p >= 1 starts a group when its last round's
+ * word differs from position p - 1's (compared directly) or one of its earlier rounds' columns does (one gather launch
+ * per earlier round, flags in scratch); consecutive mode compares the columns at p and p - 1 in input order.  Heads are
+ * counted per tile of 2048 positions, the tile counts scanned, and a second read of the tiles writes index_out,
+ * inverse_out (a scatter through the input index in sorted mode) and the group starts, from which counts_out follows.
+ * The scratch is the shard buffer the sort does not hold; nothing is allocated.  stats: passes and skipped count the
+ * sort's passes (what lsb_lexsort_device runs; 0 in consecutive mode), kernel_launches every launch of the call.
+ * The contract of lsb_lexsort_device otherwise: one GPU, the context's pass-shape flags and radix_bits apply, count ==
+ * here, the library's stream waits on `stream`, synchronous on return, and with count == 0 *num_unique = 0 and no device
+ * pointer is looked at.  Afterwards the shard holds internal records: what lsb_download, lsb_checksum and
+ * lsb_verify_device report is unspecified until the next sort.
+ * LSB_ERR_ARG, with a message naming the column where one applies: every refusal of lsb_lexsort_device's context,
+ * columns and count (world_size > 1, key-order flags on the context, num_columns < 1, columns == NULL, a column's
+ * key_type, flags or keys, count != here); unique_flags other than 0 or LSB_UNIQUE_CONSECUTIVE; num_unique == NULL; and
+ * for count > 0 an output not aligned to 8 bytes, not device memory of the context's device, overlapping the context's
+ * shards, another output or any column. */
+int lsb_unique_device(lsb_ctx* ctx, const lsb_key_column* columns, int32_t num_columns, uint32_t unique_flags,
+                      int64_t* index_out, int64_t* inverse_out, int64_t* counts_out, int64_t count,
+                      int64_t* num_unique /* host */, void* stream, lsb_stats* stats);
+
 /* ---- test hooks into the pass (same tables the reference computes) ---------------- */
 
 /* counts[d], d < 2^bits(digit): the localShuffle count loop (:226-229) on this shard; d is the
