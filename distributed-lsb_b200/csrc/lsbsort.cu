@@ -29,6 +29,7 @@
 #include "lsb_segments.cuh"
 #include "lsb_lexsort.cuh"
 #include "lsb_unique.cuh"
+#include "lsb_bucket.cuh"
 
 #include <nccl.h>  // types only: the library itself is bound at run time, see NcclApi
 #include <dlfcn.h>
@@ -84,6 +85,9 @@ struct Tuning {
                          // resident CTAs, ~3 us ahead of the tile's own CTA).  Measured at 2^30 (7.09 ms per launch
                          // without): 74 or 148 tiles -> 6.48 ms, 296 -> 6.91 ms, 592 -> 7.66 ms (the prefetched
                          // lines do not survive in L2 next to the output stream), profiles/r2_final_sweep.log
+  int bk_mode = 0;       // bucket pass (plan_bucket): 0 = when the plan accepts the input, 1 = never (byte steps only),
+                         // 2 = whenever the sort's shape allows, without the size threshold and the histogram test
+  int bk_bytes = 0;      // bucket pass: scatter steps on the top bytes before it (2..7), 0 = from the shard size
 };
 Tuning g_tune;
 
@@ -166,6 +170,9 @@ struct lsb_ctx {
   int64_t launches = 0;
   int64_t part_elems = 0;
   int skipped = 0;
+  unsigned* bk_overflow = nullptr;  // set by bucket_sort_kernel when a bucket does not fit a chunk
+  bool bk_launched = false;         // this call ran the bucket pass ...
+  int bk_resolved = 0;              // ... and it resolved this many low bytes (0: it overflowed)
   std::string err;
 };
 
@@ -282,6 +289,8 @@ int begin_call(lsb_ctx* c) {
   c->launches = 0;
   c->part_elems = 0;
   c->skipped = 0;
+  c->bk_launched = false;
+  c->bk_resolved = 0;
   c->next_counter = 0;
   CU(c, cudaMemsetAsync(c->tile_counters, 0, TILE_COUNTERS * sizeof(uint32_t), c->stream));
   CU(c, cudaMemsetAsync(c->op_err, 0, sizeof(unsigned), c->stream));
@@ -327,7 +336,8 @@ int end_call(lsb_ctx* c, lsb_stats* st, int passes, int subpasses) {
     CU(c, cudaEventElapsedTime(&d, c->xev[i], c->xev[i + 1]));
     st->exchange_ms += d;
   }
-  st->partition_launches = subpasses;
+  // scatter-type launches: one per 8-bit step; the bucket pass is one launch for the bytes it resolved
+  st->partition_launches = subpasses - c->bk_resolved + (c->bk_launched ? 1 : 0);
   st->partition_elements = c->part_elems;
   if (c->G > 1) {
     for (int g = 0; g < c->G; g++) st->sent[g] = (int64_t)c->host_small[g];
@@ -845,9 +855,92 @@ int pass_global(lsb_ctx* c, const KeyPlan& k, int digit, int* subpasses, bool fu
   return LSB_OK;
 }
 
+// Bucket plan of a whole one-GPU sort of 64-bit keys in the two-step shape whose steps are exactly bytes 0..7 (radix 8
+// or 16): k stable steps on the top k bytes, then bucket_sort_kernel finishes every run of equal top bytes on chip --
+// k + 1 trips through HBM instead of 8.  k is the least k >= 2 with here <= 128 * 256^k (buckets of at most 128
+// records on average: 2^30 and 2^31 records take k = 3).  Returns k when the shape allows the plan, 0 otherwise; the
+// input is judged by bucket_accepts once its byte counts are on the host.
+int plan_bucket(const lsb_ctx* c, const KeyPlan& k, const std::vector<SubPass>& subs, bool whole_sort) {
+  if (!whole_sort || k.bits != 64 || subs.size() != 8 || c->here < 1 || c->tune.bk_mode == 1) return 0;
+  for (int s = 0; s < 8; s++)
+    if (subs[s].shift != 8 * s || subs[s].bits != 8) return 0;
+  if (c->tune.bk_mode != 2 && c->here < (1 << 20)) return 0;
+  if (c->tune.bk_bytes) return c->tune.bk_bytes;
+  int kb = 2;
+  while (kb < 7 && (double)c->here > 128.0 * std::ldexp(1.0, 8 * kb)) kb++;
+  return kb;
+}
+
+// The byte counts (host_hist[8][256]) accept the bucket plan when no bin of the top kb bytes holds more than twice its
+// share (2 * here / 256: masked keys, heavy hitters and few distinct keys stay on the byte steps, whose cost does not
+// depend on the keys) and, when constant bytes may be skipped, no byte is constant (so the steps skipped are the same
+// on both paths: none).
+bool bucket_accepts(const lsb_ctx* c, int kb, bool may_skip) {
+  const unsigned long long here = (unsigned long long)c->here;
+  for (int s = 0; s < 8; s++)
+    for (int b = 0; b < 256; b++) {
+      const unsigned long long v = c->host_hist[s * 256 + b];
+      if (may_skip && v == here) return false;
+      if (c->tune.bk_mode != 2 && s >= 8 - kb && v * 128 > here) return false;
+    }
+  return true;
+}
+
+// launch of bucket_sort_kernel over buf[cur] -> buf[cur ^ 1], records stably sorted by the top kb bytes of their order key
+int launch_bucket(lsb_ctx* c, uint32_t korder, int kb) {
+  CU(c, cudaMemsetAsync(c->bk_overflow, 0, sizeof(unsigned), c->stream));
+  BucketArgs a;
+  a.src = c->buf[c->cur];
+  a.dst = c->buf[c->cur ^ 1];
+  a.n = c->here;
+  a.top_shift = 64 - 8 * kb;
+  a.ord_shift = 72 - 8 * kb;
+  a.low_mask = (1ULL << (64 - 8 * kb)) - 1;
+  a.overflow = c->bk_overflow;
+  a.korder = korder;
+  const unsigned grid = (unsigned)div_ceil(c->here, BK_TILE);
+  if (korder) bucket_sort_kernel<true><<<grid, BK_THREADS, BK_SMEM, c->stream>>>(a);
+  else bucket_sort_kernel<false><<<grid, BK_THREADS, BK_SMEM, c->stream>>>(a);
+  c->launches++;
+  c->part_elems += c->here;
+  c->bk_launched = true;
+  CU(c, cudaGetLastError());
+  return phase_mark(c, 2);
+}
+
+// the bucket plan after the count launch: kb steps on the top bytes, the bucket pass, and -- when a bucket did not fit
+// a chunk -- all 8 byte steps over the bucket pass's input (a stable permutation of the original by the top bytes, so
+// their stable sort of it is the stable sort of the original)
+int sort_buckets(lsb_ctx* c, const KeyPlan& k, int kb, int* subpasses) {
+  int rc;
+  for (int s = 8 - kb; s < 8; s++) {
+    if ((rc = launch_partition(c, k.korder, c->buf[c->cur], c->here, 8 * s, 8, c->seg_start, c->seg_tiles, c->scan_out + (size_t)s * 257, c->buf[c->cur ^ 1])))
+      return rc;
+    c->cur ^= 1;
+    (*subpasses)++;
+  }
+  if ((rc = launch_bucket(c, k.korder, kb))) return rc;
+  CU(c, cudaMemcpyAsync(c->host_small + 9, c->bk_overflow, sizeof(unsigned), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaStreamSynchronize(c->stream));
+  if (!*reinterpret_cast<const unsigned*>(c->host_small + 9)) {
+    c->cur ^= 1;
+    c->bk_resolved = 8 - kb;
+    (*subpasses) += 8 - kb;
+    return LSB_OK;
+  }
+  for (int s = 0; s < 8; s++) {
+    if ((rc = launch_partition(c, k.korder, c->buf[c->cur], c->here, 8 * s, 8, c->seg_start, c->seg_tiles, c->scan_out + (size_t)s * 257, c->buf[c->cur ^ 1])))
+      return rc;
+    c->cur ^= 1;
+    (*subpasses)++;
+  }
+  return LSB_OK;
+}
+
 // passes [d0, d1) on one GPU: one read counts the digits of every pass, then one launch per pass
-// (LSB_FLAG_ONE_PASS) or per 8-bit step (default) that reads the shard once and writes it once
-int passes_single(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) {
+// (LSB_FLAG_ONE_PASS) or per 8-bit step (default) that reads the shard once and writes it once.
+// whole_sort: the passes are a whole lsb_sort-type call, which may take the bucket plan (plan_bucket).
+int passes_single(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses, bool whole_sort) {
   if (!(c->cfg.flags & LSB_FLAG_ONE_PASS)) {
     // two-step shape: one histogram read for all sub-digits, then one HBM -> HBM step per sub-digit
     std::vector<SubPass> subs;
@@ -856,15 +949,17 @@ int passes_single(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) 
       if (p.lo_bits) subs.push_back({p.shift, p.lo_bits});
       subs.push_back({p.shift + p.lo_bits, p.hi_bits});
     }
+    const int kb = plan_bucket(c, k, subs, whole_sort);
     int rc;
     for (size_t s0 = 0; s0 < subs.size(); s0 += HIST_MAX_SUB) {
       const int ns = (int)std::min<size_t>(HIST_MAX_SUB, subs.size() - s0);
       if ((rc = launch_subdigit_hist(c, k.korder, c->buf[c->cur], subs.data() + s0, ns))) return rc;
       const bool may_skip = !(c->cfg.flags & LSB_FLAG_NO_SKIP) && c->here > 0;
-      if (may_skip) {  // a digit that is constant over the shard makes its stable step the identity
+      if (may_skip || kb) {  // a digit that is constant over the shard makes its stable step the identity
         CU(c, cudaMemcpyAsync(c->host_hist, c->hist, sizeof(unsigned long long) * 256 * ns, cudaMemcpyDeviceToHost, c->stream));
         CU(c, cudaStreamSynchronize(c->stream));  // once per sort (per 16 sub-digits), before the first step
       }
+      if (kb && bucket_accepts(c, kb, may_skip)) return sort_buckets(c, k, kb, subpasses);
       for (int s = 0; s < ns; s++) {
         const SubPass& sp = subs[s0 + s];
         if (may_skip) {
@@ -924,10 +1019,10 @@ int passes_single(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) 
   return LSB_OK;
 }
 
-// the passes [d0, d1) of the plan `k` in the context's pass shape
-int run_passes(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses) {
+// the passes [d0, d1) of the plan `k` in the context's pass shape; whole_sort: see passes_single
+int run_passes(lsb_ctx* c, const KeyPlan& k, int d0, int d1, int* subpasses, bool whole_sort = false) {
   c->dense_ready_digit = -1;
-  if (!c->two_level) return passes_single(c, k, d0, d1, subpasses);
+  if (!c->two_level) return passes_single(c, k, d0, d1, subpasses, whole_sort);
   int rc = plan_fusion(c, k);
   if (rc) return rc;
   for (int d = d0; d < d1; d++)
@@ -948,7 +1043,7 @@ int sort_shard(lsb_ctx* c, const KeyPlan& k, lsb_stats* st) {
   if (rc) return rc;
   int subpasses = 0;
   const int np = num_passes(c, k);
-  if ((rc = run_passes(c, k, 0, np, &subpasses))) return rc;
+  if ((rc = run_passes(c, k, 0, np, &subpasses, true))) return rc;
   return end_call(c, st, np, subpasses);
 }
 
@@ -1486,6 +1581,8 @@ int lsb_tune(const char* key, int value) {
   else if (k == "pt_chunks" && value >= 0 && value <= 4) g_tune.pt_chunks = value;
   else if (k == "pt_variant" && value >= 0 && value <= 1) g_tune.pt_variant = value;
   else if (k == "pt_pf_tiles" && value >= 0 && value <= 65536) g_tune.pt_pf_tiles = value;
+  else if (k == "bk_mode" && value >= 0 && value <= 2) g_tune.bk_mode = value;
+  else if (k == "bk_bytes" && (value == 0 || (value >= 2 && value <= 7))) g_tune.bk_bytes = value;
   else return fail(nullptr, LSB_ERR_ARG, "lsb_tune: unknown key or value out of range: " + k);
   return LSB_OK;
 }
@@ -1587,6 +1684,9 @@ int lsb_create(lsb_ctx** out, const lsb_config* cfg) {
   LSB_OP_ATTR(TileCfg, false, true)
   LSB_OP_ATTR(TileCfgS, false, true)
 #undef LSB_OP_ATTR
+  CUC(cudaFuncSetAttribute(bucket_sort_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BK_SMEM));
+  CUC(cudaFuncSetAttribute(bucket_sort_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BK_SMEM));
+  CUC(cudaMalloc(&c->bk_overflow, sizeof(unsigned)));
   CUC(cudaFuncSetAttribute(digit_hist_kernel<0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
   CUC(cudaFuncSetAttribute(digit_hist_kernel<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
   CUC(cudaFuncSetAttribute(digit_hist_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, DH_SMEM));
@@ -1713,7 +1813,7 @@ void lsb_destroy(lsb_ctx* c) {
   void* dev[] = {c->seg_start, c->seg_tiles, c->hist, c->scan_out, c->buf[0], c->buf[1], c->lookback, c->tile_counters, c->hist16, c->starts16, c->dig_meta, c->skip_flags,
                  c->counts_all, c->mybase, c->op_ctl, c->op_X, c->op_oc, c->op_F, c->op_err, c->op_prof,
                  c->scratch[0], c->scratch[1], c->dense_local, c->dense_mine, c->next_dense, c->c_all, c->totals, c->fuse_live, c->digit_base,
-                 c->mybase_v, c->localbase_v, c->bases_v, c->small, c->small_all};
+                 c->mybase_v, c->localbase_v, c->bases_v, c->small, c->small_all, c->bk_overflow};
   for (void* p : dev) cudaFree(p);
   for (int q = 0; q < LSB_MAX_PARTS; q++) {
     if (c->ev_sorted[q]) cudaEventDestroy(c->ev_sorted[q]);
@@ -1875,7 +1975,7 @@ int lsb_pass(lsb_ctx* c, int digit, lsb_stats* st) {
   if ((rc = begin_call(c))) return rc;
   c->dense_ready_digit = -1;
   int subpasses = 0;
-  if (!c->two_level) rc = passes_single(c, context_plan(c), digit, digit + 1, &subpasses);
+  if (!c->two_level) rc = passes_single(c, context_plan(c), digit, digit + 1, &subpasses, false);
   else rc = pass_global(c, context_plan(c), digit, &subpasses, false);
   if (rc) return rc;
   return end_call(c, st, 1, subpasses);

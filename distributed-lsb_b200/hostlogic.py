@@ -173,3 +173,49 @@ def onepass_dependencies(item, nx, t1, tiles_last, nsuper):
     if s > 0:
         deps.append(("K2", s - 1, idx))
     return deps
+
+
+# ---- the bucket plan of a one-GPU sort of 64-bit keys (plan_bucket / bucket_accepts in csrc/lsbsort.cu) -------------
+def bucket_bytes(here, forced=0):
+    """scatter steps on the top bytes before the bucket pass: the least k >= 2 with here <= 128 * 256^k (buckets of at
+    most 128 records on average), or `forced` (tune key bk_bytes)"""
+    if forced:
+        return forced
+    k = 2
+    while k < 7 and here > 128 * 256 ** k:
+        k += 1
+    return k
+
+
+def bucket_plan(byte_counts, here, radix_bits=16, no_skip=False, mode=0, forced=0):
+    """k when a whole lsb_sort-type call of 64-bit keys on one GPU in the two-step shape takes the bucket plan (k stable
+    steps on the top bytes, then the bucket pass), 0 when it runs the 8 byte steps.  byte_counts[s][b]: records whose
+    order key has byte s equal to b.  mode: tune key bk_mode (0 auto, 1 never, 2 whenever the shape allows)."""
+    if mode == 1 or radix_bits not in (8, 16) or here < 1 or (mode != 2 and here < 1 << 20):
+        return 0
+    k = bucket_bytes(here, forced)
+    c = np.asarray(byte_counts, dtype=np.int64)
+    if not no_skip and (c == here).any():
+        return 0  # a constant byte: the byte steps skip it
+    if mode != 2 and (c[8 - k:] * 128 > here).any():
+        return 0  # a top byte with a bin over twice its share
+    return k
+
+
+def byte_counts(order_keys):
+    """[8][256] counts of every byte of the order keys"""
+    k = np.asarray(order_keys, dtype=np.uint64)
+    return np.stack([np.bincount(((k >> np.uint64(8 * s)) & np.uint64(255)).astype(np.int64), minlength=256)
+                     for s in range(8)])
+
+
+def sort_stats(k, overflow=False, skipped=0):
+    """(subpasses, partition_launches, kernel_launches) of a whole one-GPU sort in the two-step shape with one count
+    launch over 8 byte steps: the bucket plan with k (0 = the byte steps, `skipped` of them skipped), and whether the
+    bucket pass overflowed into the 8 byte steps"""
+    if not k:
+        steps = 8 - skipped
+        return steps, steps, 2 + steps
+    if overflow:
+        return k + 8, k + 9, 2 + k + 1 + 8
+    return 8, k + 1, 2 + k + 1

@@ -141,7 +141,9 @@ typedef struct lsb_config {
 typedef struct lsb_stats {
   double device_ms;       /* whole call: first kernel start -> last kernel end             */
   int32_t passes;         /* reference passes run (N_DIGITS, :22)                          */
-  int32_t subpasses;      /* scatter-kernel launches (2 per 16-bit pass and part; 1 with ONE_PASS) */
+  int32_t subpasses;      /* 8-bit steps resolved (2 per 16-bit pass and part; 1 per pass with ONE_PASS);
+                             the bucket plan (below) counts 8: its k steps and the 8 - k bytes of the bucket pass,
+                             k + 8 when the bucket pass overflowed into the 8 byte steps */
   int32_t skipped;        /* steps (ONE_PASS: passes) skipped because their digit was constant */
   int32_t reserved0;
   int64_t elements;       /* elements of THIS shard that took part                         */
@@ -151,7 +153,7 @@ typedef struct lsb_stats {
   double exchange_ms;     /* G > 1: exchange kernels (NVLink stores)                       */
   double subpass_ms[LSB_MAX_SUBPASSES]; /* per partition-kernel launch                     */
   int64_t sent[LSB_MAX_GPUS]; /* last pass: elements this shard sent to each GPU (:553-554) */
-  int64_t partition_launches;
+  int64_t partition_launches; /* scatter-type launches: subpasses, or k + 1 on the bucket plan (k + 9 after an overflow) */
   int64_t partition_elements; /* elements moved by all partition launches of the call          */
   int64_t kernel_launches; /* all kernels launched by the call                             */
 } lsb_stats;
@@ -189,6 +191,20 @@ const char* lsb_status_string(int status);
  * (prefetch distance in tiles, 0 = half the SM count).
  * Unknown key / bad value: LSB_ERR_ARG. */
 int lsb_tune(const char* key, int value);
+/*
+ * The bucket plan.  A whole sort of 64-bit keys (lsb_sort, lsb_sort_host, lsb_sort_device[_typed] with an 8-byte key)
+ * on one GPU in the two-step shape at radix 8 or 16, of here >= 2^20 records, counts the 8 bytes of order_key as usual,
+ * reads the counts back, and then -- when no bin of the top k bytes holds more than 2 * here / 256 records and, unless
+ * LSB_FLAG_NO_SKIP, no byte is constant -- runs k stable steps on the top k bytes and ONE bucket pass that sorts every
+ * run of equal top bytes on chip: k + 1 trips through HBM instead of 8, the same output.  k is the least k >= 2 with
+ * here <= 128 * 256^k (2^30 and 2^31 records: k = 3).  A run of more than 256 records is copied as it is when its
+ * order keys are already in order (equal keys: the NaNs of a float64 sort, a repeated key); one that is not (correlated
+ * bytes) makes the call sort the bucket pass's input with the 8 byte steps after all.  Every other call, and any input that fails the
+ * test, takes the byte steps.  Definition: plan_bucket in csrc/lsbsort.cu, csrc/lsb_bucket.cuh.
+ * Two more lsb_tune keys, for tests and A/B comparisons of the two paths: "bk_mode" (0 = the rule above [default],
+ * 1 = never take the bucket plan, 2 = take it whenever the call's shape allows: no size threshold, no histogram test)
+ * and "bk_bytes" (k, 2..7; 0 = from the shard size [default]).
+ */
 
 /* ---- multi-GPU wiring (MPI_Init / MPI_COMM_WORLD, :588,:613-616) ----------------- */
 
