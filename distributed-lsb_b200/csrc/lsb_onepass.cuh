@@ -140,7 +140,8 @@ __device__ __noinline__ bool op_wait_ge(const unsigned* p, unsigned want, const 
 #define OP_T(i) do {} while (0)
 #endif
 constexpr int OP_NPROF1 = 24;  // one-pass kernel's own stage clocks
-constexpr int OP_NPROF = 40;   // the whole table: 0..23 one-pass kernel, 24..39 partition_kernel (PT_PROF0)
+constexpr int OP_NPROF = 56;   // the whole table: 0..23 one-pass kernel, 24..39 partition_kernel (PT_PROF0),
+                               // 40..55 bucket_sort_kernel (BK_PROF0)
 
 // K1 tile body after the tile has landed in shared memory: rank by the low byte, publish the
 // pieces, write the tile sorted by low byte into its place in the supertile scratch.

@@ -898,6 +898,7 @@ int launch_bucket(lsb_ctx* c, uint32_t korder, int kb) {
   a.low_mask = (1ULL << (64 - 8 * kb)) - 1;
   a.overflow = c->bk_overflow;
   a.korder = korder;
+  a.prof = c->op_prof;
   const unsigned grid = (unsigned)div_ceil(c->here, BK_TILE);
   if (korder) bucket_sort_kernel<true><<<grid, BK_THREADS, BK_SMEM, c->stream>>>(a);
   else bucket_sort_kernel<false><<<grid, BK_THREADS, BK_SMEM, c->stream>>>(a);
@@ -1588,7 +1589,8 @@ int lsb_tune(const char* key, int value) {
 }
 
 #ifdef LSB_OP_PROF
-// tools/ only: read and clear the one-pass kernel's stage clocks
+static_assert(BK_PROF0 + BK_NPROF <= OP_NPROF, "the bucket kernel's stage clocks fit the table");
+// tools/ only: read and clear the stage clocks (OP_NPROF words: one-pass, partition and bucket kernels)
 int lsb_debug_prof(lsb_ctx* c, unsigned long long* out) {
   if (!c || !out) return LSB_ERR_ARG;
   CU(c, cudaMemcpy(out, c->op_prof, sizeof(unsigned long long) * OP_NPROF, cudaMemcpyDeviceToHost));

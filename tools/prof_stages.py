@@ -32,7 +32,7 @@ PT_NAMES = ["ticket (atomic) + clear counters + barrier", "segment lookup + bulk
             "look-back (thread 0's bin)", "barrier after the look-back", "gather + stores issued"]
 if a.two_step:
     with lsb.DistributedSorter(n, ranks=1, flags=L.FLAG_NO_SKIP) as s:
-        out = (ctypes.c_uint64 * 40)()
+        out = (ctypes.c_uint64 * 56)()
         s.generate()
         s.my_sort()
         lib.lsb_debug_prof(s._ctx, out)
@@ -51,7 +51,7 @@ if a.two_step:
 with lsb.DistributedSorter(n, ranks=1, flags=L.FLAG_NO_SKIP | L.FLAG_ONE_PASS) as s:
     s.generate()
     s.my_sort()
-    out = (ctypes.c_uint64 * 40)()
+    out = (ctypes.c_uint64 * 56)()
     lib.lsb_debug_prof(s._ctx, out)
     s.generate()
     st = s.my_sort()
